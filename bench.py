@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torchrun, one rank per GPU)
     python bench.py --impl reference ...                      (CPU port of the reference's scan, rank 0 only)
     python bench.py --workload config1|dictionary|config2|config3|config4 [--scaling strong] [--bytes B]
+    python bench.py ... --dump-outputs DIR                    (the records of the last timed step as DIR/*.npy)
 
 A "step" is one pass of the hot path over one rank's shard of the input:
   * `value`  : device-resident -- input already in HBM, one pfac_scan_device launch sequence per step,
@@ -72,7 +73,37 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-job", action="store_true", help="skip the pfac_job_run leg (N>1, rank 0 over all devices)")
     ap.add_argument("--e2e-steps", type=int, default=0, help="steps of the end-to-end leg (default min(steps, 10))")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the records of the last timed step (rank 0) as DIR/*.npy, see dump_outputs()")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        # the reference arm scans a sample whose size comes from a timing calibration: not the same bytes every run
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
+
+
+DUMP_MAX_RECORDS = 2_000_000     # 3 float64 arrays of this length: 48 MB, under the 64 MB the dump may take
+
+
+def dump_outputs(out_dir, records):
+    """Writes what a caller of the timed path receives, the (pos, id) records of one scan, so that two builds can be
+    compared output for output: count.npy (the number of records), pos.npy and id.npy (float64, exact for 32-bit
+    values), and rows.npy, the record numbers pos/id hold -- all records up to DUMP_MAX_RECORDS, beyond that a fixed
+    seeded sample of them in record order.  Positions are as the records hold them, relative to the start of the
+    dumping rank's shard (rank 0's starts at 0)."""
+    n = len(records)
+    if n <= DUMP_MAX_RECORDS:
+        rows = np.arange(n)
+    else:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_RECORDS, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"count": np.array([n], dtype=np.float64), "rows": rows.astype(np.float64),
+           "pos": (records[rows, 0].astype(np.int64) & 0xFFFFFFFF).astype(np.float64),   # uint32 held in an int32
+           "id": records[rows, 1].astype(np.float64)}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def workload_patterns(name):
@@ -482,6 +513,8 @@ def main():
         return ev0.elapsed_time(ev1)
 
     ms = timed_steps()      # the bench value: exactly args.steps steps, nothing between the kernels of a step
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_out[:int(d_cnt.item())].cpu().numpy())
     # the roofline's kernel time: the same steps once more with an event pair around the dominant kernel of every
     # launch sequence, on its stream (the pair sits between the kernels of a step, so these steps are not the value)
     m.set_timing(True)

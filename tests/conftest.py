@@ -78,6 +78,12 @@ def golden():
     return json.load(open(os.path.join(GOLDEN, "golden.json")))
 
 
+@pytest.fixture(scope="session")
+def ref_live():
+    """What the reference computed on the seeded inputs of _ref_sets.py (tests/golden/make_ref_live.py)."""
+    return json.load(open(os.path.join(GOLDEN, "ref_live.json")))
+
+
 def sha_i32(a):
     return hashlib.sha256(np.ascontiguousarray(a, dtype=np.int32).tobytes()).hexdigest()
 

@@ -50,6 +50,30 @@ def test_reference_arm_other_ranks_print_nothing():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_dump_outputs(tmp_path, monkeypatch):
+    """--dump-outputs: float64 arrays, every record up to DUMP_MAX_RECORDS, a fixed sample beyond (the same on every
+    run), under 64 MB at the largest sample."""
+    import numpy as np
+    import bench
+    rec = np.array([[5, 3], [-1, 7], [1 << 30, 10000]], dtype=np.int32)
+    bench.dump_outputs(tmp_path / "small", rec)
+    got = {n: np.load(tmp_path / "small" / f"{n}.npy") for n in ("count", "rows", "pos", "id")}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert got["count"].tolist() == [3] and got["rows"].tolist() == [0, 1, 2]
+    assert got["pos"].tolist() == [5, 2 ** 32 - 1, 1 << 30] and got["id"].tolist() == [3, 7, 10000]
+    big = np.random.default_rng(1).integers(0, 1 << 31, (bench.DUMP_MAX_RECORDS + 1, 2)).astype(np.int32)
+    for run in ("a", "b"):
+        bench.dump_outputs(tmp_path / run, big)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 << 20
+    for f in files:
+        assert np.array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)), f
+    rows = np.load(tmp_path / "a" / "rows.npy").astype(np.int64)
+    assert len(rows) == bench.DUMP_MAX_RECORDS and (np.diff(rows) > 0).all()
+    assert np.array_equal(np.load(tmp_path / "a" / "pos.npy"), big[rows, 0].astype(np.float64))
+    assert np.load(tmp_path / "a" / "count.npy").tolist() == [bench.DUMP_MAX_RECORDS + 1]
+
+
 def test_shared_config_is_a_function_of_the_command_line():
     import bench
     a = SimpleNamespace(scaling="weak", bytes=0, streams=4)

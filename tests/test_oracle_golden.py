@@ -2,13 +2,13 @@
 reference's own table builder (tests/golden/make_golden.py), the known-answer counts in the
 reference tree, and -- where oracle/_ref was built -- the reference builder itself, live."""
 import hashlib
-import os
 import re
 
 import numpy as np
 import pytest
 
 from _oracle import Oracle, RefBuild, ref_available, render_result, scan_tables_cpu
+from _ref_sets import oracle_builder_sets
 from conftest import digest, parse_key
 
 
@@ -108,24 +108,21 @@ def test_oracle_error_cases():
     Oracle(b"x" * 1022 + b"\n", 1, 4096)
 
 
-@pytest.mark.skipif(not ref_available() or not os.path.isdir("/root/reference"),
-                    reason="oracle/_ref not built or reference tree absent (GPU box)")
-def test_oracle_equals_live_reference_builder(fixtures, tmp_path):
-    """Random pattern sets through the reference's own create_PFAC_table_reorder + FFDM."""
-    rng = np.random.default_rng(7)
-    for trial in range(6):
-        n = int(rng.integers(5, 400))
-        alpha = int(rng.integers(2, 40))
-        pats = set()
-        while len(pats) < n:
-            L = int(rng.integers(1, 12))
-            pats.add(bytes((rng.integers(0, alpha, L) + 97).astype(np.uint8)))
-        blob = b"".join(p + b"\n" for p in sorted(pats, key=lambda _: rng.random()))
-        f = tmp_path / f"p{trial}"
-        f.write_bytes(blob)
-        width = int(2 ** rng.integers(0, 13))
-        rb = RefBuild(str(f), streamnum=1 + trial % 2, width=width)
-        o = Oracle(blob, n_parts=rb.n_parts, width=width)
-        assert o.max_pat_len == rb.max_pat_len
-        for g in range(rb.n_parts):
-            assert o.part(g).same_as(rb.part(g)), (trial, g, width)
+def test_oracle_equals_live_reference_builder(ref_live, tmp_path):
+    """Random pattern sets through the reference's own create_PFAC_table_reorder + FFDM: its tables as stored in
+    tests/golden/ref_live.json, and the live builder too where oracle/_ref was built."""
+    live = ref_available()
+    for trial, (blob, streamnum, width) in enumerate(oracle_builder_sets()):
+        want = ref_live["oracle_builder"][trial]
+        assert (want["streamnum"], want["width"]) == (streamnum, width), trial
+        o = Oracle(blob, n_parts=len(want["parts"]), width=width)
+        assert o.max_pat_len == want["max_pat_len"], trial
+        for g, d in enumerate(want["parts"]):
+            assert digest(o.part(g)) == d, (trial, g, width)
+        if live:
+            f = tmp_path / f"p{trial}"
+            f.write_bytes(blob)
+            rb = RefBuild(str(f), streamnum=streamnum, width=width)
+            assert rb.n_parts == o.n_parts and o.max_pat_len == rb.max_pat_len
+            for g in range(rb.n_parts):
+                assert o.part(g).same_as(rb.part(g)), (trial, g, width)

@@ -589,16 +589,24 @@ def test_c_host_example_end_to_end(fixtures, golden, tmp_path):
     assert hashlib.md5(out).hexdigest() == golden["results"]["dictionary_x_1M"]["md5"]
 
 
-def test_records_equal_the_reference_gpu_kernel():
+def test_records_equal_the_reference_gpu_kernel(ref_live):
     """The reference's own TraceTable_kernel (master_kernel.cu built for sm_100a by `make -C oracle
-    refgpu`, texture fetches replaced by __ldg) run on this GPU: its dense result, sifted the way
-    main.cc:304-350 does, equals the product's records for the config-3 pattern set."""
+    refgpu`, texture fetches replaced by __ldg): its dense result, sifted the way main.cc:304-350 does,
+    equals the product's records for the config-3 pattern set -- as stored in tests/golden/ref_live.json,
+    and run live on this GPU too where oracle/_ref was built."""
     import json
-    torch_cuda()
+    from _ref_sets import gpu_kernel_case
+    torch = torch_cuda()
+    want = ref_live["gpu_kernel_config3"]
+    pats, text = gpu_kernel_case()
+    assert len(text) == want["bytes"] and len(want["pos"]) > 0
+    m = pf.Matcher(pf.Tables.from_bytes(pats, 1, 256))
+    for got in (m.scan_host(text), m.scan_device(torch.from_numpy(text).cuda())):
+        assert got["pos"].astype(np.int64).tolist() == want["pos"] and got["id"].astype(np.int64).tolist() == want["id"]
+    m.close()
     tool = os.path.join(os.path.dirname(os.path.abspath(__file__)), "refgpu_bench.py")
     r = subprocess.run([sys.executable, tool, "--mib", "3"], capture_output=True, text=True, timeout=170)
     assert r.returncode == 0, r.stderr[-2000:]
     line = json.loads(r.stdout.strip().splitlines()[-1])
-    if "unavailable" in line:
-        pytest.skip(line["unavailable"])
-    assert line["records_equal_to_product"] is True and line["matches"] > 0, line
+    if "unavailable" not in line:
+        assert line["records_equal_to_product"] is True and line["matches"] == len(want["pos"]), line

@@ -9,6 +9,7 @@ import pytest
 import phfpfac_b200 as pf
 import pfac_synth as synth
 from _oracle import Oracle, RefBuild, ref_available
+from _ref_sets import product_builder_sets, random_patterns
 from conftest import digest, parse_key
 
 
@@ -31,16 +32,6 @@ def test_kat_counts(fixtures, golden):
     for name, k in golden["kat_counts"].items():
         p = pf.Tables.from_bytes(fixtures[name], n_parts=1, width=k["width"]).part(0)
         assert (p.state_num, p.n_final, p.n_keys, p.max_key) == (k["state_num"], k["n_final"], k["n_keys"], k["max_key"])
-
-
-def random_patterns(rng, n, alpha, max_len, base=97):
-    pats = set()
-    while len(pats) < n:
-        L = int(rng.integers(1, max_len + 1))
-        pats.add(bytes((rng.integers(0, alpha, L) + base).astype(np.uint8)))
-    pats = list(pats)
-    rng.shuffle(pats)
-    return b"".join(p + b"\n" for p in pats)
 
 
 @pytest.mark.parametrize("seed", range(8))
@@ -160,21 +151,24 @@ def test_large_set_beyond_reference_limits():
         assert s == rank and p.idmap[s] == order[rank] + 1
 
 
-@pytest.mark.skipif(not ref_available() or not os.path.isdir("/root/reference"),
-                    reason="oracle/_ref not built or reference tree absent (GPU box)")
-def test_tables_equal_live_reference_builder(tmp_path):
-    rng = np.random.default_rng(17)
-    for trial in range(4):
-        blob = random_patterns(rng, int(rng.integers(10, 600)), int(rng.integers(2, 60)), 14)
-        f = tmp_path / f"p{trial}"
-        f.write_bytes(blob)
-        width = int(2 ** rng.integers(3, 13))
-        rb = RefBuild(str(f), streamnum=1, width=width)
+def test_tables_equal_live_reference_builder(ref_live, tmp_path):
+    """Random sets in 4 partitions and as one automaton: the reference builder's tables as stored in
+    tests/golden/ref_live.json, and the live builder too where oracle/_ref was built."""
+    live = ref_available()
+    for trial, (blob, width) in enumerate(product_builder_sets()):
+        want = ref_live["product_builder"][trial]
+        assert want["width"] == width, trial
         t = pf.Tables.from_bytes(blob, n_parts=4, width=width)
-        for g in range(4):
-            assert same(t.part(g), rb.part(g)), (trial, g)
-        rb1 = RefBuild(str(f), width=width, single=True)
-        assert same(pf.Tables.from_bytes(blob, n_parts=1, width=width).part(0), rb1.part(0))
+        t1 = pf.Tables.from_bytes(blob, n_parts=1, width=width)
+        assert [digest(t.part(g)) for g in range(4)] == want["parts"], trial
+        assert digest(t1.part(0)) == want["single"], trial
+        if live:
+            f = tmp_path / f"p{trial}"
+            f.write_bytes(blob)
+            rb = RefBuild(str(f), streamnum=1, width=width)
+            for g in range(4):
+                assert same(t.part(g), rb.part(g)), (trial, g)
+            assert same(t1.part(0), RefBuild(str(f), width=width, single=True).part(0))
 
 
 @pytest.mark.parametrize("case", ["experimentpattern", "xad", "dictionary", "short", "config3", "binary"])
