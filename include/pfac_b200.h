@@ -11,7 +11,8 @@
  * Layers
  *   pfac_tables_*  : pattern file -> PFAC trie -> PHF (r/HT/val) arrays, bit-compatible with
  *                    create_PFAC_table_reorder() + FFDM()  (create_PFAC_table_reorder.c:6, phf.c:151)
- *   pfac_ctx_*     : one device: table upload + scan of device-resident or host buffers
+ *   pfac_ctx_*     : one device: table upload + scan of device-resident or host buffers, and of
+ *                    batches of independent device-resident documents (pfac_scan_batch_device)
  *                    (GPU_Malloc_Memory / GPU_TraceTable / GPU_Free_memory, main.cc:35-37)
  *   pfac_job_*     : all GPUs of the box: contiguous input chunk + halo per GPU, stream pipeline
  *                    per GPU (the scan loop of main.cc:171-272)
@@ -120,6 +121,10 @@ int pfac_tables_filter_profile(const pfac_tables *t, int part, uint32_t t2_bytes
                                uint32_t tm2_bytes, const void *text, uint64_t n, uint64_t counts[12]);
 /* One transition through the PHF exactly as master_kernel.cu:52-64 does it; -1 = none. */
 int32_t pfac_tables_lookup(const pfac_tables *t, int part, int32_t state, int32_t byte);
+/* Pattern length of every id: lengths[id] = depth of the final state that reports id, 0 for ids no final
+ * state reports (earlier duplicates).  lengths may be NULL: *n_ids receives max id + 1 (size of the array).
+ * PFAC_ERR_ARG if the automaton is not a tree, PFAC_ERR_OUTPUT_FULL if n < max id + 1. */
+int pfac_tables_pattern_lengths(const pfac_tables *t, int part, int32_t *lengths, int32_t n, int32_t *n_ids);
 
 /* ------------------------------------------------------------------------------ device
  * pfac_ctx_create replaces GPU_Malloc_Memory (master_kernel.cu:188-257) and the table half
@@ -148,6 +153,30 @@ int pfac_scan_device(pfac_ctx *ctx, const void *d_in, uint64_t n_starts, uint64_
 /* Same, synchronous; *count receives the device count.  PFAC_ERR_OUTPUT_FULL if *count > cap. */
 int pfac_scan_device_sync(pfac_ctx *ctx, const void *d_in, uint64_t n_starts, uint64_t n_valid,
                           uint64_t base_pos, void *d_out, uint64_t cap, uint64_t *count, void *stream);
+
+/* Batch of independent documents (packets, log lines, requests) in ONE launch sequence; the reference has
+ * no counterpart.  The result of document i is exactly what pfac_scan_device returns for it alone
+ * (n_starts = n_valid = its length, base_pos = 0): a match never crosses from one document into the next.
+ * The packed buffer is scanned once; a split pass then drops the records whose pattern runs past the end
+ * of their document and makes positions relative to it.  Supported by contexts whose automaton is a tree
+ * (PFAC_ERR_ARG otherwise: sets wrapped from arrays may share states) and whose patterns are at most 513
+ * bytes long (PFAC_ERR_LIMIT otherwise: beyond that the reference's 4096+512 tile bound makes results
+ * depend on where a document lies in the buffer).
+ *
+ * n_docs independent documents packed back to back in d_in: document i = d_in[doc_offsets[i], doc_offsets[i+1]).
+ * doc_offsets is a HOST array of n_docs + 1 entries, doc_offsets[0] = 0, non-decreasing; the total
+ * doc_offsets[n_docs] < 4 GiB as for pfac_scan_device.  The array is read before the call returns.
+ * d_out: device array of `cap` pfac_match, pos relative to the record's document; records ordered by
+ * (document, pos, pattern length).  d_doc_first: device uint64[n_docs + 1], the records of document i are
+ * d_out[d_doc_first[i], d_doc_first[i+1]).  d_count: device uint64.  If the count exceeds cap, nothing is
+ * written past d_out[cap), d_out and d_doc_first are unspecified, and the count is a capacity that suffices
+ * for a rescan (it may exceed the records the rescan returns by the matches straddling document boundaries).
+ * Same stream and ordering rules as pfac_scan_device (shares its working set). */
+int pfac_scan_batch_device(pfac_ctx *ctx, const void *d_in, const uint64_t *doc_offsets, uint32_t n_docs,
+                           void *d_out, uint64_t cap, void *d_doc_first, void *d_count, void *stream);
+/* Same, synchronous; *count receives the device count.  PFAC_ERR_OUTPUT_FULL if *count > cap. */
+int pfac_scan_batch_device_sync(pfac_ctx *ctx, const void *d_in, const uint64_t *doc_offsets, uint32_t n_docs,
+                                void *d_out, uint64_t cap, void *d_doc_first, uint64_t *count, void *stream);
 
 /* Whole GPU_TraceTable (H2D + kernel + D2H, master_kernel.cu:359-428) on HOST input, as a
  * pipeline of chunk_bytes sub-chunks (+halo) over n_streams streams.  h_in[0, n_starts) are

@@ -9,6 +9,7 @@ Host-side mirror of the reference's operator interface for the scan path
     thread_data{s0Table,r,HT,val,HTSize,...}    Tables.part(g)  (canonical arrays, bit-compatible)
     GPU_Malloc_Memory(...)                      Matcher(tables, device=...)
     GPU_TraceTable(...)                         Matcher.scan_host(...) / Matcher.scan_device(...)
+    (none: many independent documents)          Matcher.scan_batch(...) / Matcher.scan_docs(...)
     GPU_Free_memory(...)                        Matcher.close()
     merge + fprintf loop (main.cc:304-350)      format_records / write_result
 
@@ -126,6 +127,16 @@ class Tables:
                 "slices_flagged", "slices")
         return dict(zip(keys, list(c)))
 
+    def pattern_lengths(self, g=0):
+        """np.int32[n_ids]: the length of every pattern id of partition g (0 for ids no final state reports:
+        the earlier copies of a duplicated line).  Refused (PfacError) for automata that are not trees."""
+        n = C.c_int32(0)
+        check(lib.pfac_tables_pattern_lengths(self._h, g, None, 0, C.byref(n)))
+        out = np.zeros(n.value, dtype=np.int32)
+        if n.value:
+            check(lib.pfac_tables_pattern_lengths(self._h, g, out.ctypes.data, n.value, C.byref(n)))
+        return out
+
     def lookup(self, state, byte, g=0):
         return lib.pfac_tables_lookup(self._h, g, state, byte)
 
@@ -219,6 +230,52 @@ class Matcher:
             res = np.zeros(cnt.value, dtype=MATCH_DTYPE)
             res["pos"], res["id"] = rec[:, 0], rec[:, 1]
             return res
+
+    # -- many independent documents packed back to back: one launch sequence, per-document results
+    def scan_batch(self, values, offsets, cap=None, offset=0):
+        """values: torch uint8 CUDA tensor (or host bytes / uint8 array, uploaded through torch) holding the
+        documents back to back from byte `offset` on; offsets: n_docs + 1 integers, document i = bytes
+        [offsets[i], offsets[i+1]).  Returns (doc_first: np.uint64[n_docs + 1], records: MATCH_DTYPE): the records
+        of document i are records[doc_first[i]:doc_first[i+1]], positions relative to the document -- exactly
+        what scan_device returns for that document alone (synchronous)."""
+        import torch
+        if not isinstance(values, torch.Tensor):
+            values = torch.from_numpy(_as_u8(values).copy()).cuda(self.device)
+        offs = np.asarray(offsets)
+        if offs.ndim != 1 or len(offs) < 1 or not np.issubdtype(offs.dtype, np.integer):
+            raise ValueError("offsets must be a 1-D sequence of n_docs + 1 integers")
+        if (offs < 0).any() or int(offs.max()) > values.numel() - offset:
+            raise ValueError("offsets point outside the values")
+        offs = np.ascontiguousarray(offs, dtype=np.uint64)
+        n_docs = len(offs) - 1
+        cap = max(1024, int(offs[-1]) // 8) if cap is None else cap
+        stream = torch.cuda.current_stream(values.device).cuda_stream
+        while True:
+            out = torch.empty((max(cap, 1), 2), dtype=torch.int32, device=values.device)
+            first = torch.empty(n_docs + 1, dtype=torch.int64, device=values.device)
+            cnt = C.c_uint64(0)
+            if stream == 0:     # the legacy default stream: 0 means "the library's own stream" to the C ABI
+                torch.cuda.current_stream(values.device).synchronize()
+            rc = lib.pfac_scan_batch_device_sync(self._h, values.data_ptr() + offset if values.numel() else None,
+                                                 offs.ctypes.data, n_docs, out.data_ptr(), cap, first.data_ptr(),
+                                                 C.byref(cnt), stream or None)
+            if rc == PFAC_ERR_OUTPUT_FULL:
+                cap = cnt.value
+                continue
+            check(rc)
+            rec = out[:cnt.value].cpu().numpy().astype(np.uint32).reshape(-1, 2)
+            res = np.zeros(cnt.value, dtype=MATCH_DTYPE)
+            res["pos"], res["id"] = rec[:, 0], rec[:, 1]
+            return first.cpu().numpy().view(np.uint64), res
+
+    def scan_docs(self, docs):
+        """docs: list of bytes-like documents -> list of per-document MATCH_DTYPE arrays (one batch scan)."""
+        parts = [_as_u8(d) for d in docs]
+        offs = np.zeros(len(parts) + 1, dtype=np.uint64)
+        offs[1:] = np.cumsum([len(p) for p in parts], dtype=np.uint64)
+        buf = np.concatenate(parts) if parts else np.zeros(0, dtype=np.uint8)
+        first, rec = self.scan_batch(buf, offs)
+        return [rec[int(first[i]):int(first[i + 1])] for i in range(len(parts))]
 
     # -- host input: H2D + kernel + D2H pipeline
     def scan_host(self, data, n_starts=None, base_pos=0, cap=None):

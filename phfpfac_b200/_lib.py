@@ -18,9 +18,10 @@ ABI_SYMBOLS = [
     "pfac_tables_source_hash", "pfac_pattern_file_hash",
     "pfac_tables_n_parts", "pfac_tables_n_patterns", "pfac_tables_max_pat_len", "pfac_tables_width",
     "pfac_tables_part_info", "pfac_tables_s0", "pfac_tables_r", "pfac_tables_HT", "pfac_tables_val",
-    "pfac_tables_idmap", "pfac_tables_lookup", "pfac_tables_derive_check", "pfac_tables_filter_profile",
+    "pfac_tables_idmap", "pfac_tables_lookup", "pfac_tables_pattern_lengths", "pfac_tables_derive_check",
+    "pfac_tables_filter_profile",
     "pfac_device_count", "pfac_ctx_create", "pfac_ctx_destroy", "pfac_ctx_device",
-    "pfac_scan_device", "pfac_scan_device_sync", "pfac_scan_host", "pfac_host_alloc", "pfac_host_free", "pfac_host_register", "pfac_host_unregister",
+    "pfac_scan_device", "pfac_scan_device_sync", "pfac_scan_batch_device", "pfac_scan_batch_device_sync", "pfac_scan_host", "pfac_host_alloc", "pfac_host_free", "pfac_host_register", "pfac_host_unregister",
     "pfac_ctx_last_scan_info", "pfac_ctx_derived_info", "pfac_ctx_set_timing", "pfac_ctx_kernel_time",
     "pfac_job_create", "pfac_job_destroy", "pfac_job_run", "pfac_job_run_file", "pfac_job_n_segments", "pfac_job_segment",
     "pfac_job_last_timing", "pfac_job_plan",
@@ -29,8 +30,10 @@ ABI_SYMBOLS = [
 ]
 
 PFAC_OK = 0
+PFAC_ERR_ARG = -5
 PFAC_ERR_OUTPUT_FULL = -8
 PFAC_ERR_NO_DEVICE = -9
+PFAC_ERR_LIMIT = -10
 
 
 class PfacError(RuntimeError):
@@ -74,6 +77,7 @@ def _load():
                                                C.POINTER(C.c_uint64)]
     lib.pfac_tables_lookup.argtypes = [_vp, C.c_int, C.c_int32, C.c_int32]
     lib.pfac_tables_lookup.restype = C.c_int32
+    lib.pfac_tables_pattern_lengths.argtypes = [_vp, C.c_int, _vp, C.c_int32, C.POINTER(C.c_int32)]
     lib.pfac_device_count.argtypes = [C.POINTER(C.c_int)]
     lib.pfac_ctx_create.argtypes = [C.c_int, _vp, C.c_int, C.c_int, C.c_size_t, C.POINTER(_vp)]
     lib.pfac_ctx_destroy.argtypes = [_vp]
@@ -82,6 +86,9 @@ def _load():
     lib.pfac_scan_device.argtypes = [_vp, _vp, C.c_uint64, C.c_uint64, C.c_uint64, _vp, C.c_uint64, _vp, _vp]
     lib.pfac_scan_device_sync.argtypes = [_vp, _vp, C.c_uint64, C.c_uint64, C.c_uint64, _vp, C.c_uint64,
                                           C.POINTER(C.c_uint64), _vp]
+    lib.pfac_scan_batch_device.argtypes = [_vp, _vp, _vp, C.c_uint32, _vp, C.c_uint64, _vp, _vp, _vp]
+    lib.pfac_scan_batch_device_sync.argtypes = [_vp, _vp, _vp, C.c_uint32, _vp, C.c_uint64, _vp,
+                                                C.POINTER(C.c_uint64), _vp]
     lib.pfac_scan_host.argtypes = [_vp, _vp, C.c_uint64, C.c_uint64, C.c_uint64, _vp, C.c_uint64,
                                    C.POINTER(C.c_uint64)]
     lib.pfac_host_alloc.argtypes = [C.POINTER(_vp), C.c_size_t]

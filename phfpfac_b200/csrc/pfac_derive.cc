@@ -621,6 +621,41 @@ void derive_patdir(const Partition &P, PatDir &out)
     if (!pool.empty()) memcpy(out.image.data() + out.off_pool, pool.data(), pool.size());
 }
 
+int pattern_lengths(const Partition &P, std::vector<int32_t> &len)
+{
+    int32_t max_id = -1;
+    for (int32_t id : P.idmap) {
+        if (id < 0) return set_error(PFAC_ERR_ARG, "pattern id %d is negative", id);
+        max_id = std::max(max_id, id);
+    }
+    len.assign((size_t)(max_id + 1), 0);
+    if (P.n_final < 1 || P.s0.size() != (size_t)kCharSet) return PFAC_OK;
+    Graph g;
+    build_graph(P, g);
+    // depth-first from the root; a state reached twice (shared states or a cycle) has no single depth
+    struct Item { int32_t state; int32_t depth; };
+    std::vector<Item> stack;
+    std::vector<uint8_t> seen((size_t)g.n_states, 0);
+    for (int b = 0; b < kCharSet; b++)
+        if (P.s0[(size_t)b] >= 0) stack.push_back({P.s0[(size_t)b], 1});
+    while (!stack.empty()) {
+        const Item it = stack.back();
+        stack.pop_back();
+        if (it.state >= g.n_states) continue;   // no such state: no lookup reaches it
+        if (seen[(size_t)it.state])
+            return set_error(PFAC_ERR_ARG, "the automaton is not a tree (state %d is reached twice): pattern lengths are undefined",
+                             it.state);
+        seen[(size_t)it.state] = 1;
+        if (g.is_final(it.state)) {
+            const int32_t id = P.idmap[(size_t)it.state];
+            if (len[(size_t)id]) return set_error(PFAC_ERR_ARG, "pattern id %d is reported by two final states", id);
+            len[(size_t)id] = it.depth;
+        }
+        for (uint32_t e = g.begin(it.state); e < g.end(it.state); e++) stack.push_back({g.edges[e].next, it.depth + 1});
+    }
+    return PFAC_OK;
+}
+
 // Host model of the directory look-up (tests): id of the pattern text[0, d), -1 if it is none.
 int64_t patdir_lookup(const PatDir &pd, const uint8_t *text, uint32_t d)
 {

@@ -231,6 +231,13 @@ void derive_patdir(const Partition &P, PatDir &out);
 int64_t patdir_lookup(const PatDir &pd, const uint8_t *text, uint32_t d);
 int patdir_selfcheck(const Partition &P, const PatDir &pd);   // 0 = the directory answers like the walk
 
+// ---- pattern length of every id (batch scans: a record is kept iff its pattern ends inside its document).
+// len[id] = depth of the final state that reports id, 0 for ids no reachable final state reports (the earlier
+// copies of a duplicated line); len.size() = max id + 1.  The automaton is a trie, so a final state's depth is
+// its pattern's length.  PFAC_ERR_ARG (message set) if it is not a tree -- a state reached twice, as in sets
+// wrapped from arrays that share states -- or if two final states report one id.
+int pattern_lengths(const Partition &P, std::vector<int32_t> &len);
+
 // t2/t3/tm2_bytes: shared-memory budget of the variable sections (rounded down to powers of two)
 void derive_tables(const Partition &P, uint32_t t2_bytes, uint32_t t3_bytes, uint32_t tm2_bytes, Derived &out);
 

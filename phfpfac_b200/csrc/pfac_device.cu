@@ -8,6 +8,7 @@
 #include <memory>
 #include <mutex>
 
+#include "pfac_batch.cuh"
 #include "pfac_derive.h"
 #include "pfac_internal.h"
 #include "pfac_kernel.cuh"
@@ -42,6 +43,16 @@ struct Slot {
     uint2 *d_scratch = nullptr;
     size_t scratch_cap = 0;   // records
     bool dirty = false;       // a launch sequence failed half way: the control block is reset before the next scan
+    // batch scans (pfac_batch.cuh): raw records of the packed buffer and the global positions of the kept ones
+    // (raw_cap each), the document offsets (pinned staging + device copy, doc_cap entries; doc_copied = end of
+    // the last upload from the staging buffer) and the split pass's per-CTA counts
+    uint2 *d_raw = nullptr;
+    uint32_t *d_kpos = nullptr;
+    size_t raw_cap = 0;
+    uint32_t *h_doc = nullptr, *d_doc = nullptr;
+    size_t doc_cap = 0;
+    cudaEvent_t doc_copied = nullptr;
+    unsigned long long *d_blk = nullptr;
 };
 
 struct Stage {   // one pipeline stage of pfac_scan_host
@@ -75,6 +86,11 @@ struct pfac_ctx {
     uint32_t wc_bytes = 0;
     size_t dense_smem = 0;
     bool dense_first = false;      // no detector: the dense-match kernel walks every tile (sets with patterns <= 3 bytes)
+    // batch scans: pattern length of every id; batch_rc != PFAC_OK: the set does not support them (batch_why)
+    int32_t *d_patlen = nullptr;
+    uint32_t n_ids = 0;
+    int batch_rc = PFAC_OK;
+    std::string batch_why;
     Derived dv;   // image layout and hash parameters (the image bytes are dropped after the upload)
     uint32_t image_bytes = 0;
     int32_t ht_size = 0, width_bit = 0, n_final = 0, max_pat_len = 0;
@@ -137,6 +153,12 @@ void slot_free(Slot &s)
     if (s.d_tile_src) cudaFree(s.d_tile_src);
     if (s.d_tile_nc) cudaFree(s.d_tile_nc);
     if (s.d_scratch) cudaFree(s.d_scratch);
+    if (s.d_raw) cudaFree(s.d_raw);
+    if (s.d_kpos) cudaFree(s.d_kpos);
+    if (s.d_doc) cudaFree(s.d_doc);
+    if (s.h_doc) cudaFreeHost(s.h_doc);
+    if (s.doc_copied) cudaEventDestroy(s.doc_copied);
+    if (s.d_blk) cudaFree(s.d_blk);
     s = Slot();
 }
 
@@ -393,6 +415,107 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
     return PFAC_OK;
 }
 
+// Enqueue a batch scan on `stream` (pfac_batch.cuh): the documents' offsets are uploaded, the packed buffer is
+// scanned into the slot's raw-record buffer, the split pass writes the caller's records, d_doc_first and
+// d_count.  On completion slot.d_result holds {count, error}.  info: the counters of pfac_ctx_last_scan_info.
+int launch_batch(pfac_ctx *ctx, Slot &slot, const void *d_in, const uint64_t *doc_offsets, uint32_t n_docs,
+                 void *d_out, uint64_t cap, void *d_doc_first, void *d_count, cudaStream_t stream, uint64_t info[8])
+{
+    if (ctx->batch_rc != PFAC_OK) return set_error(ctx->batch_rc, "%s", ctx->batch_why.c_str());
+    if (n_docs == 0xFFFFFFFFu) return set_error(PFAC_ERR_LIMIT, "a batch holds fewer than 2^32 - 1 documents");
+    if (doc_offsets[0] != 0)
+        return set_error(PFAC_ERR_ARG, "doc_offsets[0] = %llu: the first document starts at 0", (unsigned long long)doc_offsets[0]);
+    const uint64_t total = doc_offsets[n_docs];
+    if (total >= (1ull << 32)) return set_error(PFAC_ERR_LIMIT, "one batch covers less than 4 GiB; split the input");
+    if (!d_in && total) return set_error(PFAC_ERR_ARG, "null input of %llu bytes", (unsigned long long)total);
+    int e = slot_init(slot);
+    if (e) return e;
+    const uint32_t grid = 2u * (uint32_t)ctx->sm_count;   // CTAs of the count and split kernels
+    if (!slot.d_blk) CU_TRY(cudaMalloc(&slot.d_blk, (grid + 1) * sizeof(unsigned long long)));
+    if (!slot.doc_copied) CU_TRY(cudaEventCreateWithFlags(&slot.doc_copied, cudaEventDisableTiming));
+    // grow the offset and raw-record buffers (synchronises the stream first: the old ones may still be in use)
+    const size_t n_off = (size_t)n_docs + 1;
+    if (n_off > slot.doc_cap) {
+        CU_TRY(cudaStreamSynchronize(stream));
+        if (slot.d_doc) cudaFree(slot.d_doc);
+        if (slot.h_doc) cudaFreeHost(slot.h_doc);
+        slot.d_doc = slot.h_doc = nullptr;
+        slot.doc_cap = 0;
+        const size_t n = std::max<size_t>(n_off, 4096);
+        CU_TRY(cudaMalloc(&slot.d_doc, n * sizeof(uint32_t)));
+        CU_TRY(cudaHostAlloc(&slot.h_doc, n * sizeof(uint32_t), cudaHostAllocPortable));
+        slot.doc_cap = n;
+    }
+    const size_t want = (size_t)std::max<uint64_t>(cap, 4096);
+    if (want > slot.raw_cap) {
+        CU_TRY(cudaStreamSynchronize(stream));
+        if (slot.d_raw) cudaFree(slot.d_raw);
+        if (slot.d_kpos) cudaFree(slot.d_kpos);
+        slot.d_raw = nullptr;
+        slot.d_kpos = nullptr;
+        slot.raw_cap = 0;
+        CU_TRY(cudaMalloc(&slot.d_raw, want * sizeof(uint2)));
+        CU_TRY(cudaMalloc(&slot.d_kpos, want * sizeof(uint32_t)));
+        slot.raw_cap = want;
+    }
+    // offsets -> pinned staging once the previous upload from it is done, checked on the way (32 bits suffice:
+    // total < 4 GiB) -> device
+    CU_TRY(cudaEventSynchronize(slot.doc_copied));
+    uint64_t prev = 0;
+    bool decreasing = false;
+    for (size_t i = 0; i < n_off; i++) {
+        const uint64_t v = doc_offsets[i];
+        decreasing |= v < prev;
+        prev = v;
+        slot.h_doc[i] = (uint32_t)v;
+    }
+    if (decreasing) return set_error(PFAC_ERR_ARG, "doc_offsets decrease");
+    CU_TRY(cudaMemcpyAsync(slot.d_doc, slot.h_doc, n_off * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+    CU_TRY(cudaEventRecord(slot.doc_copied, stream));
+
+    uint64_t tiles = 0, ctas = 0, launches = 0;
+    e = launch_scan(ctx, slot, d_in, total, total, 0, 0u, slot.d_raw, slot.raw_cap, nullptr, stream, &tiles, &ctas,
+                    &launches);
+    if (e) return e;
+    BatchParams bp;
+    memset(&bp, 0, sizeof bp);
+    bp.raw = slot.d_raw;
+    bp.raw_cap = slot.raw_cap;
+    bp.doc = slot.d_doc;
+    bp.n_docs = n_docs;
+    bp.len = ctx->d_patlen;
+    bp.n_ids = ctx->n_ids;
+    bp.blk = slot.d_blk;
+    bp.out = (uint2 *)d_out;
+    bp.cap = cap;
+    bp.kpos = slot.d_kpos;
+    bp.doc_first = (unsigned long long *)d_doc_first;
+    bp.result = slot.d_result;
+    bp.count_out = (unsigned long long *)d_count;
+    cudaLaunchAttribute pdl[1];
+    pdl[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    pdl[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t lc = {};
+    lc.stream = stream;
+    lc.attrs = pdl;
+    lc.numAttrs = ctx->use_pdl ? 1 : 0;
+    lc.blockDim = dim3(kBatchThreads);
+    lc.gridDim = dim3(grid);
+    CU_TRY(cudaLaunchKernelEx(&lc, pfac_batch_count_kernel, bp));
+    CU_TRY(cudaLaunchKernelEx(&lc, pfac_batch_split_kernel, bp));
+    lc.gridDim = dim3((uint32_t)std::min<uint64_t>((n_off + kBatchThreads - 1) / kBatchThreads, grid));
+    CU_TRY(cudaLaunchKernelEx(&lc, pfac_batch_docs_kernel, bp));
+    info[0] = launches + 3;
+    info[1] = tiles;
+    info[2] = ctas;
+    info[3] = ctx->smem_bytes;
+    info[4] = n_off * sizeof(uint32_t);
+    info[5] = 0;
+    info[6] = 1;
+    info[7] = 0;
+    return PFAC_OK;
+}
+
 void free_stage(Stage &s)
 {
     if (s.d_in) cudaFree(s.d_in);
@@ -562,6 +685,24 @@ int pfac_ctx_create(int device, const pfac_tables *t, int part, int n_streams, s
         CU_TRY(cudaFuncSetAttribute(pfac_dense_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max));
         CU_TRY(cudaFuncSetAttribute(pfac_dense_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max));
     }
+    {   // batch scans need each id's pattern length (a tree-shaped automaton) and results that do not depend on
+        // where a document lies in the packed buffer (no reference tile bound: patterns of <= 513 bytes)
+        std::vector<int32_t> len;
+        if (pattern_lengths(P, len) != PFAC_OK) {
+            ctx->batch_rc = PFAC_ERR_ARG;
+            ctx->batch_why = pfac_last_error();
+        } else if (P.max_len > kRefHalo + 1) {
+            ctx->batch_rc = PFAC_ERR_LIMIT;
+            ctx->batch_why = "batch scans need patterns of at most 513 bytes (the reference's 4096+512 tile bound "
+                             "would make results depend on where a document lies in the batch)";
+        } else {
+            ctx->n_ids = (uint32_t)len.size();
+            CU_TRY(cudaMalloc(&ctx->d_patlen, std::max<size_t>(len.size(), 1) * sizeof(int32_t)));
+            if (!len.empty())
+                CU_TRY(cudaMemcpy(ctx->d_patlen, len.data(), len.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+            ctx->table_bytes += std::max<size_t>(len.size(), 1) * sizeof(int32_t);
+        }
+    }
     ctx->dense_first = ctx->dv.has_short != 0;
     if (const char *v = getenv("PFAC_DENSE_FIRST")) ctx->dense_first = atoi(v) != 0;   // experiments: force either path
     ctx->table_bytes += n_r * 4 + n_ht * 8 + n_id * 4 + 1024 + ctx->image_bytes + ctx->dv.gimage.size() + ctx->wc_bytes + (ctx->d_step ? n_ht * 16 + 2048 : 0);
@@ -612,6 +753,7 @@ void pfac_ctx_destroy(pfac_ctx *ctx)
     if (ctx->d_s0) cudaFree(ctx->d_s0);
     if (ctx->d_gimage) cudaFree(ctx->d_gimage);
     if (ctx->d_wcache) cudaFree(ctx->d_wcache);
+    if (ctx->d_patlen) cudaFree(ctx->d_patlen);
     for (auto e : ctx->ev)
         if (e) cudaEventDestroy(e);
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
@@ -728,6 +870,53 @@ int pfac_scan_device_sync(pfac_ctx *ctx, const void *d_in, uint64_t n_starts, ui
         ctx->info[3] = ctx->smem_bytes;
         ctx->info[4] = ctx->info[5] = 0;
         ctx->info[6] = 1;
+        if (ctx->own.h_result->error_flag)
+            return set_error(PFAC_ERR_INTERNAL, "device watchdog tripped (code %u)", ctx->own.h_result->error_flag);
+        *count = ctx->own.h_result->count;
+    }
+    if (*count > cap) return set_error(PFAC_ERR_OUTPUT_FULL, "%llu matches exceed the capacity of %llu records",
+                                       (unsigned long long)*count, (unsigned long long)cap);
+    return PFAC_OK;
+}
+
+int pfac_scan_batch_device(pfac_ctx *ctx, const void *d_in, const uint64_t *doc_offsets, uint32_t n_docs,
+                           void *d_out, uint64_t cap, void *d_doc_first, void *d_count, void *stream)
+{
+    if (!ctx || !doc_offsets || (!d_out && cap) || !d_doc_first || !d_count)
+        return set_error(PFAC_ERR_ARG, "bad arguments to pfac_scan_batch_device");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DeviceGuard g(ctx->device);
+    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
+    uint64_t info[8];
+    int e = own_enter(ctx, st);
+    if (e) return e;
+    e = launch_batch(ctx, ctx->own, d_in, doc_offsets, n_docs, d_out, cap, d_doc_first, d_count, st, info);
+    if (e) return e;
+    e = own_leave(ctx, st);
+    if (e) return e;
+    memcpy(ctx->info, info, sizeof info);
+    return PFAC_OK;
+}
+
+int pfac_scan_batch_device_sync(pfac_ctx *ctx, const void *d_in, const uint64_t *doc_offsets, uint32_t n_docs,
+                                void *d_out, uint64_t cap, void *d_doc_first, uint64_t *count, void *stream)
+{
+    if (!ctx || !doc_offsets || (!d_out && cap) || !d_doc_first || !count)
+        return set_error(PFAC_ERR_ARG, "bad arguments to pfac_scan_batch_device_sync");
+    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
+    {
+        std::lock_guard<std::mutex> lk(ctx->mu);
+        DeviceGuard g(ctx->device);
+        uint64_t info[8];
+        int e = own_enter(ctx, st);
+        if (e) return e;
+        e = launch_batch(ctx, ctx->own, d_in, doc_offsets, n_docs, d_out, cap, d_doc_first, nullptr, st, info);
+        if (e) return e;
+        CU_TRY(cudaMemcpyAsync(ctx->own.h_result, ctx->own.d_result, sizeof(Result), cudaMemcpyDeviceToHost, st));
+        e = own_leave(ctx, st);
+        if (e) return e;
+        CU_TRY(cudaStreamSynchronize(st));
+        memcpy(ctx->info, info, sizeof info);
         if (ctx->own.h_result->error_flag)
             return set_error(PFAC_ERR_INTERNAL, "device watchdog tripped (code %u)", ctx->own.h_result->error_flag);
         *count = ctx->own.h_result->count;

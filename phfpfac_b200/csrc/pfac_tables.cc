@@ -808,6 +808,26 @@ const int32_t *pfac_tables_HT(const pfac_tables *t, int part) { const Partition 
 const int32_t *pfac_tables_val(const pfac_tables *t, int part) { const Partition *P = part_of(t, part); return P ? P->val.data() : nullptr; }
 const int32_t *pfac_tables_idmap(const pfac_tables *t, int part) { const Partition *P = part_of(t, part); return P ? P->idmap.data() : nullptr; }
 
+int pfac_tables_pattern_lengths(const pfac_tables *t, int part, int32_t *lengths, int32_t n, int32_t *n_ids)
+{
+    const Partition *P = part_of(t, part);
+    if (!P || !n_ids || n < 0) return set_error(PFAC_ERR_ARG, "bad arguments to pfac_tables_pattern_lengths");
+    try {
+        std::vector<int32_t> len;
+        const int e = pattern_lengths(*P, len);
+        if (e) return e;
+        *n_ids = (int32_t)len.size();
+        if (!lengths) return PFAC_OK;
+        if (n < *n_ids)
+            return set_error(PFAC_ERR_OUTPUT_FULL, "%d pattern ids need an array of %d entries, not %d", *n_ids, *n_ids, n);
+        if (!len.empty()) memcpy(lengths, len.data(), len.size() * sizeof(int32_t));
+        std::fill(lengths + len.size(), lengths + n, 0);
+        return PFAC_OK;
+    } catch (const std::bad_alloc &) {
+        return set_error(PFAC_ERR_NOMEM, "out of memory");
+    }
+}
+
 int pfac_tables_derive_check(const pfac_tables *t, int part, uint32_t t2_bytes, uint32_t t3_bytes, uint32_t tm2_bytes,
                              uint64_t stats[10])
 {
