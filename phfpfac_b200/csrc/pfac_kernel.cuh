@@ -134,7 +134,7 @@ constexpr int kSlice = 512;           // start positions per stage-1 step of a w
 #define PFAC_TILE_SLICES 16
 #endif
 constexpr int kSlicesPerTile = PFAC_TILE_SLICES;    // (<= 32: one flag bit each in the stage's `done` word)
-constexpr int kTile = kSlicesPerTile * kSlice;   // 16,384 start positions per tile
+constexpr int kTile = kSlicesPerTile * kSlice;   // 8,192 start positions per tile
 // Slices a warp takes at a time (a slot): stage 2 then runs over the survivors of all of them.
 // Shared-memory mode: 2 (more would leave too few slots in flight for the ring to prefetch).  Global
 // mode: 4 -- stage 2 waits on L2 there, and a fuller queue means more loads in flight per wait.
@@ -322,6 +322,8 @@ extern __shared__ __align__(128) uint8_t smem[];
 // result has one nibble per position, bit 0 of nibble j set iff start j passes stage 1:
 //     P01(j) and (Short(j) or (P12(j+1) and P23(j+2)))
 // lo = positions 0..7, hi = positions 8..15.  18 windows are looked up (16 + the two after them).
+// The entries are packed one per nibble, so only those four planes may be kept: T1 also carries P34 and ShortC
+// (bits 4 and 5, for stage 2 and mode 0), which would otherwise land in, and carry into, the next nibbles.
 __device__ __forceinline__ void filter16(const uint4 v, const uint32_t nx, const int lane, uint32_t &lo, uint32_t &hi)
 {
     const uint8_t *t1 = smem;
@@ -336,17 +338,17 @@ __device__ __forceinline__ void filter16(const uint4 v, const uint32_t nx, const
         const uint32_t i3 = __funnelshift_r(w[k], w[k + 1], 24) & 0xffffu;
         uint32_t &a = acc[k >> 1];
         const int sh = (k & 1) * 16;
-        const uint32_t e0 = t1[i0], e1 = t1[i1];
+        const uint32_t e0 = t1[i0] & 15u, e1 = t1[i1] & 15u;
         if (k == 0) first2 = e0 | (e1 << 4);
         a += e0 << sh;
         a += e1 << (sh + 4);
-        a += (uint32_t)t1[i2] << (sh + 8);
-        a += (uint32_t)t1[i3] << (sh + 12);
+        a += ((uint32_t)t1[i2] & 15u) << (sh + 8);
+        a += ((uint32_t)t1[i3] & 15u) << (sh + 12);
     }
     // windows 16 and 17 (their P12 / P23 planes belong to starts 14..15) are the next lane's windows
     // 0 and 1: one shuffle instead of two more bank-conflicted look-ups; lane 31 has no neighbour
     uint32_t ex = __shfl_down_sync(0xffffffffu, first2, 1);
-    if (lane == 31) ex = (uint32_t)t1[w[4] & 0xffffu] | ((uint32_t)t1[__byte_perm(w[4], 0u, 0x4421)] << 4);
+    if (lane == 31) ex = ((uint32_t)t1[w[4] & 0xffffu] & 15u) | (((uint32_t)t1[__byte_perm(w[4], 0u, 0x4421)] & 15u) << 4);
     // plane bits: 1 = P01, 2 = P12, 4 = P23, 8 = Short.  Align P12 of j+1 (shift 4+1), P23 of j+2
     // (shift 8+2) and Short of j (shift 3) with bit 0 of nibble j.
     const uint32_t y_lo = __funnelshift_r(acc[0], acc[1], 5), y_hi = __funnelshift_r(acc[1], ex, 5);

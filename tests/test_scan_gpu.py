@@ -86,38 +86,57 @@ def test_random_patterns_and_texts(seed):
                      chunk_bytes=int(rng.integers(1, 8)) * 16384)
 
 
-def test_edge_sizes_and_alignment():
-    """Empty input, inputs shorter than a pattern, every misalignment of the device pointer,
-    tile-edge lengths."""
+def detector_set(kind, monkeypatch):
+    """-> (tables, reference scan, text) of one of the detector cases of test_detector_paths_host.py ("A": mode 0,
+    "H": global mode, "J1": mode 1), with its environment set."""
+    from test_detector_paths_host import get_case, phase_text, set_env
+    case = get_case(kind)
+    set_env(monkeypatch, case.spec)
+    text, _ = phase_text(case)
+    return case.tables, case.reference, text[:600000].copy()
+
+
+def check_edge_sizes_and_alignment(t, ref, base, want_matches):
     torch = torch_cuda()
-    pats = b"abcab\nab\nb\ncabcabcabc\nabcabcabcabcabcabcabcabcabcabcabcab\n"
-    o = Oracle(pats, 1, 256)
-    t = pf.Tables.from_bytes(pats, 1, 256)
     m = pf.Matcher(t, device=0, n_streams=2, chunk_bytes=16384)
-    base = np.frombuffer((b"abc" * 30000)[:70001], dtype=np.uint8)
     d = torch.from_numpy(base.copy()).cuda()
     assert len(m.scan_host(np.zeros(0, dtype=np.uint8))) == 0
     for n in (0, 1, 2, 3, 4, 15, 16, 17, 31, 33, 4095, 4096, 4097, 16383, 16384, 16385, 32768, 49151, 65536, 70001):
-        pos, ids = o.scan(base[:n])
+        pos, ids = ref(base[:n])
         got = m.scan_host(base[:n])
         assert np.array_equal(got["pos"], pos) and np.array_equal(got["id"], ids), n
     for off in range(0, 19):
         n = 40000
-        pos, ids = o.scan(base[off:off + n])
+        pos, ids = ref(base[off:off + n])
         got = m.scan_device(d, n_starts=n, n_valid=n, offset=off)
         assert np.array_equal(got["pos"], pos) and np.array_equal(got["id"], ids), off
+        assert len(pos) > 0 or not want_matches
     m.close()
 
 
-def test_halo_semantics_and_shard_concatenation(fixtures):
-    """n_starts < n_valid: only matches STARTING in [0, n_starts) are reported, walks may read the
-    halo; concatenating shards reproduces the whole scan (SURVEY.md 8(e))."""
-    torch = torch_cuda()
-    pats = fixtures["xab"] + b"England were\ncricket than England in the past four years.\n"
-    data = np.frombuffer(fixtures["1M"][:-1], dtype=np.uint8)[:500000]
+def test_edge_sizes_and_alignment():
+    """Empty input, inputs shorter than a pattern, every misalignment of the device pointer,
+    tile-edge lengths."""
+    pats = b"abcab\nab\nb\ncabcabcabc\nabcabcabcabcabcabcabcabcabcabcabcab\n"
     o = Oracle(pats, 1, 256)
-    pos, ids = o.scan(data)
     t = pf.Tables.from_bytes(pats, 1, 256)
+    base = np.frombuffer((b"abc" * 30000)[:70001], dtype=np.uint8)
+    check_edge_sizes_and_alignment(t, o.scan, base, False)
+
+
+@pytest.mark.parametrize("kind", ["A", "H", "J1"])
+def test_edge_sizes_and_alignment_detector_sets(kind, monkeypatch):
+    """The same on sets that run a detector kernel (the set above has a pattern of <= 3 bytes: the
+    dense-match kernel alone): mode 0, global mode, mode 1."""
+    t, ref, text = detector_set(kind, monkeypatch)
+    check_edge_sizes_and_alignment(t, ref, text[8192 - 300:8192 - 300 + 70001], True)
+
+
+def check_halo_semantics_and_shard_concatenation(t, ref, data, b_cut):
+    """b_cut: an input length that cuts a match (reported only with the halo)."""
+    torch = torch_cuda()
+    pos, ids = ref(data)
+    assert len(pos) > 0
     m = pf.Matcher(t, device=0)
     d = torch.from_numpy(data.copy()).cuda()
     for cuts in ([0, 1, 500000], [0, 65536, 131072 + 7, 400001, 500000], [0, 499999, 500000]):
@@ -129,11 +148,29 @@ def test_halo_semantics_and_shard_concatenation(fixtures):
             is_.append(got["id"].astype(np.int32))
         assert np.array_equal(np.concatenate(ps), pos) and np.array_equal(np.concatenate(is_), ids), cuts
     # without the halo, a match that would straddle the end is NOT reported (walk stops at n_valid)
-    a, b = 0, 402 * 3 + 5          # "England were" starts at multiples of 402
-    got = m.scan_device(d, n_starts=b, n_valid=b, offset=0)
-    p2, i2 = o.scan(data[:b])
+    got = m.scan_device(d, n_starts=b_cut, n_valid=b_cut, offset=0)
+    p2, i2 = ref(data[:b_cut])
     assert np.array_equal(got["pos"], p2) and np.array_equal(got["id"], i2)
     m.close()
+
+
+def test_halo_semantics_and_shard_concatenation(fixtures):
+    """n_starts < n_valid: only matches STARTING in [0, n_starts) are reported, walks may read the
+    halo; concatenating shards reproduces the whole scan (SURVEY.md 8(e))."""
+    pats = fixtures["xab"] + b"England were\ncricket than England in the past four years.\n"
+    data = np.frombuffer(fixtures["1M"][:-1], dtype=np.uint8)[:500000]
+    o = Oracle(pats, 1, 256)
+    t = pf.Tables.from_bytes(pats, 1, 256)
+    check_halo_semantics_and_shard_concatenation(t, o.scan, data, 402 * 3 + 5)   # "England were" starts at multiples of 402
+
+
+@pytest.mark.parametrize("kind", ["A", "H", "J1"])
+def test_halo_semantics_and_shard_concatenation_detector_sets(kind, monkeypatch):
+    """The same on sets that run a detector kernel: mode 0, global mode, mode 1."""
+    t, ref, text = detector_set(kind, monkeypatch)
+    data = text[:500000]
+    pos, _ = ref(data)
+    check_halo_semantics_and_shard_concatenation(t, ref, data, int(pos[1]) + 1)   # the second match, cut after its first byte
 
 
 def test_dense_matches_and_capacity_overflow():
@@ -170,7 +207,8 @@ def test_dense_matches_and_capacity_overflow():
 def test_candidate_list_boundaries(n_plants):
     """The detector hands a tile's surviving starts to the emit kernel as a list of at most 32
     candidates; beyond that (or when a slice has too many stage-1 survivors) whole slices are handed
-    over.  Plant 1..3000 matches inside one 16,384-byte tile and across its borders."""
+    over.  Plant 1..3000 matches from 300 bytes before byte 32,768 on: across that border between two tiles
+    (of 8,192 starts each) and through the tiles after it."""
     torch = torch_cuda()
     pats = synth.synth_patterns(1, 3000, 3, 4, 64)
     lines = pats.split(b"\n")[:-1]
