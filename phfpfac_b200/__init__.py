@@ -38,6 +38,25 @@ def _as_u8(data):
     return np.frombuffer(bytes(data), dtype=np.uint8)
 
 
+def _until_fits(scan, cap):
+    """scan(cap) -> (rc, count, buffers), called again with cap = count while the records do not fit
+    (PFAC_ERR_OUTPUT_FULL: count is then the capacity they need).  -> (buffers, count) of the call that fit."""
+    while True:
+        rc, count, bufs = scan(cap)
+        if rc != PFAC_ERR_OUTPUT_FULL:
+            check(rc)
+            return bufs, count
+        cap = count
+
+
+def _records(out, n):
+    """The first n records of an int32 [cap, 2] torch device buffer as a MATCH_DTYPE array."""
+    rec = out[:n].cpu().numpy().astype(np.uint32).reshape(-1, 2)
+    res = np.zeros(n, dtype=MATCH_DTYPE)
+    res["pos"], res["id"] = rec[:, 0], rec[:, 1]
+    return res
+
+
 def _arr(ptr, n):
     if n <= 0 or not ptr:
         return np.zeros(0, dtype=np.int32)
@@ -213,7 +232,8 @@ class Matcher:
         n_valid = total if n_valid is None else n_valid
         n_starts = n_valid if n_starts is None else n_starts
         cap = max(1024, n_starts // 8) if cap is None else cap
-        while True:
+
+        def scan(cap):
             out = torch.empty((max(cap, 1), 2), dtype=torch.int32, device=t_in.device)
             cnt = C.c_uint64(0)
             # on torch's current stream: ordered after whatever produced t_in (and allocated `out`) there
@@ -222,14 +242,10 @@ class Matcher:
                 torch.cuda.current_stream(t_in.device).synchronize()
             rc = lib.pfac_scan_device_sync(self._h, t_in.data_ptr() + offset, n_starts, n_valid, base_pos,
                                            out.data_ptr(), cap, C.byref(cnt), stream or None)
-            if rc == PFAC_ERR_OUTPUT_FULL:
-                cap = cnt.value
-                continue
-            check(rc)
-            rec = out[:cnt.value].cpu().numpy().astype(np.uint32).reshape(-1, 2)
-            res = np.zeros(cnt.value, dtype=MATCH_DTYPE)
-            res["pos"], res["id"] = rec[:, 0], rec[:, 1]
-            return res
+            return rc, cnt.value, out
+
+        out, n = _until_fits(scan, cap)
+        return _records(out, n)
 
     # -- many independent documents packed back to back: one launch sequence, per-document results
     def scan_batch(self, values, offsets, cap=None, offset=0):
@@ -250,7 +266,8 @@ class Matcher:
         n_docs = len(offs) - 1
         cap = max(1024, int(offs[-1]) // 8) if cap is None else cap
         stream = torch.cuda.current_stream(values.device).cuda_stream
-        while True:
+
+        def scan(cap):
             out = torch.empty((max(cap, 1), 2), dtype=torch.int32, device=values.device)
             first = torch.empty(n_docs + 1, dtype=torch.int64, device=values.device)
             cnt = C.c_uint64(0)
@@ -259,14 +276,10 @@ class Matcher:
             rc = lib.pfac_scan_batch_device_sync(self._h, values.data_ptr() + offset if values.numel() else None,
                                                  offs.ctypes.data, n_docs, out.data_ptr(), cap, first.data_ptr(),
                                                  C.byref(cnt), stream or None)
-            if rc == PFAC_ERR_OUTPUT_FULL:
-                cap = cnt.value
-                continue
-            check(rc)
-            rec = out[:cnt.value].cpu().numpy().astype(np.uint32).reshape(-1, 2)
-            res = np.zeros(cnt.value, dtype=MATCH_DTYPE)
-            res["pos"], res["id"] = rec[:, 0], rec[:, 1]
-            return first.cpu().numpy().view(np.uint64), res
+            return rc, cnt.value, (out, first)
+
+        (out, first), n = _until_fits(scan, cap)
+        return first.cpu().numpy().view(np.uint64), _records(out, n)
 
     def scan_docs(self, docs):
         """docs: list of bytes-like documents -> list of per-document MATCH_DTYPE arrays (one batch scan)."""
@@ -283,16 +296,16 @@ class Matcher:
         n_valid = len(buf)
         n_starts = n_valid if n_starts is None else n_starts
         cap = max(1024, n_starts // 8) if cap is None else cap
-        while True:
+
+        def scan(cap):
             out = np.zeros(max(cap, 1), dtype=MATCH_DTYPE)
             cnt = C.c_uint64(0)
             rc = lib.pfac_scan_host(self._h, buf.ctypes.data if len(buf) else None, n_starts, n_valid, base_pos,
                                     out.ctypes.data, cap, C.byref(cnt))
-            if rc == PFAC_ERR_OUTPUT_FULL:
-                cap = cnt.value
-                continue
-            check(rc)
-            return out[:cnt.value]
+            return rc, cnt.value, out
+
+        out, n = _until_fits(scan, cap)
+        return out[:n]
 
 
 class Job:

@@ -25,44 +25,114 @@ using namespace pfac;
 
 namespace {
 
+// cap() elements of T in device memory (Host: pinned host memory), owned: the destructor frees them.  Every
+// buffer of this file is one of these.
+template <typename T, bool Host = false>
+class Buf {
+public:
+    Buf() = default;
+    Buf(const Buf &) = delete;
+    Buf &operator=(const Buf &) = delete;
+    ~Buf() { release(); }
+    T *get() const { return p_; }
+    size_t cap() const { return cap_; }
+    size_t bytes() const { return cap_ * sizeof(T); }
+
+    // n elements in place of the old ones, which nothing may still use; zero: filled with zero bytes.  On
+    // failure the buffer is left empty.
+    int alloc(size_t n, bool zero = false)
+    {
+        release();
+        void *p = nullptr;
+        const size_t b = n * sizeof(T);
+        cudaError_t e = Host ? cudaHostAlloc(&p, b, cudaHostAllocPortable) : cudaMalloc(&p, b);
+        if (e == cudaSuccess) {
+            p_ = static_cast<T *>(p);
+            if (zero) e = cudaMemset(p, 0, b);
+        }
+        if (e != cudaSuccess) {
+            release();
+            return set_error(PFAC_ERR_CUDA, "%s(%zu bytes) failed: %s", Host ? "cudaHostAlloc" : "cudaMalloc", b,
+                             cudaGetErrorString(e));
+        }
+        cap_ = n;
+        return PFAC_OK;
+    }
+    // At least n elements (a growth allocates max(n, floor)).  Growing synchronises `stream` first: the old
+    // buffer may still be in use there.  Steady-state calls return at once.
+    int reserve(size_t n, size_t floor, cudaStream_t stream, bool zero = false)
+    {
+        if (n <= cap_) return PFAC_OK;
+        CU_TRY(cudaStreamSynchronize(stream));
+        return alloc(std::max(n, floor), zero);
+    }
+    // a device copy of v
+    int upload(const std::vector<T> &v)
+    {
+        int e = alloc(v.size());
+        if (e) return e;
+        CU_TRY(cudaMemcpy(p_, v.data(), bytes(), cudaMemcpyHostToDevice));
+        return PFAC_OK;
+    }
+
+private:
+    void release()
+    {
+        if (p_) Host ? cudaFreeHost(p_) : cudaFree(p_);
+        p_ = nullptr;
+        cap_ = 0;
+    }
+    T *p_ = nullptr;
+    size_t cap_ = 0;
+};
+
 // Everything one in-flight scan needs besides the tables: control block, result block, tile
 // directory and the arrival-order scratch.  One per user of a stream (the context's own slot for
 // pfac_scan_device, one per pipeline stage for pfac_scan_host).
 struct Slot {
-    Ctrl *d_ctrl = nullptr;
-    Result *d_result = nullptr;
-    Result *h_result = nullptr;   // pinned
+    Buf<Ctrl> d_ctrl;
+    Buf<Result> d_result;
+    Buf<Result, true> h_result;
     // [2][kMaxParts] matches per tile range (walks -> ordering pass).  Two buffers, alternating per scan:
     // the walks of a scan add to one while its detector zeroes the other for the next scan (a buffer
     // zeroed at the start of the scan that uses it would race with the first walks)
-    unsigned long long *d_partial = nullptr;
+    Buf<unsigned long long> d_partial;
     unsigned flip = 0;
-    unsigned int *d_tile_cnt = nullptr, *d_tile_nc = nullptr;
-    unsigned long long *d_tile_src = nullptr;
-    size_t tile_cap = 0;
-    uint2 *d_scratch = nullptr;
-    size_t scratch_cap = 0;   // records
+    Buf<unsigned int> d_tile_cnt, d_tile_nc;
+    Buf<unsigned long long> d_tile_src;
+    Buf<uint2> d_scratch;
     bool dirty = false;       // a launch sequence failed half way: the control block is reset before the next scan
-    // batch scans (pfac_batch.cuh): raw records of the packed buffer and the global positions of the kept ones
-    // (raw_cap each), the document offsets (pinned staging + device copy, doc_cap entries; doc_copied = end of
-    // the last upload from the staging buffer) and the split pass's per-CTA counts
-    uint2 *d_raw = nullptr;
-    uint32_t *d_kpos = nullptr;
-    size_t raw_cap = 0;
-    uint32_t *h_doc = nullptr, *d_doc = nullptr;
-    size_t doc_cap = 0;
+    // batch scans (pfac_batch.cuh): raw records of the packed buffer and the global positions of the kept ones,
+    // the document offsets (pinned staging + device copy; doc_copied = end of the last upload from the staging
+    // buffer) and the split pass's per-CTA counts
+    Buf<uint2> d_raw;
+    Buf<uint32_t> d_kpos;
+    Buf<uint32_t, true> h_doc;
+    Buf<uint32_t> d_doc;
     cudaEvent_t doc_copied = nullptr;
-    unsigned long long *d_blk = nullptr;
+    Buf<unsigned long long> d_blk;
+    ~Slot()
+    {
+        if (doc_copied) cudaEventDestroy(doc_copied);
+    }
 };
 
 struct Stage {   // one pipeline stage of pfac_scan_host
     cudaStream_t stream = nullptr;
-    uint8_t *d_in = nullptr;
-    size_t d_in_cap = 0;
-    pfac_match *d_out = nullptr;
-    size_t d_out_cap = 0;   // records
+    Buf<uint8_t> d_in;
+    Buf<pfac_match> d_out;
     Slot slot;
     cudaEvent_t done = nullptr;
+    ~Stage()
+    {
+        if (done) cudaEventDestroy(done);
+        if (stream) cudaStreamDestroy(stream);
+    }
+};
+
+// What a call enqueued: the counters of pfac_ctx_last_scan_info
+struct Counters {
+    uint64_t launches = 0, tiles = 0, ctas = 0, h2d = 0, d2h = 0, chunks = 1;
 };
 
 }  // namespace
@@ -73,38 +143,38 @@ struct pfac_ctx {
     int n_streams = 1;
     size_t chunk_bytes = 0;
     // tables (device): canonical s0Table, r, {HT, val}, idmap + the detector's shared-memory image
-    int32_t *d_r = nullptr, *d_idmap = nullptr, *d_s0 = nullptr;
-    int2 *d_htval = nullptr;
-    int4 *d_step = nullptr;    // {HT, val, r[row of val]}: the candidate walks' one-load layout (PHF width >= 256)
-    int2 *d_s0r = nullptr;     // {s0Table[b], r[row of it]}
-    uint8_t *d_patdir = nullptr;   // pattern directory of the candidate walks (pfac_derive.h PatDir); null: none
-    PatDir pd;                     // its layout (the image bytes are dropped after the upload)
-    uint4 *d_image = nullptr;
-    uint8_t *d_gimage = nullptr;   // mode 2: T1 | Tm | Tm2 | T3 in global memory
-    uint8_t *d_wcache = nullptr;   // walk cache of the dense-match kernel (pfac_derive.h)
-    WalkCache wc;                  // its layout (the image bytes are dropped after the upload)
-    uint32_t wc_bytes = 0;
+    Buf<int32_t> d_r, d_idmap, d_s0;
+    Buf<int2> d_htval;
+    Buf<int4> d_step;       // {HT, val, r[row of val]}: the candidate walks' one-load layout (PHF width >= 256)
+    Buf<int2> d_s0r;        // {s0Table[b], r[row of it]}
+    Buf<uint8_t> d_patdir;  // pattern directory of the candidate walks (pfac_derive.h PatDir); empty: none
+    Buf<uint8_t> d_image;
+    Buf<uint8_t> d_gimage;  // mode 2: T1 | Tm | Tm2 | T3 in global memory
+    Buf<uint8_t> d_wcache;  // walk cache of the dense-match kernel (pfac_derive.h)
     size_t dense_smem = 0;
     bool dense_first = false;      // no detector: the dense-match kernel walks every tile (sets with patterns <= 3 bytes)
     // batch scans: pattern length of every id; batch_rc != PFAC_OK: the set does not support them (batch_why)
-    int32_t *d_patlen = nullptr;
+    Buf<int32_t> d_patlen;
     uint32_t n_ids = 0;
     int batch_rc = PFAC_OK;
     std::string batch_why;
     Derived dv;   // image layout and hash parameters (the image bytes are dropped after the upload)
     uint32_t image_bytes = 0;
-    int32_t ht_size = 0, width_bit = 0, n_final = 0, max_pat_len = 0;
+    int32_t max_pat_len = 0;
     uint32_t halo = 16;
     uint32_t n_stages = 0;
     size_t smem_bytes = 0;
-    size_t table_bytes = 0;
+    // the per-context part of every scan's kernel parameters (tables, image layout, walk cache); launch_scan
+    // copies them and sets the per-scan fields
+    ScanParams scan;
+    DenseParams dense;
     // pfac_scan_device: own stream and slot
     cudaStream_t own_stream = nullptr;
-    Slot own;                          // working set of pfac_scan_device[_sync]
+    Slot own;                          // working set of pfac_scan_device[_sync] and pfac_scan_batch_device[_sync]
     cudaEvent_t own_done = nullptr;    // end of the last device scan; a call on another stream waits for it
     cudaStream_t own_last = nullptr;
     bool own_used = false;
-    std::vector<Stage> stages;
+    std::unique_ptr<Stage[]> stages;   // [n_streams], set up by the first pfac_scan_host that uses them
     uint64_t info[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     // optional CUDA-event timing of the detector kernel alone (bench.py's roofline leg)
     bool timing = false;
@@ -113,6 +183,12 @@ struct pfac_ctx {
     uint32_t debug = 0;   // PFAC_DEBUG env (timing experiments only)
     bool use_pdl = true;  // PFAC_NO_PDL=1: plain stream-ordered launches (timing experiments only)
     std::mutex mu;
+
+    size_t table_bytes() const
+    {
+        return d_r.bytes() + d_idmap.bytes() + d_s0.bytes() + d_htval.bytes() + d_step.bytes() + d_s0r.bytes() +
+               d_patdir.bytes() + d_image.bytes() + d_gimage.bytes() + d_wcache.bytes() + d_patlen.bytes();
+    }
 };
 
 namespace {
@@ -131,73 +207,81 @@ struct DeviceGuard {
     }
 };
 
-int slot_init(Slot &s)
+// The detector kernels: mode 2 (global tables), mode 1 (T1 + T2), and mode 0 (pfac_scan2_kernel<HAS_SHORT, HAS_SC,
+// W3>) with patterns of <= 3 bytes, then with or without patterns of 4 bytes (ShortC) and the third window.
+using DetectorKernel = void (*)(ScanParams);
+const DetectorKernel kDetectors[7] = {
+    pfac_scan_kernel<2>,
+    pfac_scan_kernel<1>,
+    pfac_scan2_kernel<true, true, false>,
+    pfac_scan2_kernel<false, true, true>,
+    pfac_scan2_kernel<false, true, false>,
+    pfac_scan2_kernel<false, false, true>,
+    pfac_scan2_kernel<false, false, false>,
+};
+
+// The detector kernel a context's derived tables select (unless the dense-match kernel runs alone: dense_first)
+DetectorKernel detector_kernel(const Derived &d)
 {
-    if (s.d_ctrl) return PFAC_OK;
-    CU_TRY(cudaMalloc(&s.d_ctrl, sizeof(Ctrl)));
-    CU_TRY(cudaMemset(s.d_ctrl, 0, sizeof(Ctrl)));
-    CU_TRY(cudaMalloc(&s.d_result, sizeof(Result)));
-    CU_TRY(cudaMalloc(&s.d_partial, 2 * kMaxParts * sizeof(unsigned long long)));
-    CU_TRY(cudaMemset(s.d_partial, 0, 2 * kMaxParts * sizeof(unsigned long long)));
-    CU_TRY(cudaHostAlloc(&s.h_result, sizeof(Result), cudaHostAllocPortable));
+    if (d.mode == 2) return kDetectors[0];
+    if (d.mode == 1) return kDetectors[1];
+    if (d.has_short) return kDetectors[2];
+    return kDetectors[3 + (d.has_shortc ? 0 : 2) + (d.has_w3 ? 0 : 1)];
+}
+
+// Every kernel of a scan is a programmatic dependent launch: its CTAs are set up (and the detector's filter
+// image is on its way into shared memory) while the kernel before it -- the ordering pass of the previous
+// scan on this stream, for the detector -- still runs; each kernel waits (griddepcontrol.wait) before it
+// touches anything an earlier kernel may write.
+cudaLaunchConfig_t launch_config(const pfac_ctx *ctx, cudaStream_t stream, uint32_t grid, uint32_t block, size_t smem)
+{
+    static cudaLaunchAttribute pdl = [] {
+        cudaLaunchAttribute a = {};
+        a.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        a.val.programmaticStreamSerializationAllowed = 1;
+        return a;
+    }();
+    cudaLaunchConfig_t lc = {};
+    lc.stream = stream;
+    lc.attrs = &pdl;
+    lc.numAttrs = ctx->use_pdl ? 1 : 0;
+    lc.gridDim = dim3(grid);
+    lc.blockDim = dim3(block);
+    lc.dynamicSmemBytes = smem;
+    return lc;
+}
+
+// The device watchdog, then the records against the capacity: *count = r.count unless the watchdog tripped.
+int check_result(const Result &r, uint64_t cap, uint64_t *count)
+{
+    if (r.error_flag) return set_error(PFAC_ERR_INTERNAL, "device watchdog tripped (code %u)", r.error_flag);
+    *count = r.count;
+    if (r.count > cap)
+        return set_error(PFAC_ERR_OUTPUT_FULL, "%llu matches exceed the capacity of %llu records",
+                         (unsigned long long)r.count, (unsigned long long)cap);
     return PFAC_OK;
 }
 
-void slot_free(Slot &s)
+void set_info(pfac_ctx *ctx, const Counters &c)
 {
-    if (s.d_ctrl) cudaFree(s.d_ctrl);
-    if (s.d_result) cudaFree(s.d_result);
-    if (s.d_partial) cudaFree(s.d_partial);
-    if (s.h_result) cudaFreeHost(s.h_result);
-    if (s.d_tile_cnt) cudaFree(s.d_tile_cnt);
-    if (s.d_tile_src) cudaFree(s.d_tile_src);
-    if (s.d_tile_nc) cudaFree(s.d_tile_nc);
-    if (s.d_scratch) cudaFree(s.d_scratch);
-    if (s.d_raw) cudaFree(s.d_raw);
-    if (s.d_kpos) cudaFree(s.d_kpos);
-    if (s.d_doc) cudaFree(s.d_doc);
-    if (s.h_doc) cudaFreeHost(s.h_doc);
-    if (s.doc_copied) cudaEventDestroy(s.doc_copied);
-    if (s.d_blk) cudaFree(s.d_blk);
-    s = Slot();
+    const uint64_t v[8] = {c.launches, c.tiles, c.ctas, ctx->smem_bytes, c.h2d, c.d2h, c.chunks, 0};
+    memcpy(ctx->info, v, sizeof v);
 }
 
-// Grow the tile directory / scratch of a slot.  Growing synchronises the stream first (the old
-// buffers may still be in use); steady-state calls never get here.
-int slot_reserve(Slot &s, size_t n_tiles, size_t records, cudaStream_t stream)
+int slot_init(Slot &s)
 {
-    if (n_tiles > s.tile_cap) {
-        CU_TRY(cudaStreamSynchronize(stream));
-        if (s.d_tile_cnt) cudaFree(s.d_tile_cnt);
-        if (s.d_tile_src) cudaFree(s.d_tile_src);
-        if (s.d_tile_nc) cudaFree(s.d_tile_nc);
-                s.d_tile_cnt = s.d_tile_nc = nullptr;
-        s.d_tile_src = nullptr;
-        s.tile_cap = 0;
-        const size_t n = std::max<size_t>(n_tiles, 1024);
-        CU_TRY(cudaMalloc(&s.d_tile_cnt, n * sizeof(unsigned int)));
-        CU_TRY(cudaMalloc(&s.d_tile_src, n * sizeof(unsigned long long)));
-        CU_TRY(cudaMemset(s.d_tile_src, 0, n * sizeof(unsigned long long)));   // (epoch 0 = never published: DIRECT dense scans)
-        CU_TRY(cudaMalloc(&s.d_tile_nc, n * sizeof(unsigned int)));
-        s.tile_cap = n;
-    }
-    if (records > s.scratch_cap) {
-        CU_TRY(cudaStreamSynchronize(stream));
-        if (s.d_scratch) cudaFree(s.d_scratch);
-        s.d_scratch = nullptr;
-        s.scratch_cap = 0;
-        const size_t n = std::max<size_t>(records, 4096);
-        CU_TRY(cudaMalloc(&s.d_scratch, n * sizeof(uint2)));
-        s.scratch_cap = n;
-    }
+    if (s.h_result.get()) return PFAC_OK;
+    int e;
+    if ((e = s.d_ctrl.alloc(1, true)) || (e = s.d_result.alloc(1)) || (e = s.d_partial.alloc(2 * kMaxParts, true)) ||
+        (e = s.h_result.alloc(1)))
+        return e;
     return PFAC_OK;
 }
 
 // Enqueue one scan (scan kernel + ordering pass) on `stream`.  On completion slot.d_result holds
-// {count, error}; d_count (optional, device) receives the count as well.
+// {count, error}; d_count (optional, device) receives the count as well.  n: launches, tiles and CTAs.
 int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, uint64_t n_valid, uint64_t base_pos,
-                uint32_t pos_bias, void *d_out, uint64_t cap, void *d_count, cudaStream_t stream,
-                uint64_t *tiles_out, uint64_t *ctas_out, uint64_t *launches_out)
+                uint32_t pos_bias, void *d_out, uint64_t cap, void *d_count, cudaStream_t stream, Counters &n)
 {
     if (n_valid < n_starts) return set_error(PFAC_ERR_ARG, "n_valid < n_starts");
     const uint64_t useful = n_starts + (uint64_t)(ctx->max_pat_len > 0 ? ctx->max_pat_len - 1 : 0);
@@ -205,19 +289,16 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
     const uint32_t mis = (uint32_t)((uintptr_t)d_in & 15u);
     if (n_valid + mis + (uint64_t)kTile + 4096 >= (1ull << 32))
         return set_error(PFAC_ERR_LIMIT, "one scan call covers less than 4 GiB; split the input");
-    if (tiles_out) *tiles_out = 0;
-    if (ctas_out) *ctas_out = 0;
-    if (launches_out) *launches_out = 0;
     int e = slot_init(slot);
     if (e) return e;
     if (n_starts == 0 || ctx->max_pat_len == 0) {
-        CU_TRY(cudaMemsetAsync(slot.d_result, 0, sizeof(Result), stream));
+        CU_TRY(cudaMemsetAsync(slot.d_result.get(), 0, sizeof(Result), stream));
         if (d_count) CU_TRY(cudaMemsetAsync(d_count, 0, sizeof(unsigned long long), stream));
         return PFAC_OK;
     }
     if (slot.dirty) {   // a previous launch sequence failed between the kernels: start from a clean control block
-        CU_TRY(cudaMemsetAsync(slot.d_ctrl, 0, sizeof(Ctrl), stream));
-        CU_TRY(cudaMemsetAsync(slot.d_partial, 0, 2 * kMaxParts * sizeof(unsigned long long), stream));
+        CU_TRY(cudaMemsetAsync(slot.d_ctrl.get(), 0, sizeof(Ctrl), stream));
+        CU_TRY(cudaMemsetAsync(slot.d_partial.get(), 0, slot.d_partial.bytes(), stream));
         slot.dirty = false;
     }
     struct DirtyOnError {   // set back to false on the success path
@@ -225,91 +306,47 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
         bool armed = true;
         ~DirtyOnError() { if (armed) s.dirty = true; }
     } guard{slot};
-    ScanParams p;
-    memset(&p, 0, sizeof p);
+    if (ctx->n_stages < (uint32_t)min_stages((int)ctx->dv.mode))
+        return set_error(PFAC_ERR_INTERNAL, "input ring of %u stages is too shallow for the slot scheme", ctx->n_stages);
+    ScanParams p = ctx->scan;
     p.in_al = (const uint8_t *)d_in - mis;
     p.mis = mis;
     p.a_start_end = (uint32_t)(mis + n_starts);
     p.a_valid_end = (uint32_t)(mis + n_valid);
     p.n_tiles = (uint32_t)(((uint64_t)p.a_start_end + kTile - 1) / kTile);
-    p.halo = ctx->halo;
-    p.max_pat_len = (uint32_t)ctx->max_pat_len;
-    p.use_ref_bound = ctx->max_pat_len > kRefHalo + 1;   // only then can the 4096+512 bound cut a walk
     p.base_pos = base_pos;
-    p.image = ctx->d_image;
-    p.image_bytes = ctx->image_bytes;
-    p.off_t2 = ctx->dv.off_t2;
-    p.off_tm = ctx->dv.off_tm;
-    p.off_tm2 = ctx->dv.off_tm2;
-    p.off_t3 = ctx->dv.off_t3;
-    p.t2_shift = ctx->dv.t2_shift;
-    p.has_short = ctx->dv.has_short;
-    p.has_t3 = ctx->dv.has_t3;
-    p.t3_shift = ctx->dv.t3_shift;
-    p.tm_bits = ctx->dv.tm_bits;
-    p.tm2_bits = ctx->dv.tm2_bits;
-    p.off_d1 = ctx->dv.off_d1;
-    p.off_e1 = ctx->dv.off_e1;
-    p.nb1 = ctx->dv.nb1;
-    p.ns1 = ctx->dv.ns1;
-    p.off_d2 = ctx->dv.off_d2;
-    p.off_e2 = ctx->dv.off_e2;
-    p.nb2 = ctx->dv.nb2;
-    p.ns2 = ctx->dv.ns2;
-    p.gimage = ctx->d_gimage;
-    if (ctx->n_stages < (uint32_t)min_stages((int)ctx->dv.mode))
-        return set_error(PFAC_ERR_INTERNAL, "input ring of %u stages is too shallow for the slot scheme", ctx->n_stages);
-    p.n_stages = ctx->n_stages;
-    p.stage_magic = (uint32_t)((1ull << 32) / ctx->n_stages) + 1u;
-    e = slot_reserve(slot, p.n_tiles, (size_t)std::max<uint64_t>(cap, 4096), stream);
-    if (e) return e;
-    p.tile_cnt = slot.d_tile_cnt;
-    p.tile_nc = slot.d_tile_nc;
-    unsigned long long *partial_now = slot.d_partial + (slot.flip & 1u) * kMaxParts;
+    // tile directory and scratch (epoch 0 in tile_src = never published: DIRECT dense scans)
+    if ((e = slot.d_tile_cnt.reserve(p.n_tiles, 1024, stream)) || (e = slot.d_tile_src.reserve(p.n_tiles, 1024, stream, true)) ||
+        (e = slot.d_tile_nc.reserve(p.n_tiles, 1024, stream)) ||
+        (e = slot.d_scratch.reserve((size_t)std::max<uint64_t>(cap, 4096), 4096, stream)))
+        return e;
+    p.tile_cnt = slot.d_tile_cnt.get();
+    p.tile_nc = slot.d_tile_nc.get();
+    unsigned long long *partial_now = slot.d_partial.get() + (slot.flip & 1u) * kMaxParts;
     p.partial = partial_now;
-    p.partial_next = slot.d_partial + ((slot.flip + 1u) & 1u) * kMaxParts;
-    p.ctrl = slot.d_ctrl;
-    p.debug = ctx->debug;
+    p.partial_next = slot.d_partial.get() + ((slot.flip + 1u) & 1u) * kMaxParts;
+    p.ctrl = slot.d_ctrl.get();
     const uint32_t grid = (uint32_t)std::min<uint64_t>(p.n_tiles, (uint64_t)ctx->sm_count);
     // tile ranges of the ordering pass: many small ones, so that dense outputs (every tile a long run
     // of records) are moved by the whole GPU
     const uint32_t fgrid = (uint32_t)std::min<uint64_t>((p.n_tiles + 7) / 8, (uint64_t)kMaxParts);
     const uint32_t tiles_per_part = (p.n_tiles + fgrid - 1) / fgrid;
-    EmitParams ep;
-    memset(&ep, 0, sizeof ep);
+    EmitParams &ep = p.emit;
     ep.in_al = p.in_al;
     ep.mis = p.mis;
     ep.a_start_end = p.a_start_end;
     ep.a_valid_end = p.a_valid_end;
-    ep.max_pat_len = p.max_pat_len;
-    ep.use_ref_bound = p.use_ref_bound;
     ep.base_pos = base_pos;
     ep.pos_bias = pos_bias;
-    ep.r = ctx->d_r;
-    ep.htval = ctx->d_htval;
-    ep.idmap = ctx->d_idmap;
-    ep.s0 = ctx->d_s0;
-    ep.step = ctx->d_step;
-    ep.s0r = ctx->d_s0r;
-    if (ctx->d_patdir) {
-        ep.dir = reinterpret_cast<const uint4 *>(ctx->d_patdir);
-        ep.pool = ctx->d_patdir + ctx->pd.off_pool;
-        ep.dir_slots = ctx->pd.n_slots;
-        ep.len_mask = ctx->pd.len_mask;
-    }
-    ep.ht_size = ctx->ht_size;
-    ep.width_bit = ctx->width_bit;
-    ep.n_final = ctx->n_final;
-    ep.scratch = slot.d_scratch;
-    ep.scratch_cap = slot.scratch_cap;
-    ep.tile_cnt = slot.d_tile_cnt;
-    ep.tile_src = slot.d_tile_src;
-    ep.tile_nc = slot.d_tile_nc;
+    ep.scratch = slot.d_scratch.get();
+    ep.scratch_cap = slot.d_scratch.cap();
+    ep.tile_cnt = slot.d_tile_cnt.get();
+    ep.tile_src = slot.d_tile_src.get();
+    ep.tile_nc = slot.d_tile_nc.get();
     ep.n_tiles = p.n_tiles;
     ep.tiles_per_part = tiles_per_part;
     ep.partial = partial_now;
-    ep.ctrl = slot.d_ctrl;
-    p.emit = ep;
+    ep.ctrl = slot.d_ctrl.get();
 
     p.ticket_batch = std::max<uint32_t>(1u, std::min<uint32_t>((uint32_t)kTicketBatch, p.n_tiles / (4u * grid)));
     cudaEvent_t ev_after = nullptr;
@@ -324,92 +361,49 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
     // match at a large share of the start positions of natural text: no filter pays off, the dense-match
     // kernel walks every tile straight away.
     const bool dense_first = ctx->dense_first;
-    // Every kernel of a scan is a programmatic dependent launch: its CTAs are set up (and the detector's filter
-    // image is on its way into shared memory) while the kernel before it -- the ordering pass of the previous
-    // scan on this stream, for the detector -- still runs; each kernel waits (griddepcontrol.wait) before it
-    // touches anything an earlier kernel may write.
-    cudaLaunchAttribute pdl[1];
-    pdl[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    pdl[0].val.programmaticStreamSerializationAllowed = 1;
-    cudaLaunchConfig_t lc;
-    memset(&lc, 0, sizeof lc);
-    lc.stream = stream;
-    lc.attrs = pdl;
-    lc.numAttrs = ctx->use_pdl ? 1 : 0;
-    lc.gridDim = dim3(grid);
-    lc.blockDim = dim3(kThreads);
-    lc.dynamicSmemBytes = ctx->smem_bytes;
-    if (dense_first) {}
-    else if (ctx->dv.mode == 2) CU_TRY(cudaLaunchKernelEx(&lc, pfac_scan_kernel<2>, p));
-    else if (ctx->dv.mode == 1) CU_TRY(cudaLaunchKernelEx(&lc, pfac_scan_kernel<1>, p));
-    else if (ctx->dv.has_short) CU_TRY(cudaLaunchKernelEx(&lc, pfac_scan2_kernel<true, true, false>, p));
-    else if (ctx->dv.has_shortc && ctx->dv.has_w3) CU_TRY(cudaLaunchKernelEx(&lc, pfac_scan2_kernel<false, true, true>, p));
-    else if (ctx->dv.has_shortc) CU_TRY(cudaLaunchKernelEx(&lc, pfac_scan2_kernel<false, true, false>, p));
-    else if (ctx->dv.has_w3) CU_TRY(cudaLaunchKernelEx(&lc, pfac_scan2_kernel<false, false, true>, p));
-    else CU_TRY(cudaLaunchKernelEx(&lc, pfac_scan2_kernel<false, false, false>, p));
-    if (ev_after && !dense_first) CU_TRY(cudaEventRecord(ev_after, stream));
-
+    if (!dense_first) {
+        const cudaLaunchConfig_t lc = launch_config(ctx, stream, grid, kThreads, ctx->smem_bytes);
+        CU_TRY(cudaLaunchKernelEx(&lc, detector_kernel(ctx->dv), p));
+        if (ev_after) CU_TRY(cudaEventRecord(ev_after, stream));
+    }
 
     // the tiles the detector handed over whole (dense matches); returns at once when there are none
-    DenseParams dp;
-    memset(&dp, 0, sizeof dp);
+    DenseParams dp = ctx->dense;
     dp.e = ep;
-    dp.wc_image = ctx->d_wcache;
-    dp.wc_bytes = ctx->wc_bytes;
-    dp.wc_depth = ctx->wc.depth;
-    dp.wc_off_d = ctx->wc.off_d;
-    dp.wc_off_e = ctx->wc.off_e;
-    dp.wc_nb = ctx->wc.nb;
-    dp.wc_ns = ctx->wc.ns;
-    dp.halo = ctx->halo;
-    dp.n_dense = &slot.d_ctrl->n_dense;
+    dp.n_dense = &slot.d_ctrl.get()->n_dense;
+    const cudaLaunchConfig_t dl = launch_config(ctx, stream, grid, kDenseThreads, ctx->dense_smem);
     if (dense_first) {   // the dense-match kernel is the whole scan: records go straight to the caller's buffer
         dp.out = (uint2 *)d_out;
         dp.cap = cap;
-        dp.prefix = slot.d_tile_src;
+        dp.prefix = slot.d_tile_src.get();
         dp.epoch = slot.flip % 0xFFFFFEu + 1u;
-        dp.result = slot.d_result;
+        dp.result = slot.d_result.get();
         dp.count_out = (unsigned long long *)d_count;
-        lc.gridDim = dim3(grid);
-        lc.blockDim = dim3(kDenseThreads);
-        lc.dynamicSmemBytes = ctx->dense_smem;
-        CU_TRY(cudaLaunchKernelEx(&lc, pfac_dense_kernel<true>, dp));
+        CU_TRY(cudaLaunchKernelEx(&dl, pfac_dense_kernel<true>, dp));
         if (ev_after) CU_TRY(cudaEventRecord(ev_after, stream));
-        if (tiles_out) *tiles_out = p.n_tiles;
-        if (ctas_out) *ctas_out = grid;
-        if (launches_out) *launches_out = 1;
-        slot.flip++;
-        guard.armed = false;
-        return PFAC_OK;
+    } else {   // dense-match pass and ordering pass
+        CU_TRY(cudaLaunchKernelEx(&dl, pfac_dense_kernel<false>, dp));
+        FinalizeParams f;
+        f.tile_cnt = slot.d_tile_cnt.get();
+        f.tile_src = slot.d_tile_src.get();
+        f.scratch = slot.d_scratch.get();
+        f.scratch_cap = slot.d_scratch.cap();
+        f.out = (uint2 *)d_out;
+        f.cap = cap;
+        f.n_tiles = p.n_tiles;
+        f.tiles_per_part = tiles_per_part;
+        f.partial = partial_now;
+        f.ctrl = slot.d_ctrl.get();
+        f.result = slot.d_result.get();
+        f.count_out = (unsigned long long *)d_count;
+        f.debug = ctx->debug;
+        f.trace_ctas = grid;
+        const cudaLaunchConfig_t fl = launch_config(ctx, stream, fgrid, kFinThreads, 0);
+        CU_TRY(cudaLaunchKernelEx(&fl, pfac_finalize_kernel, f));
     }
-    // dense-match pass and ordering pass
-    lc.gridDim = dim3(grid);
-    lc.blockDim = dim3(kDenseThreads);
-    lc.dynamicSmemBytes = ctx->dense_smem;
-    CU_TRY(cudaLaunchKernelEx(&lc, pfac_dense_kernel<false>, dp));
-
-    FinalizeParams f;
-    f.tile_cnt = slot.d_tile_cnt;
-    f.tile_src = slot.d_tile_src;
-    f.scratch = slot.d_scratch;
-    f.scratch_cap = slot.scratch_cap;
-    f.out = (uint2 *)d_out;
-    f.cap = cap;
-    f.n_tiles = p.n_tiles;
-    f.tiles_per_part = tiles_per_part;
-    f.partial = partial_now;
-    f.ctrl = slot.d_ctrl;
-    f.result = slot.d_result;
-    f.count_out = (unsigned long long *)d_count;
-    f.debug = ctx->debug;
-    f.trace_ctas = grid;
-    lc.gridDim = dim3(fgrid);
-    lc.blockDim = dim3(kFinThreads);
-    lc.dynamicSmemBytes = 0;
-    CU_TRY(cudaLaunchKernelEx(&lc, pfac_finalize_kernel, f));
-    if (tiles_out) *tiles_out = p.n_tiles;
-    if (ctas_out) *ctas_out = grid;
-    if (launches_out) *launches_out = 3;
+    n.launches = dense_first ? 1 : 3;
+    n.tiles = p.n_tiles;
+    n.ctas = grid;
     slot.flip++;
     guard.armed = false;
     return PFAC_OK;
@@ -417,9 +411,9 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
 
 // Enqueue a batch scan on `stream` (pfac_batch.cuh): the documents' offsets are uploaded, the packed buffer is
 // scanned into the slot's raw-record buffer, the split pass writes the caller's records, d_doc_first and
-// d_count.  On completion slot.d_result holds {count, error}.  info: the counters of pfac_ctx_last_scan_info.
+// d_count.  On completion slot.d_result holds {count, error}.
 int launch_batch(pfac_ctx *ctx, Slot &slot, const void *d_in, const uint64_t *doc_offsets, uint32_t n_docs,
-                 void *d_out, uint64_t cap, void *d_doc_first, void *d_count, cudaStream_t stream, uint64_t info[8])
+                 void *d_out, uint64_t cap, void *d_doc_first, void *d_count, cudaStream_t stream, Counters &n)
 {
     if (ctx->batch_rc != PFAC_OK) return set_error(ctx->batch_rc, "%s", ctx->batch_why.c_str());
     if (n_docs == 0xFFFFFFFFu) return set_error(PFAC_ERR_LIMIT, "a batch holds fewer than 2^32 - 1 documents");
@@ -431,33 +425,13 @@ int launch_batch(pfac_ctx *ctx, Slot &slot, const void *d_in, const uint64_t *do
     int e = slot_init(slot);
     if (e) return e;
     const uint32_t grid = 2u * (uint32_t)ctx->sm_count;   // CTAs of the count and split kernels
-    if (!slot.d_blk) CU_TRY(cudaMalloc(&slot.d_blk, (grid + 1) * sizeof(unsigned long long)));
+    if (!slot.d_blk.get() && (e = slot.d_blk.alloc(grid + 1))) return e;
     if (!slot.doc_copied) CU_TRY(cudaEventCreateWithFlags(&slot.doc_copied, cudaEventDisableTiming));
-    // grow the offset and raw-record buffers (synchronises the stream first: the old ones may still be in use)
     const size_t n_off = (size_t)n_docs + 1;
-    if (n_off > slot.doc_cap) {
-        CU_TRY(cudaStreamSynchronize(stream));
-        if (slot.d_doc) cudaFree(slot.d_doc);
-        if (slot.h_doc) cudaFreeHost(slot.h_doc);
-        slot.d_doc = slot.h_doc = nullptr;
-        slot.doc_cap = 0;
-        const size_t n = std::max<size_t>(n_off, 4096);
-        CU_TRY(cudaMalloc(&slot.d_doc, n * sizeof(uint32_t)));
-        CU_TRY(cudaHostAlloc(&slot.h_doc, n * sizeof(uint32_t), cudaHostAllocPortable));
-        slot.doc_cap = n;
-    }
     const size_t want = (size_t)std::max<uint64_t>(cap, 4096);
-    if (want > slot.raw_cap) {
-        CU_TRY(cudaStreamSynchronize(stream));
-        if (slot.d_raw) cudaFree(slot.d_raw);
-        if (slot.d_kpos) cudaFree(slot.d_kpos);
-        slot.d_raw = nullptr;
-        slot.d_kpos = nullptr;
-        slot.raw_cap = 0;
-        CU_TRY(cudaMalloc(&slot.d_raw, want * sizeof(uint2)));
-        CU_TRY(cudaMalloc(&slot.d_kpos, want * sizeof(uint32_t)));
-        slot.raw_cap = want;
-    }
+    if ((e = slot.d_doc.reserve(n_off, 4096, stream)) || (e = slot.h_doc.reserve(n_off, 4096, stream)) ||
+        (e = slot.d_raw.reserve(want, want, stream)) || (e = slot.d_kpos.reserve(want, want, stream)))
+        return e;
     // offsets -> pinned staging once the previous upload from it is done, checked on the way (32 bits suffice:
     // total < 4 GiB) -> device
     CU_TRY(cudaEventSynchronize(slot.doc_copied));
@@ -467,63 +441,245 @@ int launch_batch(pfac_ctx *ctx, Slot &slot, const void *d_in, const uint64_t *do
         const uint64_t v = doc_offsets[i];
         decreasing |= v < prev;
         prev = v;
-        slot.h_doc[i] = (uint32_t)v;
+        slot.h_doc.get()[i] = (uint32_t)v;
     }
     if (decreasing) return set_error(PFAC_ERR_ARG, "doc_offsets decrease");
-    CU_TRY(cudaMemcpyAsync(slot.d_doc, slot.h_doc, n_off * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+    CU_TRY(cudaMemcpyAsync(slot.d_doc.get(), slot.h_doc.get(), n_off * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
     CU_TRY(cudaEventRecord(slot.doc_copied, stream));
 
-    uint64_t tiles = 0, ctas = 0, launches = 0;
-    e = launch_scan(ctx, slot, d_in, total, total, 0, 0u, slot.d_raw, slot.raw_cap, nullptr, stream, &tiles, &ctas,
-                    &launches);
+    e = launch_scan(ctx, slot, d_in, total, total, 0, 0u, slot.d_raw.get(), slot.d_raw.cap(), nullptr, stream, n);
     if (e) return e;
     BatchParams bp;
     memset(&bp, 0, sizeof bp);
-    bp.raw = slot.d_raw;
-    bp.raw_cap = slot.raw_cap;
-    bp.doc = slot.d_doc;
+    bp.raw = slot.d_raw.get();
+    bp.raw_cap = slot.d_raw.cap();
+    bp.doc = slot.d_doc.get();
     bp.n_docs = n_docs;
-    bp.len = ctx->d_patlen;
+    bp.len = ctx->d_patlen.get();
     bp.n_ids = ctx->n_ids;
-    bp.blk = slot.d_blk;
+    bp.blk = slot.d_blk.get();
     bp.out = (uint2 *)d_out;
     bp.cap = cap;
-    bp.kpos = slot.d_kpos;
+    bp.kpos = slot.d_kpos.get();
     bp.doc_first = (unsigned long long *)d_doc_first;
-    bp.result = slot.d_result;
+    bp.result = slot.d_result.get();
     bp.count_out = (unsigned long long *)d_count;
-    cudaLaunchAttribute pdl[1];
-    pdl[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    pdl[0].val.programmaticStreamSerializationAllowed = 1;
-    cudaLaunchConfig_t lc = {};
-    lc.stream = stream;
-    lc.attrs = pdl;
-    lc.numAttrs = ctx->use_pdl ? 1 : 0;
-    lc.blockDim = dim3(kBatchThreads);
-    lc.gridDim = dim3(grid);
+    const cudaLaunchConfig_t lc = launch_config(ctx, stream, grid, kBatchThreads, 0);
     CU_TRY(cudaLaunchKernelEx(&lc, pfac_batch_count_kernel, bp));
     CU_TRY(cudaLaunchKernelEx(&lc, pfac_batch_split_kernel, bp));
-    lc.gridDim = dim3((uint32_t)std::min<uint64_t>((n_off + kBatchThreads - 1) / kBatchThreads, grid));
-    CU_TRY(cudaLaunchKernelEx(&lc, pfac_batch_docs_kernel, bp));
-    info[0] = launches + 3;
-    info[1] = tiles;
-    info[2] = ctas;
-    info[3] = ctx->smem_bytes;
-    info[4] = n_off * sizeof(uint32_t);
-    info[5] = 0;
-    info[6] = 1;
-    info[7] = 0;
+    const cudaLaunchConfig_t dl =
+        launch_config(ctx, stream, (uint32_t)std::min<uint64_t>((n_off + kBatchThreads - 1) / kBatchThreads, grid), kBatchThreads, 0);
+    CU_TRY(cudaLaunchKernelEx(&dl, pfac_batch_docs_kernel, bp));
+    n.launches += 3;
+    n.h2d = n_off * sizeof(uint32_t);
     return PFAC_OK;
 }
 
-void free_stage(Stage &s)
+// The four entry points that scan into the context's own slot.  `launch(stream, counters)` enqueues the scan.
+// With `count` (the _sync forms) the Result block is read back and the stream synchronised, then the records
+// are checked against `cap`.  Device scans of one context share the slot: a scan enqueued on another stream
+// than the one before it is ordered after it (own_done).
+template <typename Launch>
+int run_own(pfac_ctx *ctx, void *stream, uint64_t cap, uint64_t *count, Launch &&launch)
 {
-    if (s.d_in) cudaFree(s.d_in);
-    if (s.d_out) cudaFree(s.d_out);
-    slot_free(s.slot);
-    if (s.done) cudaEventDestroy(s.done);
-    if (s.stream) cudaStreamDestroy(s.stream);
-    s = Stage();
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DeviceGuard g(ctx->device);
+    const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
+    if (ctx->own_used && ctx->own_last != st) CU_TRY(cudaStreamWaitEvent(st, ctx->own_done, 0));
+    Counters n;
+    int e = launch(st, n);
+    if (e) return e;
+    Slot &s = ctx->own;
+    if (count) CU_TRY(cudaMemcpyAsync(s.h_result.get(), s.d_result.get(), sizeof(Result), cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaEventRecord(ctx->own_done, st));
+    ctx->own_last = st;
+    ctx->own_used = true;
+    if (count) CU_TRY(cudaStreamSynchronize(st));
+    set_info(ctx, n);
+    return count ? check_result(*s.h_result.get(), cap, count) : PFAC_OK;
+}
+
+// shared-memory budget: T1 and the per-warp queues are fixed; T3 / Tm2 / T2 shrink until at least
+// four ring stages fit
+int size_shared_memory(pfac_ctx &ctx, const Partition &P, size_t smem_max)
+{
+    uint32_t t2_bytes = 32768, t3_bytes = 32768, tm2_bytes = 32768;
+    if (const char *v = getenv("PFAC_T2_BYTES")) t2_bytes = (uint32_t)atoi(v);
+    if (const char *v = getenv("PFAC_T3_BYTES")) t3_bytes = (uint32_t)atoi(v);
+    if (const char *v = getenv("PFAC_TM2_BYTES")) tm2_bytes = (uint32_t)atoi(v);
+    bool widened = false;
+    while (true) {
+        derive_tables(P, t2_bytes, t3_bytes, tm2_bytes, ctx.dv);
+        if (ctx.dv.mode == 2 && !widened && !getenv("PFAC_T2_BYTES")) {
+            // global mode: T2 is stage 1 and the only shared-memory table -- give it all the room
+            widened = true;
+            t2_bytes = 131072;
+            continue;
+        }
+        ctx.image_bytes = (uint32_t)ctx.dv.image.size();
+        const size_t fixed = scan_smem_bytes(ctx.image_bytes, ctx.halo, 0, ctx.dv.mode);
+        const size_t stride = scan_buf_stride(ctx.halo);
+        const size_t fit = smem_max > fixed ? (smem_max - fixed) / stride : 0;
+        const bool minimal = t2_bytes < 2048 && (ctx.dv.mode == 2 || (t3_bytes < 2048 && tm2_bytes < 2048));
+        const size_t need = (size_t)min_stages((int)ctx.dv.mode);   // 2 (shared-memory mode) or 4 (global mode)
+        // mode 0 wants a deep ring (bytes in flight hide the HBM latency): T3 gives way down to 16 KiB
+        const bool deepen = ctx.dv.mode == 0 && fit < 9 && t3_bytes > 16384 && !getenv("PFAC_T3_BYTES");
+        if (!deepen && (fit >= std::max<size_t>(3, need) || (fit >= need && minimal))) {
+            ctx.n_stages = (uint32_t)std::min<size_t>(fit, kMaxStages);
+            if (const char *v = getenv("PFAC_RING_STAGES"))   // tests: a ring as shallow as the slot scheme allows
+                ctx.n_stages = (uint32_t)std::max<size_t>(need, std::min<size_t>(ctx.n_stages, (size_t)atoi(v)));
+            ctx.smem_bytes = scan_smem_bytes(ctx.image_bytes, ctx.halo, ctx.n_stages, ctx.dv.mode);
+            return PFAC_OK;
+        }
+        if (minimal)
+            return set_error(PFAC_ERR_CUDA, "scan kernel needs more than the %zu B of shared memory the device offers",
+                             smem_max);
+        // halve the largest section that is actually in the image
+        if (ctx.dv.mode == 2) {
+            t2_bytes /= 2;
+        } else if (ctx.dv.has_t3) {
+            if (t3_bytes > 8192) t3_bytes /= 2;          // T3 first: it only gets a little less selective
+            else if (tm2_bytes >= 2048) tm2_bytes /= 2;  // then level 2 (all or nothing per size)
+            else t3_bytes /= 2;
+        } else {
+            t3_bytes = tm2_bytes = 0;
+            t2_bytes /= 2;
+        }
+    }
+}
+
+// canonical arrays -> device, unchanged: s0Table, r, {HT, val} interleaved, idmap; + the detector images, the
+// walks' one-load layout and the pattern directory.  Fills the per-context part of ctx.scan.
+int upload_tables(pfac_ctx &ctx, const Partition &P)
+{
+    const size_t n_ht = std::max<size_t>((size_t)P.ht_size, 1);
+    std::vector<int32_t> r(P.r), idmap(std::max<size_t>((size_t)P.n_final, 1), 0), s0(256, -1);
+    r.resize(std::max<size_t>(P.r.size(), 1), -1);
+    std::copy_n(P.idmap.begin(), (size_t)P.n_final, idmap.begin());
+    if (!P.s0.empty()) std::copy_n(P.s0.begin(), 256, s0.begin());
+    std::vector<int2> htval(n_ht, make_int2(-1, -1));
+    for (int32_t i = 0; i < P.ht_size; i++) htval[(size_t)i] = make_int2(P.HT[(size_t)i], P.val[(size_t)i]);
+    int e;
+    if ((e = ctx.d_r.upload(r)) || (e = ctx.d_htval.upload(htval)) || (e = ctx.d_idmap.upload(idmap)) ||
+        (e = ctx.d_s0.upload(s0)) || (e = ctx.d_image.upload(ctx.dv.image)))
+        return e;
+    const int width_bit = width_bits(P.width);
+    if (width_bit >= 8 && !P.r.empty()) {
+        // the one-load layout of the candidate walks: the row of a state's transitions depends on the state
+        // alone when a row holds at least 256 keys, so every entry can carry its successor's r[] value
+        const int sh = width_bit - 8;
+        auto r_of = [&](int32_t state) -> int32_t {
+            const size_t row = (size_t)state >> sh;
+            return state >= 0 && row < P.r.size() ? P.r[row] : -1;
+        };
+        std::vector<int4> step(n_ht, make_int4(-1, -1, -1, 0));
+        for (int32_t i = 0; i < P.ht_size; i++) step[(size_t)i] = make_int4(P.HT[(size_t)i], P.val[(size_t)i], r_of(P.val[(size_t)i]), 0);
+        std::vector<int2> s0r(256);
+        for (int b = 0; b < 256; b++) s0r[(size_t)b] = make_int2(s0[(size_t)b], r_of(s0[(size_t)b]));
+        if ((e = ctx.d_step.upload(step)) || (e = ctx.d_s0r.upload(s0r))) return e;
+    }
+    PatDir pd;
+    if (!getenv("PFAC_NO_PATDIR")) derive_patdir(P, pd);
+    if (pd.n_slots && (e = ctx.d_patdir.upload(pd.image))) return e;
+    if (!ctx.dv.gimage.empty() && (e = ctx.d_gimage.upload(ctx.dv.gimage))) return e;
+
+    const Derived &d = ctx.dv;
+    ScanParams &p = ctx.scan;
+    memset(&p, 0, sizeof p);
+    p.halo = ctx.halo;
+    p.max_pat_len = (uint32_t)ctx.max_pat_len;
+    p.use_ref_bound = ctx.max_pat_len > kRefHalo + 1;   // only then can the 4096+512 bound cut a walk
+    p.image = reinterpret_cast<const uint4 *>(ctx.d_image.get());
+    p.image_bytes = ctx.image_bytes;
+    p.off_t2 = d.off_t2;
+    p.off_tm = d.off_tm;
+    p.off_tm2 = d.off_tm2;
+    p.off_t3 = d.off_t3;
+    p.t2_shift = d.t2_shift;
+    p.has_short = d.has_short;
+    p.has_t3 = d.has_t3;
+    p.t3_shift = d.t3_shift;
+    p.tm_bits = d.tm_bits;
+    p.tm2_bits = d.tm2_bits;
+    p.off_d1 = d.off_d1;
+    p.off_e1 = d.off_e1;
+    p.nb1 = d.nb1;
+    p.ns1 = d.ns1;
+    p.off_d2 = d.off_d2;
+    p.off_e2 = d.off_e2;
+    p.nb2 = d.nb2;
+    p.ns2 = d.ns2;
+    p.gimage = ctx.d_gimage.get();
+    p.n_stages = ctx.n_stages;
+    p.stage_magic = (uint32_t)((1ull << 32) / ctx.n_stages) + 1u;
+    p.debug = ctx.debug;
+    EmitParams &ep = p.emit;
+    ep.max_pat_len = p.max_pat_len;
+    ep.use_ref_bound = p.use_ref_bound;
+    ep.r = ctx.d_r.get();
+    ep.htval = ctx.d_htval.get();
+    ep.idmap = ctx.d_idmap.get();
+    ep.s0 = ctx.d_s0.get();
+    ep.step = ctx.d_step.get();
+    ep.s0r = ctx.d_s0r.get();
+    if (pd.n_slots) {
+        ep.dir = reinterpret_cast<const uint4 *>(ctx.d_patdir.get());
+        ep.pool = ctx.d_patdir.get() + pd.off_pool;
+        ep.dir_slots = pd.n_slots;
+        ep.len_mask = pd.len_mask;
+    }
+    ep.ht_size = P.ht_size;
+    ep.width_bit = width_bit;
+    ep.n_final = P.n_final;
+    return PFAC_OK;
+}
+
+// walk cache of the dense-match kernel: as deep as fits beside its text tile and result arrays.  Fills the
+// per-context part of ctx.dense.
+int upload_walk_cache(pfac_ctx &ctx, const Partition &P, size_t smem_max)
+{
+    const size_t fixed = dense_smem_bytes(0, ctx.halo);
+    const uint32_t budget = smem_max > fixed + 4096 ? (uint32_t)std::min<size_t>(smem_max - fixed, 128u << 10) : 2048u;
+    WalkCache wc;
+    derive_walk_cache(P, budget, wc);
+    const uint32_t wc_bytes = (uint32_t)((wc.image.size() + 15) & ~(size_t)15);
+    wc.image.resize(wc_bytes, 0);
+    ctx.dense_smem = dense_smem_bytes(wc_bytes, ctx.halo);
+    if (ctx.dense_smem > smem_max)
+        return set_error(PFAC_ERR_CUDA, "dense-match kernel needs %zu B of shared memory (patterns too long)", ctx.dense_smem);
+    int e = ctx.d_wcache.upload(wc.image);
+    if (e) return e;
+    DenseParams &d = ctx.dense;
+    memset(&d, 0, sizeof d);
+    d.wc_image = ctx.d_wcache.get();
+    d.wc_bytes = wc_bytes;
+    d.wc_depth = wc.depth;
+    d.wc_off_d = wc.off_d;
+    d.wc_off_e = wc.off_e;
+    d.wc_nb = wc.nb;
+    d.wc_ns = wc.ns;
+    d.halo = ctx.halo;
+    return PFAC_OK;
+}
+
+// batch scans need each id's pattern length (a tree-shaped automaton) and results that do not depend on
+// where a document lies in the packed buffer (no reference tile bound: patterns of <= 513 bytes)
+int upload_pattern_lengths(pfac_ctx &ctx, const Partition &P)
+{
+    std::vector<int32_t> len;
+    if (pattern_lengths(P, len) != PFAC_OK) {
+        ctx.batch_rc = PFAC_ERR_ARG;
+        ctx.batch_why = pfac_last_error();
+    } else if (P.max_len > kRefHalo + 1) {
+        ctx.batch_rc = PFAC_ERR_LIMIT;
+        ctx.batch_why = "batch scans need patterns of at most 513 bytes (the reference's 4096+512 tile bound "
+                        "would make results depend on where a document lies in the batch)";
+    } else {
+        ctx.n_ids = (uint32_t)len.size();
+        len.resize(std::max<size_t>(len.size(), 1), 0);
+        return ctx.d_patlen.upload(len);
+    }
+    return PFAC_OK;
 }
 
 }  // namespace
@@ -554,10 +710,11 @@ int pfac_ctx_create(int device, const pfac_tables *t, int part, int n_streams, s
     DeviceGuard g(device);
     if (!g.ok) return set_error(PFAC_ERR_CUDA, "cudaSetDevice(%d) failed", device);
     const Partition &P = t->parts[(size_t)part];
-    // (every early return below releases what was allocated so far: pfac_ctx_destroy tolerates null members)
+    // (every early return below releases what was allocated so far)
     std::unique_ptr<pfac_ctx, void (*)(pfac_ctx *)> ctx(new pfac_ctx, pfac_ctx_destroy);
     ctx->device = device;
     ctx->n_streams = n_streams;
+    ctx->stages.reset(new Stage[(size_t)n_streams]);
     ctx->chunk_bytes = chunk_bytes ? chunk_bytes : ((size_t)32 << 20);
     ctx->chunk_bytes = (ctx->chunk_bytes + kTile - 1) / kTile * kTile;
     cudaDeviceProp prop;
@@ -566,171 +723,34 @@ int pfac_ctx_create(int device, const pfac_tables *t, int part, int n_streams, s
         return set_error(PFAC_ERR_NO_DEVICE, "device %d is sm_%d%d; this library is built for sm_100a only",
                          device, prop.major, prop.minor);
     ctx->sm_count = prop.multiProcessorCount;
-    ctx->ht_size = P.ht_size;
-    ctx->width_bit = width_bits(P.width);
-    ctx->n_final = P.n_final;
     ctx->max_pat_len = P.max_len;
     ctx->halo = (uint32_t)std::max(16, ((P.max_len > 0 ? P.max_len - 1 : 0) + 15) / 16 * 16);
     if (const char *dbg = getenv("PFAC_DEBUG")) ctx->debug = (uint32_t)atoi(dbg);
     if (const char *v = getenv("PFAC_NO_PDL")) ctx->use_pdl = atoi(v) == 0;
 
-    // shared-memory budget: T1 and the per-warp queues are fixed; T3 / Tm2 / T2 shrink until at least
-    // four ring stages fit
     const size_t smem_max = (size_t)prop.sharedMemPerBlockOptin;
-    uint32_t t2_bytes = 32768, t3_bytes = 32768, tm2_bytes = 32768;
-    if (const char *v = getenv("PFAC_T2_BYTES")) t2_bytes = (uint32_t)atoi(v);
-    if (const char *v = getenv("PFAC_T3_BYTES")) t3_bytes = (uint32_t)atoi(v);
-    if (const char *v = getenv("PFAC_TM2_BYTES")) tm2_bytes = (uint32_t)atoi(v);
-    bool widened = false;
-    while (true) {
-        derive_tables(P, t2_bytes, t3_bytes, tm2_bytes, ctx->dv);
-        if (ctx->dv.mode == 2 && !widened && !getenv("PFAC_T2_BYTES")) {
-            // global mode: T2 is stage 1 and the only shared-memory table -- give it all the room
-            widened = true;
-            t2_bytes = 131072;
-            continue;
-        }
-        ctx->image_bytes = (uint32_t)ctx->dv.image.size();
-        const size_t fixed = scan_smem_bytes(ctx->image_bytes, ctx->halo, 0, ctx->dv.mode);
-        const size_t stride = scan_buf_stride(ctx->halo);
-        const size_t fit = smem_max > fixed ? (smem_max - fixed) / stride : 0;
-        const bool minimal = t2_bytes < 2048 && (ctx->dv.mode == 2 || (t3_bytes < 2048 && tm2_bytes < 2048));
-        const size_t need = (size_t)min_stages((int)ctx->dv.mode);   // 2 (shared-memory mode) or 4 (global mode)
-        // mode 0 wants a deep ring (bytes in flight hide the HBM latency): T3 gives way down to 16 KiB
-        const bool deepen = ctx->dv.mode == 0 && fit < 9 && t3_bytes > 16384 && !getenv("PFAC_T3_BYTES");
-        if (!deepen && (fit >= std::max<size_t>(3, need) || (fit >= need && minimal))) {
-            ctx->n_stages = (uint32_t)std::min<size_t>(fit, kMaxStages);
-            if (const char *v = getenv("PFAC_RING_STAGES"))   // tests: a ring as shallow as the slot scheme allows
-                ctx->n_stages = (uint32_t)std::max<size_t>(need, std::min<size_t>(ctx->n_stages, (size_t)atoi(v)));
-            ctx->smem_bytes = scan_smem_bytes(ctx->image_bytes, ctx->halo, ctx->n_stages, ctx->dv.mode);
-            break;
-        }
-        if (minimal)
-            return set_error(PFAC_ERR_CUDA, "scan kernel needs more than the %zu B of shared memory the device offers",
-                             smem_max);
-        // halve the largest section that is actually in the image
-        if (ctx->dv.mode == 2) {
-            t2_bytes /= 2;
-        } else if (ctx->dv.has_t3) {
-            if (t3_bytes > 8192) t3_bytes /= 2;          // T3 first: it only gets a little less selective
-            else if (tm2_bytes >= 2048) tm2_bytes /= 2;  // then level 2 (all or nothing per size)
-            else t3_bytes /= 2;
-        } else {
-            t3_bytes = tm2_bytes = 0;
-            t2_bytes /= 2;
-        }
-    }
-
-    // canonical arrays -> device, unchanged: s0Table, r, {HT, val} interleaved, idmap; + the detector image
-    const size_t n_r = std::max<size_t>(P.r.size(), 1), n_ht = std::max<size_t>((size_t)P.ht_size, 1);
-    const size_t n_id = std::max<size_t>((size_t)P.n_final, 1);
-    std::vector<int2> htval(n_ht, make_int2(-1, -1));
-    for (int32_t i = 0; i < P.ht_size; i++) htval[(size_t)i] = make_int2(P.HT[(size_t)i], P.val[(size_t)i]);
-    std::vector<int32_t> s0(256, -1);
-    if (!P.s0.empty()) s0 = P.s0;
-    CU_TRY(cudaMalloc(&ctx->d_r, n_r * sizeof(int32_t)));
-    CU_TRY(cudaMalloc(&ctx->d_htval, n_ht * sizeof(int2)));
-    CU_TRY(cudaMalloc(&ctx->d_idmap, n_id * sizeof(int32_t)));
-    CU_TRY(cudaMalloc(&ctx->d_s0, 256 * sizeof(int32_t)));
-    CU_TRY(cudaMalloc(&ctx->d_image, ctx->image_bytes));
-    CU_TRY(cudaMemset(ctx->d_r, 0xFF, n_r * sizeof(int32_t)));
-    CU_TRY(cudaMemset(ctx->d_idmap, 0, n_id * sizeof(int32_t)));
-    if (!P.r.empty()) CU_TRY(cudaMemcpy(ctx->d_r, P.r.data(), P.r.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
-    CU_TRY(cudaMemcpy(ctx->d_htval, htval.data(), n_ht * sizeof(int2), cudaMemcpyHostToDevice));
-    if (P.n_final) CU_TRY(cudaMemcpy(ctx->d_idmap, P.idmap.data(), (size_t)P.n_final * sizeof(int32_t), cudaMemcpyHostToDevice));
-    CU_TRY(cudaMemcpy(ctx->d_s0, s0.data(), 256 * sizeof(int32_t), cudaMemcpyHostToDevice));
-    CU_TRY(cudaMemcpy(ctx->d_image, ctx->dv.image.data(), ctx->image_bytes, cudaMemcpyHostToDevice));
-    if (ctx->width_bit >= 8 && !P.r.empty()) {
-        // the one-load layout of the candidate walks: the row of a state's transitions depends on the state
-        // alone when a row holds at least 256 keys, so every entry can carry its successor's r[] value
-        const int sh = ctx->width_bit - 8;
-        auto r_of = [&](int32_t state) -> int32_t {
-            const size_t row = (size_t)state >> sh;
-            return state >= 0 && row < P.r.size() ? P.r[row] : -1;
-        };
-        std::vector<int4> step(n_ht, make_int4(-1, -1, -1, 0));
-        for (int32_t i = 0; i < P.ht_size; i++) step[(size_t)i] = make_int4(P.HT[(size_t)i], P.val[(size_t)i], r_of(P.val[(size_t)i]), 0);
-        std::vector<int2> s0r(256);
-        for (int b = 0; b < 256; b++) s0r[(size_t)b] = make_int2(s0[(size_t)b], r_of(s0[(size_t)b]));
-        CU_TRY(cudaMalloc(&ctx->d_step, n_ht * sizeof(int4)));
-        CU_TRY(cudaMalloc(&ctx->d_s0r, 256 * sizeof(int2)));
-        CU_TRY(cudaMemcpy(ctx->d_step, step.data(), n_ht * sizeof(int4), cudaMemcpyHostToDevice));
-        CU_TRY(cudaMemcpy(ctx->d_s0r, s0r.data(), 256 * sizeof(int2), cudaMemcpyHostToDevice));
-    }
-    if (!getenv("PFAC_NO_PATDIR")) derive_patdir(P, ctx->pd);
-    if (ctx->pd.n_slots) {
-        CU_TRY(cudaMalloc(&ctx->d_patdir, ctx->pd.image.size()));
-        CU_TRY(cudaMemcpy(ctx->d_patdir, ctx->pd.image.data(), ctx->pd.image.size(), cudaMemcpyHostToDevice));
-        ctx->table_bytes += ctx->pd.image.size();
-        ctx->pd.image.clear();
-        ctx->pd.image.shrink_to_fit();
-    }
-    if (!ctx->dv.gimage.empty()) {
-        CU_TRY(cudaMalloc(&ctx->d_gimage, ctx->dv.gimage.size()));
-        CU_TRY(cudaMemcpy(ctx->d_gimage, ctx->dv.gimage.data(), ctx->dv.gimage.size(), cudaMemcpyHostToDevice));
-    }
-    {   // walk cache of the dense-match kernel: as deep as fits beside its text tile and result arrays
-        const size_t fixed = dense_smem_bytes(0, ctx->halo);
-        const uint32_t budget = smem_max > fixed + 4096 ? (uint32_t)std::min<size_t>(smem_max - fixed, 128u << 10) : 2048u;
-        derive_walk_cache(P, budget, ctx->wc);
-        ctx->wc_bytes = (uint32_t)((ctx->wc.image.size() + 15) & ~(size_t)15);
-        ctx->wc.image.resize(ctx->wc_bytes, 0);
-        ctx->dense_smem = dense_smem_bytes(ctx->wc_bytes, ctx->halo);
-        if (ctx->dense_smem > smem_max)
-            return set_error(PFAC_ERR_CUDA, "dense-match kernel needs %zu B of shared memory (patterns too long)", ctx->dense_smem);
-        CU_TRY(cudaMalloc(&ctx->d_wcache, ctx->wc_bytes));
-        CU_TRY(cudaMemcpy(ctx->d_wcache, ctx->wc.image.data(), ctx->wc_bytes, cudaMemcpyHostToDevice));
-        ctx->wc.image.clear();
-        ctx->wc.image.shrink_to_fit();
-        CU_TRY(cudaFuncSetAttribute(pfac_dense_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max));
-        CU_TRY(cudaFuncSetAttribute(pfac_dense_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max));
-    }
-    {   // batch scans need each id's pattern length (a tree-shaped automaton) and results that do not depend on
-        // where a document lies in the packed buffer (no reference tile bound: patterns of <= 513 bytes)
-        std::vector<int32_t> len;
-        if (pattern_lengths(P, len) != PFAC_OK) {
-            ctx->batch_rc = PFAC_ERR_ARG;
-            ctx->batch_why = pfac_last_error();
-        } else if (P.max_len > kRefHalo + 1) {
-            ctx->batch_rc = PFAC_ERR_LIMIT;
-            ctx->batch_why = "batch scans need patterns of at most 513 bytes (the reference's 4096+512 tile bound "
-                             "would make results depend on where a document lies in the batch)";
-        } else {
-            ctx->n_ids = (uint32_t)len.size();
-            CU_TRY(cudaMalloc(&ctx->d_patlen, std::max<size_t>(len.size(), 1) * sizeof(int32_t)));
-            if (!len.empty())
-                CU_TRY(cudaMemcpy(ctx->d_patlen, len.data(), len.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
-            ctx->table_bytes += std::max<size_t>(len.size(), 1) * sizeof(int32_t);
-        }
-    }
+    int e;
+    if ((e = size_shared_memory(*ctx, P, smem_max)) || (e = upload_tables(*ctx, P)) ||
+        (e = upload_walk_cache(*ctx, P, smem_max)) || (e = upload_pattern_lengths(*ctx, P)))
+        return e;
     ctx->dense_first = ctx->dv.has_short != 0;
     if (const char *v = getenv("PFAC_DENSE_FIRST")) ctx->dense_first = atoi(v) != 0;   // experiments: force either path
-    ctx->table_bytes += n_r * 4 + n_ht * 8 + n_id * 4 + 1024 + ctx->image_bytes + ctx->dv.gimage.size() + ctx->wc_bytes + (ctx->d_step ? n_ht * 16 + 2048 : 0);
     ctx->dv.image.clear();
     ctx->dv.image.shrink_to_fit();
     ctx->dv.gimage.clear();
     ctx->dv.gimage.shrink_to_fit();
 
     // the attribute is per function and device, not per context: always allow the device maximum
-    CU_TRY(cudaFuncSetAttribute(pfac_scan_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max));
-    CU_TRY(cudaFuncSetAttribute(pfac_scan_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max));
-    CU_TRY(cudaFuncSetAttribute(pfac_scan2_kernel<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max));
-    CU_TRY(cudaFuncSetAttribute(pfac_scan2_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max));
-    CU_TRY(cudaFuncSetAttribute(pfac_scan2_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max));
-    CU_TRY(cudaFuncSetAttribute(pfac_scan2_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max));
-    CU_TRY(cudaFuncSetAttribute(pfac_scan2_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max));
+    std::vector<const void *> kernels = {(const void *)pfac_dense_kernel<false>, (const void *)pfac_dense_kernel<true>};
+    for (DetectorKernel k : kDetectors) kernels.push_back((const void *)k);
+    for (const void *k : kernels) CU_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max));
     int bps = 0;
-    if (ctx->dv.mode == 2)
-        CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, pfac_scan_kernel<2>, kThreads, ctx->smem_bytes));
-    else if (ctx->dv.mode == 1)
-        CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, pfac_scan_kernel<1>, kThreads, ctx->smem_bytes));
-    else
-        CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, pfac_scan2_kernel<true, true, false>, kThreads, ctx->smem_bytes));
+    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, detector_kernel(ctx->dv), kThreads, ctx->smem_bytes));
     if (bps < 1) return set_error(PFAC_ERR_CUDA, "scan kernel does not fit on an SM (smem %zu B)", ctx->smem_bytes);
 
     CU_TRY(cudaStreamCreateWithFlags(&ctx->own_stream, cudaStreamNonBlocking));
     CU_TRY(cudaEventCreateWithFlags(&ctx->own_done, cudaEventDisableTiming));
-    int e = slot_init(ctx->own);
+    e = slot_init(ctx->own);
     if (e) return e;
     *out = ctx.release();
     return PFAC_OK;
@@ -741,24 +761,11 @@ void pfac_ctx_destroy(pfac_ctx *ctx)
     if (!ctx) return;
     DeviceGuard g(ctx->device);
     cudaDeviceSynchronize();
-    for (auto &s : ctx->stages) free_stage(s);
-    slot_free(ctx->own);
-    if (ctx->d_r) cudaFree(ctx->d_r);
-    if (ctx->d_htval) cudaFree(ctx->d_htval);
-    if (ctx->d_step) cudaFree(ctx->d_step);
-    if (ctx->d_s0r) cudaFree(ctx->d_s0r);
-    if (ctx->d_patdir) cudaFree(ctx->d_patdir);
-    if (ctx->d_idmap) cudaFree(ctx->d_idmap);
-    if (ctx->d_image) cudaFree(ctx->d_image);
-    if (ctx->d_s0) cudaFree(ctx->d_s0);
-    if (ctx->d_gimage) cudaFree(ctx->d_gimage);
-    if (ctx->d_wcache) cudaFree(ctx->d_wcache);
-    if (ctx->d_patlen) cudaFree(ctx->d_patlen);
     for (auto e : ctx->ev)
         if (e) cudaEventDestroy(e);
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
     if (ctx->own_done) cudaEventDestroy(ctx->own_done);
-    delete ctx;
+    delete ctx;   // (frees the buffers, slots and stages on the context's device)
 }
 
 int pfac_ctx_device(const pfac_ctx *ctx) { return ctx ? ctx->device : -1; }
@@ -804,23 +811,8 @@ int pfac_ctx_derived_info(const pfac_ctx *ctx, uint64_t info[16])
     const uint64_t v[16] = {ctx->image_bytes, d.t1_set, d.t2_shift >= 32 ? 0 : (1ull << (32 - d.t2_shift)), d.t2_set,
                             d.n_prefix4, d.has_short, d.tm_set, d.tm2_set,
                             d.t3_shift >= 32 ? 0 : (1ull << (32 - d.t3_shift)), d.t3_set, ctx->smem_bytes,
-                            ctx->table_bytes, ctx->n_stages, d.tm2_bits, d.mode, d.tm_bits};
+                            ctx->table_bytes(), ctx->n_stages, d.tm2_bits, d.mode, d.tm_bits};
     memcpy(info, v, sizeof v);
-    return PFAC_OK;
-}
-
-// Device scans of one context share one working set (control block, tile directory, scratch): a scan
-// enqueued on another stream than the one before it is ordered after it.
-static int own_enter(pfac_ctx *ctx, cudaStream_t st)
-{
-    if (ctx->own_used && ctx->own_last != st) CU_TRY(cudaStreamWaitEvent(st, ctx->own_done, 0));
-    return PFAC_OK;
-}
-static int own_leave(pfac_ctx *ctx, cudaStream_t st)
-{
-    CU_TRY(cudaEventRecord(ctx->own_done, st));
-    ctx->own_last = st;
-    ctx->own_used = true;
     return PFAC_OK;
 }
 
@@ -828,55 +820,18 @@ int pfac_scan_device(pfac_ctx *ctx, const void *d_in, uint64_t n_starts, uint64_
                      void *d_out, uint64_t cap, void *d_count, void *stream)
 {
     if (!ctx || (!d_in && n_starts) || (!d_out && cap) || !d_count) return set_error(PFAC_ERR_ARG, "bad arguments to pfac_scan_device");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DeviceGuard g(ctx->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
-    uint64_t tiles = 0, ctas = 0, launches = 0;
-    int e = own_enter(ctx, st);
-    if (e) return e;
-    e = launch_scan(ctx, ctx->own, d_in, n_starts, n_valid, base_pos, 0u, d_out, cap, d_count, st, &tiles, &ctas, &launches);
-    if (e) return e;
-    e = own_leave(ctx, st);
-    if (e) return e;
-    ctx->info[0] = launches;
-    ctx->info[1] = tiles;
-    ctx->info[2] = ctas;
-    ctx->info[3] = ctx->smem_bytes;
-    ctx->info[4] = ctx->info[5] = 0;
-    ctx->info[6] = 1;
-    return PFAC_OK;
+    return run_own(ctx, stream, cap, nullptr, [&](cudaStream_t st, Counters &n) {
+        return launch_scan(ctx, ctx->own, d_in, n_starts, n_valid, base_pos, 0u, d_out, cap, d_count, st, n);
+    });
 }
 
 int pfac_scan_device_sync(pfac_ctx *ctx, const void *d_in, uint64_t n_starts, uint64_t n_valid, uint64_t base_pos,
                           void *d_out, uint64_t cap, uint64_t *count, void *stream)
 {
     if (!ctx || !count || (!d_in && n_starts) || (!d_out && cap)) return set_error(PFAC_ERR_ARG, "bad arguments to pfac_scan_device_sync");
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
-    {
-        std::lock_guard<std::mutex> lk(ctx->mu);
-        DeviceGuard g(ctx->device);
-        uint64_t tiles = 0, ctas = 0, launches = 0;
-        int e = own_enter(ctx, st);
-        if (e) return e;
-        e = launch_scan(ctx, ctx->own, d_in, n_starts, n_valid, base_pos, 0u, d_out, cap, nullptr, st, &tiles, &ctas, &launches);
-        if (e) return e;
-        CU_TRY(cudaMemcpyAsync(ctx->own.h_result, ctx->own.d_result, sizeof(Result), cudaMemcpyDeviceToHost, st));
-        e = own_leave(ctx, st);
-        if (e) return e;
-        CU_TRY(cudaStreamSynchronize(st));
-        ctx->info[0] = launches;
-        ctx->info[1] = tiles;
-        ctx->info[2] = ctas;
-        ctx->info[3] = ctx->smem_bytes;
-        ctx->info[4] = ctx->info[5] = 0;
-        ctx->info[6] = 1;
-        if (ctx->own.h_result->error_flag)
-            return set_error(PFAC_ERR_INTERNAL, "device watchdog tripped (code %u)", ctx->own.h_result->error_flag);
-        *count = ctx->own.h_result->count;
-    }
-    if (*count > cap) return set_error(PFAC_ERR_OUTPUT_FULL, "%llu matches exceed the capacity of %llu records",
-                                       (unsigned long long)*count, (unsigned long long)cap);
-    return PFAC_OK;
+    return run_own(ctx, stream, cap, count, [&](cudaStream_t st, Counters &n) {
+        return launch_scan(ctx, ctx->own, d_in, n_starts, n_valid, base_pos, 0u, d_out, cap, nullptr, st, n);
+    });
 }
 
 int pfac_scan_batch_device(pfac_ctx *ctx, const void *d_in, const uint64_t *doc_offsets, uint32_t n_docs,
@@ -884,18 +839,9 @@ int pfac_scan_batch_device(pfac_ctx *ctx, const void *d_in, const uint64_t *doc_
 {
     if (!ctx || !doc_offsets || (!d_out && cap) || !d_doc_first || !d_count)
         return set_error(PFAC_ERR_ARG, "bad arguments to pfac_scan_batch_device");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DeviceGuard g(ctx->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
-    uint64_t info[8];
-    int e = own_enter(ctx, st);
-    if (e) return e;
-    e = launch_batch(ctx, ctx->own, d_in, doc_offsets, n_docs, d_out, cap, d_doc_first, d_count, st, info);
-    if (e) return e;
-    e = own_leave(ctx, st);
-    if (e) return e;
-    memcpy(ctx->info, info, sizeof info);
-    return PFAC_OK;
+    return run_own(ctx, stream, cap, nullptr, [&](cudaStream_t st, Counters &n) {
+        return launch_batch(ctx, ctx->own, d_in, doc_offsets, n_docs, d_out, cap, d_doc_first, d_count, st, n);
+    });
 }
 
 int pfac_scan_batch_device_sync(pfac_ctx *ctx, const void *d_in, const uint64_t *doc_offsets, uint32_t n_docs,
@@ -903,27 +849,9 @@ int pfac_scan_batch_device_sync(pfac_ctx *ctx, const void *d_in, const uint64_t 
 {
     if (!ctx || !doc_offsets || (!d_out && cap) || !d_doc_first || !count)
         return set_error(PFAC_ERR_ARG, "bad arguments to pfac_scan_batch_device_sync");
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
-    {
-        std::lock_guard<std::mutex> lk(ctx->mu);
-        DeviceGuard g(ctx->device);
-        uint64_t info[8];
-        int e = own_enter(ctx, st);
-        if (e) return e;
-        e = launch_batch(ctx, ctx->own, d_in, doc_offsets, n_docs, d_out, cap, d_doc_first, nullptr, st, info);
-        if (e) return e;
-        CU_TRY(cudaMemcpyAsync(ctx->own.h_result, ctx->own.d_result, sizeof(Result), cudaMemcpyDeviceToHost, st));
-        e = own_leave(ctx, st);
-        if (e) return e;
-        CU_TRY(cudaStreamSynchronize(st));
-        memcpy(ctx->info, info, sizeof info);
-        if (ctx->own.h_result->error_flag)
-            return set_error(PFAC_ERR_INTERNAL, "device watchdog tripped (code %u)", ctx->own.h_result->error_flag);
-        *count = ctx->own.h_result->count;
-    }
-    if (*count > cap) return set_error(PFAC_ERR_OUTPUT_FULL, "%llu matches exceed the capacity of %llu records",
-                                       (unsigned long long)*count, (unsigned long long)cap);
-    return PFAC_OK;
+    return run_own(ctx, stream, cap, count, [&](cudaStream_t st, Counters &n) {
+        return launch_batch(ctx, ctx->own, d_in, doc_offsets, n_docs, d_out, cap, d_doc_first, nullptr, st, n);
+    });
 }
 
 int pfac_host_alloc(void **ptr, size_t bytes)
@@ -978,31 +906,18 @@ int pfac_scan_host(pfac_ctx *ctx, const void *h_in, uint64_t n_starts, uint64_t 
     const uint64_t chunk = ctx->chunk_bytes;
     const uint64_t n_chunks = (n_starts + chunk - 1) / chunk;
     const int S = (int)std::min<uint64_t>((uint64_t)ctx->n_streams, std::max<uint64_t>(n_chunks, 1));
-    if ((int)ctx->stages.size() < S) ctx->stages.resize((size_t)S);
+    const uint64_t first = std::min<uint64_t>(chunk, n_starts);
     for (int s = 0; s < S; s++) {
         Stage &st = ctx->stages[(size_t)s];
+        int e;
         if (!st.stream) {
             CU_TRY(cudaStreamCreateWithFlags(&st.stream, cudaStreamNonBlocking));
             CU_TRY(cudaEventCreateWithFlags(&st.done, cudaEventDisableTiming));
-            int e = slot_init(st.slot);
-            if (e) return e;
+            if ((e = slot_init(st.slot))) return e;
         }
-        const size_t need_in = (size_t)(std::min<uint64_t>(chunk, n_starts) + halo + 64);
-        if (st.d_in_cap < need_in) {
-            if (st.d_in) cudaFree(st.d_in);
-            st.d_in = nullptr;
-            st.d_in_cap = 0;
-            CU_TRY(cudaMalloc(&st.d_in, need_in));
-            st.d_in_cap = need_in;
-        }
-        const size_t need_out = std::max<size_t>((size_t)(std::min<uint64_t>(chunk, n_starts) / 8), 4096);
-        if (st.d_out_cap < need_out) {
-            if (st.d_out) cudaFree(st.d_out);
-            st.d_out = nullptr;
-            st.d_out_cap = 0;
-            CU_TRY(cudaMalloc(&st.d_out, need_out * sizeof(pfac_match)));
-            st.d_out_cap = need_out;
-        }
+        const size_t need_out = std::max<size_t>((size_t)(first / 8), 4096);
+        if ((e = st.d_in.reserve((size_t)(first + halo + 64), 0, st.stream)) || (e = st.d_out.reserve(need_out, 0, st.stream)))
+            return e;
     }
     // Whatever path leaves this function: no copy from h_in or into h_out may still be in flight (the
     // caller is free to release its buffers on an error).
@@ -1015,23 +930,24 @@ int pfac_scan_host(pfac_ctx *ctx, const void *h_in, uint64_t n_starts, uint64_t 
                 if (ctx->stages[(size_t)s].stream) cudaStreamSynchronize(ctx->stages[(size_t)s].stream);
         }
     } drain{ctx, S};
-    uint64_t h2d = 0, d2h = 0, launches = 0, tiles_total = 0, ctas_max = 0;
+    Counters n;
+    n.chunks = n_chunks;
     auto enqueue = [&](uint64_t c) -> int {
         Stage &st = ctx->stages[(size_t)(c % (uint64_t)S)];
         const uint64_t off = c * chunk;
         const uint64_t ns = std::min<uint64_t>(chunk, n_starts - off);
         const uint64_t nv = std::min<uint64_t>(ns + halo, n_valid - off);
-        CU_TRY(cudaMemcpyAsync(st.d_in, (const uint8_t *)h_in + off, (size_t)nv, cudaMemcpyHostToDevice, st.stream));
-        h2d += nv;
-        uint64_t tiles = 0, ctas = 0, nl = 0;
-        int e = launch_scan(ctx, st.slot, st.d_in, ns, nv, base_pos + off, (uint32_t)off, st.d_out, st.d_out_cap, nullptr,
-                            st.stream, &tiles, &ctas, &nl);
+        CU_TRY(cudaMemcpyAsync(st.d_in.get(), (const uint8_t *)h_in + off, (size_t)nv, cudaMemcpyHostToDevice, st.stream));
+        n.h2d += nv;
+        Counters k;
+        int e = launch_scan(ctx, st.slot, st.d_in.get(), ns, nv, base_pos + off, (uint32_t)off, st.d_out.get(),
+                            st.d_out.cap(), nullptr, st.stream, k);
         if (e) return e;
-        launches += nl;
-        tiles_total += tiles;
-        ctas_max = std::max(ctas_max, ctas);
-        CU_TRY(cudaMemcpyAsync(st.slot.h_result, st.slot.d_result, sizeof(Result), cudaMemcpyDeviceToHost, st.stream));
-        d2h += sizeof(Result);
+        n.launches += k.launches;
+        n.tiles += k.tiles;
+        n.ctas = std::max(n.ctas, k.ctas);
+        CU_TRY(cudaMemcpyAsync(st.slot.h_result.get(), st.slot.d_result.get(), sizeof(Result), cudaMemcpyDeviceToHost, st.stream));
+        n.d2h += sizeof(Result);
         CU_TRY(cudaEventRecord(st.done, st.stream));
         return PFAC_OK;
     };
@@ -1041,49 +957,30 @@ int pfac_scan_host(pfac_ctx *ctx, const void *h_in, uint64_t n_starts, uint64_t 
     uint64_t total = 0;
     for (uint64_t c = 0; c < n_chunks; c++) {
         Stage &st = ctx->stages[(size_t)(c % (uint64_t)S)];
+        uint64_t m = 0;
         CU_TRY(cudaEventSynchronize(st.done));
-        if (st.slot.h_result->error_flag)
-            return set_error(PFAC_ERR_INTERNAL, "device watchdog tripped (code %u)", st.slot.h_result->error_flag);
-        uint64_t m = st.slot.h_result->count;
-        if (m > st.d_out_cap) {
+        if ((rc = check_result(*st.slot.h_result.get(), UINT64_MAX, &m))) return rc;   // (the watchdog alone)
+        if (m > st.d_out.cap()) {
             // dense matches: grow this stage's record buffer and scan the sub-chunk again
-            CU_TRY(cudaStreamSynchronize(st.stream));
-            cudaFree(st.d_out);
-            st.d_out = nullptr;
-            st.d_out_cap = 0;
-            CU_TRY(cudaMalloc(&st.d_out, (size_t)m * sizeof(pfac_match)));
-            st.d_out_cap = (size_t)m;
-            if ((rc = enqueue(c)) != PFAC_OK) return rc;
+            if ((rc = st.d_out.reserve((size_t)m, 0, st.stream)) || (rc = enqueue(c))) return rc;
             CU_TRY(cudaEventSynchronize(st.done));
-            if (st.slot.h_result->error_flag)
-                return set_error(PFAC_ERR_INTERNAL, "device watchdog tripped (code %u)", st.slot.h_result->error_flag);
-            m = st.slot.h_result->count;
+            if ((rc = check_result(*st.slot.h_result.get(), UINT64_MAX, &m))) return rc;
         }
         // records already carry positions relative to h_in[0] (pos_bias = sub-chunk offset)
         const uint64_t room = total < cap ? cap - total : 0;
         const uint64_t ncopy = std::min<uint64_t>(m, room);
         if (ncopy) {
-            CU_TRY(cudaMemcpyAsync(h_out + total, st.d_out, (size_t)ncopy * sizeof(pfac_match),
+            CU_TRY(cudaMemcpyAsync(h_out + total, st.d_out.get(), (size_t)ncopy * sizeof(pfac_match),
                                    cudaMemcpyDeviceToHost, st.stream));
-            d2h += ncopy * sizeof(pfac_match);
+            n.d2h += ncopy * sizeof(pfac_match);
         }
         total += m;
         if (c + (uint64_t)S < n_chunks)
             if ((rc = enqueue(c + (uint64_t)S)) != PFAC_OK) return rc;
     }
     for (int s = 0; s < S; s++) CU_TRY(cudaStreamSynchronize(ctx->stages[(size_t)s].stream));
-    *count = total;
-    ctx->info[0] = launches;
-    ctx->info[1] = tiles_total;
-    ctx->info[2] = ctas_max;
-    ctx->info[3] = ctx->smem_bytes;
-    ctx->info[4] = h2d;
-    ctx->info[5] = d2h;
-    ctx->info[6] = n_chunks;
-    if (total > cap)
-        return set_error(PFAC_ERR_OUTPUT_FULL, "%llu matches exceed the capacity of %llu records",
-                         (unsigned long long)total, (unsigned long long)cap);
-    return PFAC_OK;
+    set_info(ctx, n);
+    return check_result(Result{total, 0u, 0u}, cap, count);
 }
 
 }  // extern "C"

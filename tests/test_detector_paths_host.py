@@ -3,7 +3,7 @@ CPU checks: the brute-force reference equals the oracle, the background byte has
 queue text hits its survivor count in the host model of the filters, and the tile geometry the texts are laid
 out against is the geometry of pfac_kernel.cuh.
 
-A scan runs one of several detector kernels (pfac_device.cu, launch_scan), chosen by the derived tables
+A scan runs one of several detector kernels (pfac_device.cu, detector_kernel), chosen by the derived tables
 (pfac_derive.cc, derive_tables) and pfac_ctx_create.  Each case below is a pattern set, an environment and the
 signature the GPU test asserts, so that a case that drifts off its kernel fails instead of passing with less
 coverage.  Texts are a background byte that no pattern contains, with patterns planted at controlled
@@ -101,7 +101,8 @@ def base_blob(name):
     raise KeyError(name)
 
 
-# name -> base set, extra patterns, environment, expected signature.  kernel: what launch_scan runs for it
+# name -> base set, extra patterns, environment, expected signature.  kernel: what a scan of it runs
+# (pfac_device.cu, detector_kernel; or the dense-match kernel alone)
 # (T/F = HAS_SHORT, HAS_SC, W3 of pfac_scan2_kernel).  launches: 3 = detector + dense-match + ordering pass,
 # 1 = the dense-match kernel alone (DIRECT).  ref: "oracle" (Oracle, one partition), "brute" (brute_force) or
 # "tables" (the oracle's scan over the case's own canonical arrays).
