@@ -14,6 +14,9 @@
  *   pfac_ctx_*     : one device: table upload + scan of device-resident or host buffers, and of
  *                    batches of independent device-resident documents (pfac_scan_batch_device)
  *                    (GPU_Malloc_Memory / GPU_TraceTable / GPU_Free_memory, main.cc:35-37)
+ *   pfac_flows_*   : streaming scan of many flows on one context: chunk by chunk, matches that
+ *                    straddle chunk boundaries included, the carried bytes kept on the device
+ *                    (pfac_scan_flows_device_sync)
  *   pfac_job_*     : all GPUs of the box: contiguous input chunk + halo per GPU, stream pipeline
  *                    per GPU (the scan loop of main.cc:171-272)
  *   pfac_write_*   : GPU_match_result.txt writer (main.cc:335-350)
@@ -56,6 +59,7 @@ typedef struct pfac_match {
 typedef struct pfac_tables pfac_tables; /* host-side table set: n_parts x {s0,r,HT,val,idmap,...} */
 typedef struct pfac_ctx pfac_ctx;       /* one device */
 typedef struct pfac_job pfac_job;       /* multi-GPU job */
+typedef struct pfac_flows pfac_flows;   /* streaming state of many flows on one context */
 
 const char *pfac_last_error(void);
 int pfac_abi_version(void);
@@ -177,6 +181,39 @@ int pfac_scan_batch_device(pfac_ctx *ctx, const void *d_in, const uint64_t *doc_
 /* Same, synchronous; *count receives the device count.  PFAC_ERR_OUTPUT_FULL if *count > cap. */
 int pfac_scan_batch_device_sync(pfac_ctx *ctx, const void *d_in, const uint64_t *doc_offsets, uint32_t n_docs,
                                 void *d_out, uint64_t cap, void *d_doc_first, uint64_t *count, void *stream);
+
+/* Streaming scan of many flows (packets or reads of many connections, one chunk at a time); the reference has
+ * no counterpart.  A flow set holds n_flows independent byte streams.  Flow f has consumed P_f bytes so far, and
+ * the device keeps its last t_f = min(max_pat_len - 1, P_f) bytes.  One call takes n_chunks chunks for DISTINCT
+ * flows; the records of chunk i (flow f) are exactly the matches of flow f's whole stream whose end lies in the
+ * chunk, (P_f, P_f + c_i], so the union of a flow's records over its calls equals one pfac_scan_device over its
+ * concatenated bytes: nothing missing, nothing twice.  Records of one chunk are ordered by (pos, pattern length);
+ * across calls they are NOT globally position-ordered (a long match that ends late is reported after a shorter
+ * one that starts after it).  Same preconditions as the batch scan: pfac_flows_create returns PFAC_ERR_ARG for a
+ * context whose automaton is not a tree and PFAC_ERR_LIMIT for patterns longer than 513 bytes.
+ *
+ * A call either commits or leaves every flow unchanged: on PFAC_ERR_OUTPUT_FULL, on refused arguments or when
+ * the device watchdog trips no tail and no P_f advances, and a rescan with the returned count as capacity gives
+ * exactly the records the call would have given with enough room.  After PFAC_ERR_CUDA the state of the set is
+ * unspecified: reset every flow.  Hence the call is synchronous only.  Calls of one set are serialised; the set
+ * uses the context's working set like pfac_scan_device (same stream ordering rules).
+ *
+ * pfac_flows_destroy before its context.  pfac_flows_reset: flow starts a new stream (P_f = 0, empty tail);
+ * pfac_flows_position: *bytes = P_f. */
+int pfac_flows_create(pfac_ctx *ctx, uint32_t n_flows, pfac_flows **out);
+void pfac_flows_destroy(pfac_flows *f);
+int pfac_flows_reset(pfac_flows *f, uint32_t flow);
+int pfac_flows_position(const pfac_flows *f, uint32_t flow, uint64_t *bytes);
+/* Chunk i = d_in[chunk_offsets[i], chunk_offsets[i+1]) (a HOST array of n_chunks + 1 entries, chunk_offsets[0] = 0,
+ * non-decreasing) goes to flow flow_ids[i] (a HOST array, distinct ids < n_flows).  d_out, d_chunk_first, *count,
+ * cap and PFAC_ERR_OUTPUT_FULL as for pfac_scan_batch_device_sync, with the chunks in place of the documents and
+ * pos relative to base[i] (a HOST uint64[n_chunks]: base[i] = P_f - t_f, the stream position of the first carried
+ * byte), so a record's stream position is base[i] + pos and flows may run past 4 GiB.  PFAC_ERR_ARG for a flow id
+ * out of range or named twice, chunk_offsets[0] != 0 or decreasing offsets; PFAC_ERR_LIMIT when the chunks, or
+ * the chunks with their carried tails, reach 4 GiB.  All refusals come before anything is enqueued. */
+int pfac_scan_flows_device_sync(pfac_flows *f, const void *d_in, const uint64_t *chunk_offsets,
+                                const uint32_t *flow_ids, uint32_t n_chunks, void *d_out, uint64_t cap,
+                                void *d_chunk_first, uint64_t *base, uint64_t *count, void *stream);
 
 /* Whole GPU_TraceTable (H2D + kernel + D2H, master_kernel.cu:359-428) on HOST input, as a
  * pipeline of chunk_bytes sub-chunks (+halo) over n_streams streams.  h_in[0, n_starts) are

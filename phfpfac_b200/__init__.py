@@ -10,6 +10,7 @@ Host-side mirror of the reference's operator interface for the scan path
     GPU_Malloc_Memory(...)                      Matcher(tables, device=...)
     GPU_TraceTable(...)                         Matcher.scan_host(...) / Matcher.scan_device(...)
     (none: many independent documents)          Matcher.scan_batch(...) / Matcher.scan_docs(...)
+    (none: streams of many flows, chunk by chunk) Matcher.flows(n) -> Flows.scan(...) / Flows.feed(...)
     GPU_Free_memory(...)                        Matcher.close()
     merge + fprintf loop (main.cc:304-350)      format_records / write_result
 
@@ -17,14 +18,16 @@ All compute happens in phfpfac_b200/_build/libpfac_b200.so (hand-written sm_100a
 module only marshals buffers.  PyTorch, when used, only supplies device memory and streams.
 """
 import ctypes as C
+import weakref
 
 import numpy as np
 
 from ._lib import PFAC_ERR_OUTPUT_FULL, PfacError, check, lib
 
 MATCH_DTYPE = np.dtype([("pos", "<u4"), ("id", "<u4")])   # struct pfac_match
+FLOW_MATCH_DTYPE = np.dtype([("pos", "<u8"), ("id", "<u4")])   # a match of a flow: absolute stream position
 
-__all__ = ["Tables", "Matcher", "Job", "PfacError", "MATCH_DTYPE", "format_records", "write_result",
+__all__ = ["Tables", "Matcher", "Flows", "Job", "PfacError", "MATCH_DTYPE", "FLOW_MATCH_DTYPE", "format_records", "write_result",
            "write_sidecar", "read_sidecar", "pattern_file_hash", "pinned", "device_count", "plan_shard"]
 
 
@@ -190,11 +193,20 @@ class Matcher:
         self._h = h
         self.tables = tables
         self.device = device
+        self._flows = weakref.WeakSet()
 
     def close(self):
+        for f in list(getattr(self, "_flows", ())):   # a flow set must not outlive its context
+            f.close()
         if self._h and lib is not None:
             lib.pfac_ctx_destroy(self._h)
         self._h = None
+
+    def flows(self, n_flows):
+        """A set of n_flows independent streams scanned chunk by chunk (Flows)."""
+        f = Flows(self, n_flows)
+        self._flows.add(f)
+        return f
 
     def __del__(self):
         self.close()
@@ -306,6 +318,95 @@ class Matcher:
 
         out, n = _until_fits(scan, cap)
         return out[:n]
+
+
+class Flows:
+    """Streams of many flows (pfac_flows_*, pfac_scan_flows_device_sync): each call scans one chunk for each of
+    several distinct flows and reports the matches that END in the chunk, straddling chunk boundaries included,
+    so the union of a flow's records equals one scan of its whole stream.  A call that fails (records beyond cap,
+    bad arguments) leaves every flow unchanged.  Keeps its Matcher alive; Matcher.close() closes it first."""
+
+    def __init__(self, matcher, n_flows):
+        self._h = None
+        h = C.c_void_p()
+        check(lib.pfac_flows_create(matcher._h, n_flows, C.byref(h)))
+        self._h = h
+        self.matcher = matcher
+        self.n_flows = n_flows
+
+    def close(self):
+        if self._h and lib is not None:
+            lib.pfac_flows_destroy(self._h)
+        self._h = None
+
+    def __del__(self):
+        self.close()
+
+    def reset(self, flow):
+        """flow starts a new stream: position 0, nothing carried."""
+        check(lib.pfac_flows_reset(self._h, flow))
+
+    def position(self, flow):
+        """Bytes flow has consumed so far."""
+        n = C.c_uint64(0)
+        check(lib.pfac_flows_position(self._h, flow, C.byref(n)))
+        return n.value
+
+    def scan(self, flow_ids, values, offsets, cap=None, offset=0):
+        """values: torch uint8 CUDA tensor (or host bytes / uint8 array, uploaded through torch) holding the chunks
+        back to back from byte `offset` on; offsets: n + 1 integers, chunk i = bytes [offsets[i], offsets[i+1]), for
+        flow flow_ids[i] (distinct).  Returns (chunk_first: np.uint64[n + 1], base: np.uint64[n], records:
+        MATCH_DTYPE): the records of chunk i are records[chunk_first[i]:chunk_first[i+1]], ordered by (pos, pattern
+        length), at stream positions base[i] + pos (synchronous)."""
+        import torch
+        m = self.matcher
+        if not isinstance(values, torch.Tensor):
+            values = torch.from_numpy(_as_u8(values).copy()).cuda(m.device)
+        offs = np.asarray(offsets)
+        if offs.ndim != 1 or len(offs) < 1 or not np.issubdtype(offs.dtype, np.integer):
+            raise ValueError("offsets must be a 1-D sequence of n + 1 integers")
+        if (offs < 0).any() or int(offs.max()) > values.numel() - offset:
+            raise ValueError("offsets point outside the values")
+        offs = np.ascontiguousarray(offs, dtype=np.uint64)
+        ids = np.ascontiguousarray(flow_ids, dtype=np.uint32).reshape(-1)
+        n = len(offs) - 1
+        if len(ids) != n:
+            raise ValueError("one flow id per chunk")
+        carried = n * max(m.tables.max_pat_len - 1, 0)
+        cap = max(1024, (int(offs[-1]) + carried) // 8) if cap is None else cap
+        base = np.zeros(n, dtype=np.uint64)
+        stream = torch.cuda.current_stream(values.device).cuda_stream
+
+        def scan(cap):
+            out = torch.empty((max(cap, 1), 2), dtype=torch.int32, device=values.device)
+            first = torch.empty(n + 1, dtype=torch.int64, device=values.device)
+            cnt = C.c_uint64(0)
+            if stream == 0:     # the legacy default stream: 0 means "the library's own stream" to the C ABI
+                torch.cuda.current_stream(values.device).synchronize()
+            rc = lib.pfac_scan_flows_device_sync(self._h, values.data_ptr() + offset if values.numel() else None,
+                                                 offs.ctypes.data, ids.ctypes.data, n, out.data_ptr(), cap,
+                                                 first.data_ptr(), base.ctypes.data, C.byref(cnt), stream or None)
+            return rc, cnt.value, (out, first)
+
+        (out, first), count = _until_fits(scan, cap)   # (exact: a call that does not fit commits nothing)
+        return first.cpu().numpy().view(np.uint64), base, _records(out, count)
+
+    def feed(self, flow_ids, chunks):
+        """chunks: bytes-like chunks for the distinct flows flow_ids -> one FLOW_MATCH_DTYPE array per chunk, with
+        absolute stream positions (one call)."""
+        parts = [_as_u8(c) for c in chunks]
+        offs = np.zeros(len(parts) + 1, dtype=np.uint64)
+        offs[1:] = np.cumsum([len(p) for p in parts], dtype=np.uint64)
+        buf = np.concatenate(parts) if parts else np.zeros(0, dtype=np.uint8)
+        first, base, rec = self.scan(flow_ids, buf, offs)
+        res = []
+        for i in range(len(parts)):
+            seg = rec[int(first[i]):int(first[i + 1])]
+            r = np.zeros(len(seg), dtype=FLOW_MATCH_DTYPE)
+            r["pos"] = seg["pos"].astype(np.uint64) + base[i]
+            r["id"] = seg["id"]
+            res.append(r)
+        return res
 
 
 class Job:

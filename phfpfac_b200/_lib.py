@@ -21,7 +21,9 @@ ABI_SYMBOLS = [
     "pfac_tables_idmap", "pfac_tables_lookup", "pfac_tables_pattern_lengths", "pfac_tables_derive_check",
     "pfac_tables_filter_profile",
     "pfac_device_count", "pfac_ctx_create", "pfac_ctx_destroy", "pfac_ctx_device",
-    "pfac_scan_device", "pfac_scan_device_sync", "pfac_scan_batch_device", "pfac_scan_batch_device_sync", "pfac_scan_host", "pfac_host_alloc", "pfac_host_free", "pfac_host_register", "pfac_host_unregister",
+    "pfac_scan_device", "pfac_scan_device_sync", "pfac_scan_batch_device", "pfac_scan_batch_device_sync",
+    "pfac_flows_create", "pfac_flows_destroy", "pfac_flows_reset", "pfac_flows_position", "pfac_scan_flows_device_sync",
+    "pfac_scan_host", "pfac_host_alloc", "pfac_host_free", "pfac_host_register", "pfac_host_unregister",
     "pfac_ctx_last_scan_info", "pfac_ctx_derived_info", "pfac_ctx_set_timing", "pfac_ctx_kernel_time",
     "pfac_job_create", "pfac_job_destroy", "pfac_job_run", "pfac_job_run_file", "pfac_job_n_segments", "pfac_job_segment",
     "pfac_job_last_timing", "pfac_job_plan",
@@ -88,6 +90,13 @@ def _load():
                                           C.POINTER(C.c_uint64), _vp]
     lib.pfac_scan_batch_device.argtypes = [_vp, _vp, _vp, C.c_uint32, _vp, C.c_uint64, _vp, _vp, _vp]
     lib.pfac_scan_batch_device_sync.argtypes = [_vp, _vp, _vp, C.c_uint32, _vp, C.c_uint64, _vp,
+                                                C.POINTER(C.c_uint64), _vp]
+    lib.pfac_flows_create.argtypes = [_vp, C.c_uint32, C.POINTER(_vp)]
+    lib.pfac_flows_destroy.argtypes = [_vp]
+    lib.pfac_flows_destroy.restype = None
+    lib.pfac_flows_reset.argtypes = [_vp, C.c_uint32]
+    lib.pfac_flows_position.argtypes = [_vp, C.c_uint32, C.POINTER(C.c_uint64)]
+    lib.pfac_scan_flows_device_sync.argtypes = [_vp, _vp, _vp, _vp, C.c_uint32, _vp, C.c_uint64, _vp, _vp,
                                                 C.POINTER(C.c_uint64), _vp]
     lib.pfac_scan_host.argtypes = [_vp, _vp, C.c_uint64, C.c_uint64, C.c_uint64, _vp, C.c_uint64,
                                    C.POINTER(C.c_uint64)]

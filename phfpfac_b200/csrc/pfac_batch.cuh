@@ -15,6 +15,10 @@
 //   pfac_batch_docs_kernel   doc_first[i] = kept records before doc[i] (a binary search of kpos)
 // A raw count beyond the raw buffer is passed on as the count (it bounds the kept count: the caller rescans
 // with a buffer that size).
+// The streaming scan (pfac_flows.cuh) runs the count and split kernels with CARRY = true: its document d is the
+// carried tail of a flow (tail[d] bytes) followed by the new chunk, and a record is kept iff its pattern ends in
+// the chunk, doc[d] + tail[d] < p + len[id] <= doc[d + 1].  doc_first needs no change: every kept record of
+// document d still starts at or after doc[d].
 #pragma once
 #include "pfac_kernel.cuh"
 
@@ -38,6 +42,7 @@ struct BatchParams {
     unsigned long long *doc_first;   // caller's n_docs + 1 offsets
     Result *result;
     unsigned long long *count_out;   // caller's count (may be null)
+    const uint32_t *tail;       // CARRY: bytes of carried tail at the start of every document (null for batches)
 };
 
 // last d in [a, b) with doc[d] <= p (doc[a] <= p)
@@ -67,15 +72,19 @@ __device__ __forceinline__ void batch_range(const BatchParams &b, unsigned long 
 }
 
 // Is raw record i kept, and in which document does it lie
+template <bool CARRY>
 __device__ __forceinline__ bool batch_keep(const BatchParams &b, unsigned long long i, uint32_t d_lo, uint32_t d_hi,
                                            uint2 &r, uint32_t &d)
 {
     r = b.raw[i];
     d = batch_doc_of(b.doc, d_lo, d_hi + 1u, r.x);
     const uint32_t L = r.y < b.n_ids ? (uint32_t)__ldg(b.len + r.y) : 0u;
-    return (unsigned long long)r.x + L <= (unsigned long long)__ldg(b.doc + d + 1);
+    const unsigned long long end = (unsigned long long)r.x + L;
+    if (CARRY && end <= (unsigned long long)__ldg(b.doc + d) + __ldg(b.tail + d)) return false;   // ends in the tail
+    return end <= (unsigned long long)__ldg(b.doc + d + 1);
 }
 
+template <bool CARRY>
 __global__ void __launch_bounds__(kBatchThreads) pfac_batch_count_kernel(const BatchParams b)
 {
     __shared__ uint32_t s_doc[2];
@@ -90,7 +99,7 @@ __global__ void __launch_bounds__(kBatchThreads) pfac_batch_count_kernel(const B
     for (unsigned long long i = lo + threadIdx.x; i < hi; i += kBatchThreads) {
         uint2 r;
         uint32_t d;
-        kept += batch_keep(b, i, s_doc[0], s_doc[1], r, d) ? 1u : 0u;
+        kept += batch_keep<CARRY>(b, i, s_doc[0], s_doc[1], r, d) ? 1u : 0u;
     }
     __shared__ unsigned int s_sum[kBatchThreads / 32];
 #pragma unroll
@@ -104,6 +113,7 @@ __global__ void __launch_bounds__(kBatchThreads) pfac_batch_count_kernel(const B
     }
 }
 
+template <bool CARRY>
 __global__ void __launch_bounds__(kBatchThreads) pfac_batch_split_kernel(const BatchParams b)
 {
     __shared__ uint32_t s_doc[2];
@@ -136,7 +146,7 @@ __global__ void __launch_bounds__(kBatchThreads) pfac_batch_split_kernel(const B
         const unsigned long long i = c0 + (unsigned long long)tid;
         uint2 r = make_uint2(0u, 0u);
         uint32_t d = 0;
-        const bool keep = i < hi && batch_keep(b, i, s_doc[0], s_doc[1], r, d);
+        const bool keep = i < hi && batch_keep<CARRY>(b, i, s_doc[0], s_doc[1], r, d);
         const uint32_t bal = __ballot_sync(0xffffffffu, keep);
         if (lane == 0) s_warp[warp] = (unsigned int)__popc(bal);
         __syncthreads();

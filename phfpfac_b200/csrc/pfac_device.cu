@@ -1,7 +1,7 @@
 // Device side of the C ABI (include/pfac_b200.h): contexts, table upload, the device-resident
-// scan and the host pipeline.  Replaces GPU_Malloc_Memory / GPU_TraceTable / GPU_Free_memory
-// (reference master_kernel.cu:188-524).  There is no CPU fallback anywhere in this file: a
-// missing GPU or any CUDA error is reported as PFAC_ERR_NO_DEVICE / PFAC_ERR_CUDA.
+// scan, the host pipeline, batch scans and streaming scans of many flows.  Replaces GPU_Malloc_Memory /
+// GPU_TraceTable / GPU_Free_memory (reference master_kernel.cu:188-524).  There is no CPU fallback
+// anywhere in this file: a missing GPU or any CUDA error is reported as PFAC_ERR_NO_DEVICE / PFAC_ERR_CUDA.
 #include <algorithm>
 #include <cstdio>
 #include <cstring>
@@ -10,6 +10,7 @@
 
 #include "pfac_batch.cuh"
 #include "pfac_derive.h"
+#include "pfac_flows.cuh"
 #include "pfac_internal.h"
 #include "pfac_kernel.cuh"
 
@@ -86,6 +87,35 @@ private:
     size_t cap_ = 0;
 };
 
+// Per-call arrays of a launch sequence (a batch's document offsets, a flow call's per-chunk arrays): filled in
+// pinned memory and uploaded with one cudaMemcpyAsync.  Before the buffer is refilled the host waits for the
+// event of its previous upload, so an asynchronous call is never overwritten by the next.
+struct Staging {
+    Buf<uint32_t, true> h;
+    Buf<uint32_t> d;
+    cudaEvent_t copied = nullptr;   // end of the last upload from h
+    Staging() = default;
+    Staging(const Staging &) = delete;
+    Staging &operator=(const Staging &) = delete;
+    ~Staging()
+    {
+        if (copied) cudaEventDestroy(copied);
+    }
+    // n words; fill(h) writes them and may refuse the call (its status is returned before anything is enqueued)
+    template <typename Fill>
+    int upload(size_t n, cudaStream_t stream, Fill &&fill)
+    {
+        if (!copied) CU_TRY(cudaEventCreateWithFlags(&copied, cudaEventDisableTiming));
+        int e;
+        if ((e = d.reserve(n, 4096, stream)) || (e = h.reserve(n, 4096, stream))) return e;
+        CU_TRY(cudaEventSynchronize(copied));
+        if ((e = fill(h.get()))) return e;
+        CU_TRY(cudaMemcpyAsync(d.get(), h.get(), n * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+        CU_TRY(cudaEventRecord(copied, stream));
+        return PFAC_OK;
+    }
+};
+
 // Everything one in-flight scan needs besides the tables: control block, result block, tile
 // directory and the arrival-order scratch.  One per user of a stream (the context's own slot for
 // pfac_scan_device, one per pipeline stage for pfac_scan_host).
@@ -103,18 +133,11 @@ struct Slot {
     Buf<uint2> d_scratch;
     bool dirty = false;       // a launch sequence failed half way: the control block is reset before the next scan
     // batch scans (pfac_batch.cuh): raw records of the packed buffer and the global positions of the kept ones,
-    // the document offsets (pinned staging + device copy; doc_copied = end of the last upload from the staging
-    // buffer) and the split pass's per-CTA counts
+    // the document offsets and the split pass's per-CTA counts
     Buf<uint2> d_raw;
     Buf<uint32_t> d_kpos;
-    Buf<uint32_t, true> h_doc;
-    Buf<uint32_t> d_doc;
-    cudaEvent_t doc_copied = nullptr;
+    Staging doc;
     Buf<unsigned long long> d_blk;
-    ~Slot()
-    {
-        if (doc_copied) cudaEventDestroy(doc_copied);
-    }
 };
 
 struct Stage {   // one pipeline stage of pfac_scan_host
@@ -189,6 +212,22 @@ struct pfac_ctx {
         return d_r.bytes() + d_idmap.bytes() + d_s0.bytes() + d_htval.bytes() + d_step.bytes() + d_s0r.bytes() +
                d_patdir.bytes() + d_image.bytes() + d_gimage.bytes() + d_wcache.bytes() + d_patlen.bytes();
     }
+};
+
+// A set of flows for the streaming scan (pfac_flows.cuh): per flow the carried tail on the device and the bytes
+// consumed on the host; the packed buffer and the per-chunk arrays of a call.  mu serialises the calls on it.
+struct pfac_flows {
+    pfac_ctx *ctx = nullptr;
+    uint32_t n_flows = 0;
+    uint32_t keep = 0;                // M - 1: bytes carried per flow
+    uint32_t stride = 0;              // tail row: keep rounded up to 16
+    Buf<uint8_t> d_tails;             // n_flows rows
+    std::vector<uint64_t> pos;        // P_f
+    Buf<uint8_t> d_packed;
+    Staging stage;                    // doc[n + 1] | tail[n] | flow[n] | src[n]
+    std::vector<uint32_t> seen;       // per flow: the last call that named it (duplicate flow ids)
+    uint32_t call = 0;
+    mutable std::mutex mu;
 };
 
 namespace {
@@ -409,6 +448,52 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
     return PFAC_OK;
 }
 
+// The slot's buffers of a batch or flow call: raw records and kept positions for max(cap, 4096) records, the split
+// pass's per-CTA counts.  *grid = the CTAs of the count and split kernels.
+int split_prepare(pfac_ctx *ctx, Slot &slot, uint64_t cap, cudaStream_t stream, uint32_t *grid)
+{
+    int e = slot_init(slot);
+    if (e) return e;
+    *grid = 2u * (uint32_t)ctx->sm_count;
+    if (!slot.d_blk.get() && (e = slot.d_blk.alloc(*grid + 1))) return e;
+    const size_t want = (size_t)std::max<uint64_t>(cap, 4096);
+    if ((e = slot.d_raw.reserve(want, want, stream)) || (e = slot.d_kpos.reserve(want, want, stream))) return e;
+    return PFAC_OK;
+}
+
+// Enqueue the split pass (pfac_batch.cuh) over the raw records of the packed scan: n_docs documents at the device
+// offsets doc[n_docs + 1]; CARRY: the first tail[d] bytes of document d are carried (device, n_docs).
+template <bool CARRY>
+int launch_split(pfac_ctx *ctx, Slot &slot, uint32_t grid, const uint32_t *doc, const uint32_t *tail, uint32_t n_docs,
+                 void *d_out, uint64_t cap, void *d_doc_first, void *d_count, cudaStream_t stream, Counters &n)
+{
+    BatchParams bp;
+    memset(&bp, 0, sizeof bp);
+    bp.raw = slot.d_raw.get();
+    bp.raw_cap = slot.d_raw.cap();
+    bp.doc = doc;
+    bp.n_docs = n_docs;
+    bp.len = ctx->d_patlen.get();
+    bp.n_ids = ctx->n_ids;
+    bp.blk = slot.d_blk.get();
+    bp.out = (uint2 *)d_out;
+    bp.cap = cap;
+    bp.kpos = slot.d_kpos.get();
+    bp.doc_first = (unsigned long long *)d_doc_first;
+    bp.result = slot.d_result.get();
+    bp.count_out = (unsigned long long *)d_count;
+    bp.tail = tail;
+    const size_t n_off = (size_t)n_docs + 1;
+    const cudaLaunchConfig_t lc = launch_config(ctx, stream, grid, kBatchThreads, 0);
+    CU_TRY(cudaLaunchKernelEx(&lc, pfac_batch_count_kernel<CARRY>, bp));
+    CU_TRY(cudaLaunchKernelEx(&lc, pfac_batch_split_kernel<CARRY>, bp));
+    const cudaLaunchConfig_t dl =
+        launch_config(ctx, stream, (uint32_t)std::min<uint64_t>((n_off + kBatchThreads - 1) / kBatchThreads, grid), kBatchThreads, 0);
+    CU_TRY(cudaLaunchKernelEx(&dl, pfac_batch_docs_kernel, bp));
+    n.launches += 3;
+    return PFAC_OK;
+}
+
 // Enqueue a batch scan on `stream` (pfac_batch.cuh): the documents' offsets are uploaded, the packed buffer is
 // scanned into the slot's raw-record buffer, the split pass writes the caller's records, d_doc_first and
 // d_count.  On completion slot.d_result holds {count, error}.
@@ -422,60 +507,116 @@ int launch_batch(pfac_ctx *ctx, Slot &slot, const void *d_in, const uint64_t *do
     const uint64_t total = doc_offsets[n_docs];
     if (total >= (1ull << 32)) return set_error(PFAC_ERR_LIMIT, "one batch covers less than 4 GiB; split the input");
     if (!d_in && total) return set_error(PFAC_ERR_ARG, "null input of %llu bytes", (unsigned long long)total);
-    int e = slot_init(slot);
+    uint32_t grid = 0;
+    int e = split_prepare(ctx, slot, cap, stream, &grid);
     if (e) return e;
-    const uint32_t grid = 2u * (uint32_t)ctx->sm_count;   // CTAs of the count and split kernels
-    if (!slot.d_blk.get() && (e = slot.d_blk.alloc(grid + 1))) return e;
-    if (!slot.doc_copied) CU_TRY(cudaEventCreateWithFlags(&slot.doc_copied, cudaEventDisableTiming));
+    // the offsets, checked on the way (32 bits suffice: total < 4 GiB)
     const size_t n_off = (size_t)n_docs + 1;
-    const size_t want = (size_t)std::max<uint64_t>(cap, 4096);
-    if ((e = slot.d_doc.reserve(n_off, 4096, stream)) || (e = slot.h_doc.reserve(n_off, 4096, stream)) ||
-        (e = slot.d_raw.reserve(want, want, stream)) || (e = slot.d_kpos.reserve(want, want, stream)))
-        return e;
-    // offsets -> pinned staging once the previous upload from it is done, checked on the way (32 bits suffice:
-    // total < 4 GiB) -> device
-    CU_TRY(cudaEventSynchronize(slot.doc_copied));
-    uint64_t prev = 0;
-    bool decreasing = false;
-    for (size_t i = 0; i < n_off; i++) {
-        const uint64_t v = doc_offsets[i];
-        decreasing |= v < prev;
-        prev = v;
-        slot.h_doc.get()[i] = (uint32_t)v;
-    }
-    if (decreasing) return set_error(PFAC_ERR_ARG, "doc_offsets decrease");
-    CU_TRY(cudaMemcpyAsync(slot.d_doc.get(), slot.h_doc.get(), n_off * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
-    CU_TRY(cudaEventRecord(slot.doc_copied, stream));
+    e = slot.doc.upload(n_off, stream, [&](uint32_t *h) {
+        uint64_t prev = 0;
+        bool decreasing = false;
+        for (size_t i = 0; i < n_off; i++) {
+            const uint64_t v = doc_offsets[i];
+            decreasing |= v < prev;
+            prev = v;
+            h[i] = (uint32_t)v;
+        }
+        return decreasing ? set_error(PFAC_ERR_ARG, "doc_offsets decrease") : PFAC_OK;
+    });
+    if (e) return e;
 
     e = launch_scan(ctx, slot, d_in, total, total, 0, 0u, slot.d_raw.get(), slot.d_raw.cap(), nullptr, stream, n);
     if (e) return e;
-    BatchParams bp;
-    memset(&bp, 0, sizeof bp);
-    bp.raw = slot.d_raw.get();
-    bp.raw_cap = slot.d_raw.cap();
-    bp.doc = slot.d_doc.get();
-    bp.n_docs = n_docs;
-    bp.len = ctx->d_patlen.get();
-    bp.n_ids = ctx->n_ids;
-    bp.blk = slot.d_blk.get();
-    bp.out = (uint2 *)d_out;
-    bp.cap = cap;
-    bp.kpos = slot.d_kpos.get();
-    bp.doc_first = (unsigned long long *)d_doc_first;
-    bp.result = slot.d_result.get();
-    bp.count_out = (unsigned long long *)d_count;
-    const cudaLaunchConfig_t lc = launch_config(ctx, stream, grid, kBatchThreads, 0);
-    CU_TRY(cudaLaunchKernelEx(&lc, pfac_batch_count_kernel, bp));
-    CU_TRY(cudaLaunchKernelEx(&lc, pfac_batch_split_kernel, bp));
-    const cudaLaunchConfig_t dl =
-        launch_config(ctx, stream, (uint32_t)std::min<uint64_t>((n_off + kBatchThreads - 1) / kBatchThreads, grid), kBatchThreads, 0);
-    CU_TRY(cudaLaunchKernelEx(&dl, pfac_batch_docs_kernel, bp));
-    n.launches += 3;
+    e = launch_split<false>(ctx, slot, grid, slot.doc.d.get(), nullptr, n_docs, d_out, cap, d_doc_first, d_count, stream, n);
+    if (e) return e;
     n.h2d = n_off * sizeof(uint32_t);
     return PFAC_OK;
 }
 
-// The four entry points that scan into the context's own slot.  `launch(stream, counters)` enqueues the scan.
+// Enqueue a streaming call on `stream` (pfac_flows.cuh): per-chunk arrays uploaded, tails and chunks packed, the
+// packed buffer scanned, the split pass with the carry-aware keep rule, the new tails written if the records fit.
+// Every refusal comes before anything is enqueued; base[i] = P_f - t_f of chunk i.
+int launch_flows(pfac_flows *f, Slot &slot, const void *d_in, const uint64_t *chunk_offsets, const uint32_t *flow_ids,
+                 uint32_t n_chunks, void *d_out, uint64_t cap, void *d_chunk_first, uint64_t *base, cudaStream_t stream,
+                 Counters &n)
+{
+    pfac_ctx *ctx = f->ctx;
+    if (n_chunks == 0xFFFFFFFFu) return set_error(PFAC_ERR_LIMIT, "a call holds fewer than 2^32 - 1 chunks");
+    if (chunk_offsets[0] != 0)
+        return set_error(PFAC_ERR_ARG, "chunk_offsets[0] = %llu: the first chunk starts at 0", (unsigned long long)chunk_offsets[0]);
+    if (++f->call == 0) {   // (the stamps wrapped: forget them all)
+        std::fill(f->seen.begin(), f->seen.end(), 0u);
+        f->call = 1;
+    }
+    uint64_t packed = 0;
+    for (uint32_t i = 0; i < n_chunks; i++) {
+        const uint32_t fl = flow_ids[i];
+        if (fl >= f->n_flows) return set_error(PFAC_ERR_ARG, "flow id %u of chunk %u: the set has %u flows", fl, i, f->n_flows);
+        if (f->seen[fl] == f->call) return set_error(PFAC_ERR_ARG, "flow %u takes two chunks in one call", fl);
+        f->seen[fl] = f->call;
+        if (chunk_offsets[i + 1] < chunk_offsets[i]) return set_error(PFAC_ERR_ARG, "chunk_offsets decrease");
+        packed += std::min<uint64_t>(f->keep, f->pos[fl]) + (chunk_offsets[i + 1] - chunk_offsets[i]);
+    }
+    const uint64_t total_in = chunk_offsets[n_chunks];
+    if (total_in >= (1ull << 32) || packed + (uint64_t)kTile + 4096 >= (1ull << 32))
+        return set_error(PFAC_ERR_LIMIT, "one call covers less than 4 GiB of chunks and carried tails; split the input");
+    if (!d_in && total_in) return set_error(PFAC_ERR_ARG, "null input of %llu bytes", (unsigned long long)total_in);
+    uint32_t grid = 0;
+    int e = split_prepare(ctx, slot, cap, stream, &grid);
+    if (e || (e = f->d_packed.reserve((size_t)packed + 48, std::max<size_t>((size_t)packed + 48, 1 << 20), stream))) return e;
+    const size_t nc = n_chunks;
+    e = f->stage.upload(4 * nc + 1, stream, [&](uint32_t *h) {
+        uint32_t *doc = h, *tail = h + nc + 1, *flow = tail + nc, *src = flow + nc;
+        doc[0] = 0;
+        for (size_t i = 0; i < nc; i++) {
+            const uint32_t fl = flow_ids[i];
+            const uint64_t t = std::min<uint64_t>(f->keep, f->pos[fl]);
+            base[i] = f->pos[fl] - t;
+            doc[i + 1] = doc[i] + (uint32_t)(t + chunk_offsets[i + 1] - chunk_offsets[i]);
+            tail[i] = (uint32_t)t;
+            flow[i] = fl;
+            src[i] = (uint32_t)chunk_offsets[i];
+        }
+        return PFAC_OK;
+    });
+    if (e) return e;
+    const uint32_t *d_stage = f->stage.d.get();
+    FlowParams fp;
+    memset(&fp, 0, sizeof fp);
+    fp.in = (const uint8_t *)d_in;
+    fp.doc = d_stage;
+    fp.tail = d_stage + nc + 1;
+    fp.flow = fp.tail + nc;
+    fp.src = fp.flow + nc;
+    fp.n = n_chunks;
+    fp.total = (uint32_t)packed;
+    fp.tails = f->d_tails.get();
+    fp.stride = f->stride;
+    fp.keep = f->keep;
+    fp.packed = f->d_packed.get();
+    fp.result = slot.d_result.get();
+    fp.cap = cap;
+    const uint32_t pgrid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((packed + 4095) / 4096, 16ull * (uint64_t)ctx->sm_count));
+    const cudaLaunchConfig_t pl = launch_config(ctx, stream, pgrid, kFlowThreads, 0);
+    CU_TRY(cudaLaunchKernelEx(&pl, pfac_flow_pack_kernel, fp));
+    n.launches = 1;
+    Counters k;
+    e = launch_scan(ctx, slot, fp.packed, packed, packed, 0, 0u, slot.d_raw.get(), slot.d_raw.cap(), nullptr, stream, k);
+    if (e) return e;
+    n.launches += k.launches;
+    n.tiles = k.tiles;
+    n.ctas = k.ctas;
+    e = launch_split<true>(ctx, slot, grid, fp.doc, fp.tail, n_chunks, d_out, cap, d_chunk_first, nullptr, stream, n);
+    if (e) return e;
+    const uint32_t tgrid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((nc + 7) / 8, 2ull * (uint64_t)ctx->sm_count));
+    const cudaLaunchConfig_t tl = launch_config(ctx, stream, tgrid, kFlowThreads, 0);
+    CU_TRY(cudaLaunchKernelEx(&tl, pfac_flow_tail_kernel, fp));
+    n.launches += 1;
+    n.h2d = (4 * nc + 1) * sizeof(uint32_t);
+    return PFAC_OK;
+}
+
+// The entry points that scan into the context's own slot.  `launch(stream, counters)` enqueues the scan.
 // With `count` (the _sync forms) the Result block is read back and the stream synchronised, then the records
 // are checked against `cap`.  Device scans of one context share the slot: a scan enqueued on another stream
 // than the one before it is ordered after it (own_done).
@@ -852,6 +993,68 @@ int pfac_scan_batch_device_sync(pfac_ctx *ctx, const void *d_in, const uint64_t 
     return run_own(ctx, stream, cap, count, [&](cudaStream_t st, Counters &n) {
         return launch_batch(ctx, ctx->own, d_in, doc_offsets, n_docs, d_out, cap, d_doc_first, nullptr, st, n);
     });
+}
+
+int pfac_flows_create(pfac_ctx *ctx, uint32_t n_flows, pfac_flows **out)
+{
+    if (!ctx || !out || n_flows == 0) return set_error(PFAC_ERR_ARG, "bad arguments to pfac_flows_create");
+    if (ctx->batch_rc != PFAC_OK) return set_error(ctx->batch_rc, "%s", ctx->batch_why.c_str());
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DeviceGuard g(ctx->device);
+    std::unique_ptr<pfac_flows> f(new pfac_flows);
+    f->ctx = ctx;
+    f->n_flows = n_flows;
+    f->keep = (uint32_t)std::max(ctx->max_pat_len - 1, 0);
+    f->stride = (f->keep + 15u) & ~15u;
+    if (f->stride) {
+        const int e = f->d_tails.alloc((size_t)n_flows * f->stride);
+        if (e) return e;
+    }
+    f->pos.assign(n_flows, 0);
+    f->seen.assign(n_flows, 0u);
+    *out = f.release();
+    return PFAC_OK;
+}
+
+void pfac_flows_destroy(pfac_flows *f)
+{
+    if (!f) return;
+    std::lock_guard<std::mutex> lk(f->ctx->mu);
+    DeviceGuard g(f->ctx->device);
+    cudaDeviceSynchronize();   // (a failed call may have left work on a stream)
+    delete f;                  // (frees the buffers on the context's device)
+}
+
+int pfac_flows_reset(pfac_flows *f, uint32_t flow)
+{
+    if (!f || flow >= f->n_flows) return set_error(PFAC_ERR_ARG, "bad arguments to pfac_flows_reset");
+    std::lock_guard<std::mutex> lk(f->mu);
+    f->pos[flow] = 0;
+    return PFAC_OK;
+}
+
+int pfac_flows_position(const pfac_flows *f, uint32_t flow, uint64_t *bytes)
+{
+    if (!f || !bytes || flow >= f->n_flows) return set_error(PFAC_ERR_ARG, "bad arguments to pfac_flows_position");
+    std::lock_guard<std::mutex> lk(f->mu);
+    *bytes = f->pos[flow];
+    return PFAC_OK;
+}
+
+int pfac_scan_flows_device_sync(pfac_flows *f, const void *d_in, const uint64_t *chunk_offsets, const uint32_t *flow_ids,
+                                uint32_t n_chunks, void *d_out, uint64_t cap, void *d_chunk_first, uint64_t *base,
+                                uint64_t *count, void *stream)
+{
+    if (!f || !chunk_offsets || (!flow_ids && n_chunks) || (!d_out && cap) || !d_chunk_first || (!base && n_chunks) || !count)
+        return set_error(PFAC_ERR_ARG, "bad arguments to pfac_scan_flows_device_sync");
+    std::lock_guard<std::mutex> lk(f->mu);
+    pfac_ctx *ctx = f->ctx;
+    const int e = run_own(ctx, stream, cap, count, [&](cudaStream_t st, Counters &n) {
+        return launch_flows(f, ctx->own, d_in, chunk_offsets, flow_ids, n_chunks, d_out, cap, d_chunk_first, base, st, n);
+    });
+    if (e) return e;   // nothing committed: the tail kernel wrote no tail either
+    for (uint32_t i = 0; i < n_chunks; i++) f->pos[flow_ids[i]] += chunk_offsets[i + 1] - chunk_offsets[i];
+    return PFAC_OK;
 }
 
 int pfac_host_alloc(void **ptr, size_t bytes)
