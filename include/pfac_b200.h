@@ -149,6 +149,8 @@ int pfac_ctx_device(const pfac_ctx *ctx);
  * d_out: device array of `cap` pfac_match; d_count: device uint64 receiving the number of
  * matches found.  If it exceeds cap nothing is written past d_out[cap) and the contents
  * of d_out are unspecified: size the buffer from the count and scan again.
+ * Size bound per call: min(n_valid, n_starts + max_pat_len - 1) + (d_in & 15) + 12,288 < 2^32
+ * (PFAC_ERR_LIMIT otherwise), i.e. up to 2^32 - 12,289 - (d_in & 15) bytes.
  * Asynchronous on `stream`.  Scans of one context share one working set: a call on another
  * stream than the previous one is ordered after it on the device (use one context per stream
  * for scans that should overlap). */
@@ -169,7 +171,8 @@ int pfac_scan_device_sync(pfac_ctx *ctx, const void *d_in, uint64_t n_starts, ui
  *
  * n_docs independent documents packed back to back in d_in: document i = d_in[doc_offsets[i], doc_offsets[i+1]).
  * doc_offsets is a HOST array of n_docs + 1 entries, doc_offsets[0] = 0, non-decreasing; the total
- * doc_offsets[n_docs] < 4 GiB as for pfac_scan_device.  The array is read before the call returns.
+ * doc_offsets[n_docs] + (d_in & 15) + 12,288 < 2^32 as for pfac_scan_device (PFAC_ERR_LIMIT otherwise).  The array
+ * is read before the call returns.
  * d_out: device array of `cap` pfac_match, pos relative to the record's document; records ordered by
  * (document, pos, pattern length).  d_doc_first: device uint64[n_docs + 1], the records of document i are
  * d_out[d_doc_first[i], d_doc_first[i+1]).  d_count: device uint64.  If the count exceeds cap, nothing is
@@ -209,8 +212,9 @@ int pfac_flows_position(const pfac_flows *f, uint32_t flow, uint64_t *bytes);
  * cap and PFAC_ERR_OUTPUT_FULL as for pfac_scan_batch_device_sync, with the chunks in place of the documents and
  * pos relative to base[i] (a HOST uint64[n_chunks]: base[i] = P_f - t_f, the stream position of the first carried
  * byte), so a record's stream position is base[i] + pos and flows may run past 4 GiB.  PFAC_ERR_ARG for a flow id
- * out of range or named twice, chunk_offsets[0] != 0 or decreasing offsets; PFAC_ERR_LIMIT when the chunks, or
- * the chunks with their carried tails, reach 4 GiB.  All refusals come before anything is enqueued. */
+ * out of range or named twice, chunk_offsets[0] != 0 or decreasing offsets; PFAC_ERR_LIMIT when the chunks reach
+ * 4 GiB or the packed bytes (chunks plus carried tails) + 12,288 reach 2^32.  All refusals come before anything is
+ * enqueued. */
 int pfac_scan_flows_device_sync(pfac_flows *f, const void *d_in, const uint64_t *chunk_offsets,
                                 const uint32_t *flow_ids, uint32_t n_chunks, void *d_out, uint64_t cap,
                                 void *d_chunk_first, uint64_t *base, uint64_t *count, void *stream);

@@ -404,7 +404,8 @@ def test_job_multi_segment_64bit_positions():
     """A shard larger than one 1 GiB segment: records carry 32-bit positions relative to a 64-bit
     segment base (the reference's int positions stop at 2 GiB, main.cc:79).  Properties: globally
     sorted, every record re-verified against its pattern, a match planted across the segment
-    border is found, and the rendered lines carry positions > 2^30."""
+    border is found, and the rendered lines carry positions > 2^30.  Positions at and above 2^31 and segment bases up
+    to 4 GiB: test_job_past_4_GiB in test_large_inputs_gpu.py."""
     torch = torch_cuda()
     pats = synth.synth_patterns(0, 1000, 1, 8, 32)
     lines = pats.split(b"\n")[:-1]
