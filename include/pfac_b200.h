@@ -77,6 +77,16 @@ int pfac_tables_build_mem(const void *pattern_bytes, size_t len, int n_parts, in
  * ctdef.h:37-99: \ooo, \xhh, \a \b \t \n \v \f \r \' \" \\) -- code the reference ships but its
  * main() never calls, hence behind a flag. */
 #define PFAC_PATTERNS_ESCAPES 1u
+/* PFAC_PATTERNS_CASELESS (this project's flag; the reference has no case-insensitive mode) builds a set that
+ * matches ASCII letters in either case.  The fold maps bytes 0x41-0x5A ('A'-'Z') to 0x61-0x7A and leaves every
+ * other byte as it is (no locale, no Unicode: 0xC1-0xDA do not fold).  The patterns are folded after the reader
+ * (so with PFAC_PATTERNS_ESCAPES, \x41 is 'a') and before the sort, so the tables are bit-identical to those of
+ * the folded pattern file, and every scan of such a set folds its text on the device first:
+ *   scan(set of P with PFAC_PATTERNS_CASELESS, T) == scan(set of fold(P), fold(T)), record for record.
+ * Lines equal after folding are duplicates: the last such line owns the match ("GET" then "get": only the
+ * second line's id is reported; pfac_tables_pattern_lengths reports 0 for the first).  One case rule per set:
+ * a set cannot mix caseless and exact patterns. */
+#define PFAC_PATTERNS_CASELESS 2u
 int pfac_tables_build_file_ext(const char *pattern_file, int n_parts, int width, unsigned flags,
                                pfac_tables **out);
 int pfac_tables_build_mem_ext(const void *pattern_bytes, size_t len, int n_parts, int width,
@@ -89,7 +99,9 @@ int pfac_tables_from_arrays(const int32_t *s0, const int32_t *r, int32_t n_r, co
                             int32_t n_final, const int32_t *idmap, int32_t max_pat_len,
                             pfac_tables **out);
 /* On-disk cache of the canonical arrays of every partition (checksummed; the reference rebuilds its
- * tables on every run, main.cc:100-126).  A loaded set scans exactly like the set that was saved. */
+ * tables on every run, main.cc:100-126).  A loaded set scans exactly like the set that was saved,
+ * caseless sets included: they are written as PFACTBL3 files (PFACTBL2 plus the flags), which older
+ * libraries refuse, and case-sensitive sets as PFACTBL2 files.  pfac_tables_load reads both. */
 /* What a table set was built from: a 64-bit hash of the pattern file image and the front-end flags
  * (0 for sets wrapped from arrays).  It travels with pfac_tables_save/_load, so that a cache can be
  * checked against the pattern file it is about to stand in for (pfac_pattern_file_hash). */
@@ -103,6 +115,9 @@ int pfac_tables_n_parts(const pfac_tables *t);
 int pfac_tables_n_patterns(const pfac_tables *t);
 int pfac_tables_max_pat_len(const pfac_tables *t); /* over all partitions, main.cc:59 */
 int pfac_tables_width(const pfac_tables *t);
+/* The front-end flags that change what a set matches: PFAC_PATTERNS_CASELESS or 0 (sets wrapped from arrays
+ * are case-sensitive). */
+unsigned pfac_tables_flags(const pfac_tables *t);
 /* info[0..8] = state_num, n_final, max_len, ht_size, n_r, n_keys, max_key, max_offset, min_len */
 int pfac_tables_part_info(const pfac_tables *t, int part, int32_t info[9]);
 const int32_t *pfac_tables_s0(const pfac_tables *t, int part);    /* 256 entries, main.cc:200 */
@@ -120,13 +135,14 @@ int pfac_tables_derive_check(const pfac_tables *t, int part, uint32_t t2_bytes, 
 /* Diagnostics: how many start positions of `text` survive each stage of the detector's filter
  * cascade (a host model that COUNTS; it reports no matches).  counts[0..8] = positions, T1 pass,
  * prefix found (T2 / level 1), level-1 window pass, level-2 window pass, bypass, starts left as
- * candidates, 512-byte slices flagged, slices. */
+ * candidates, 512-byte slices flagged, slices.  A caseless set counts its folded text, as the scan sees it. */
 int pfac_tables_filter_profile(const pfac_tables *t, int part, uint32_t t2_bytes, uint32_t t3_bytes,
                                uint32_t tm2_bytes, const void *text, uint64_t n, uint64_t counts[12]);
 /* One transition through the PHF exactly as master_kernel.cu:52-64 does it; -1 = none. */
 int32_t pfac_tables_lookup(const pfac_tables *t, int part, int32_t state, int32_t byte);
 /* Pattern length of every id: lengths[id] = depth of the final state that reports id, 0 for ids no final
- * state reports (earlier duplicates).  lengths may be NULL: *n_ids receives max id + 1 (size of the array).
+ * state reports (earlier duplicates, which caseless sets make common: with "GET" and "get" in one file
+ * only the later line's id is ever reported).  lengths may be NULL: *n_ids receives max id + 1 (size of the array).
  * PFAC_ERR_ARG if the automaton is not a tree, PFAC_ERR_OUTPUT_FULL if n < max id + 1. */
 int pfac_tables_pattern_lengths(const pfac_tables *t, int part, int32_t *lengths, int32_t n, int32_t *n_ids);
 
@@ -153,7 +169,11 @@ int pfac_ctx_device(const pfac_ctx *ctx);
  * (PFAC_ERR_LIMIT otherwise), i.e. up to 2^32 - 12,289 - (d_in & 15) bytes.
  * Asynchronous on `stream`.  Scans of one context share one working set: a call on another
  * stream than the previous one is ordered after it on the device (use one context per stream
- * for scans that should overlap). */
+ * for scans that should overlap).
+ * Caseless sets (PFAC_PATTERNS_CASELESS): the caller's bytes are never written; they are folded into a
+ * buffer of the context at the same 16-byte phase, which grows to the largest input scanned so far (up
+ * to 4 GiB) and is held until pfac_ctx_destroy.  pfac_scan_batch_device does the same; pfac_scan_host and
+ * the flow calls fold the library's own copy of the input in place. */
 int pfac_scan_device(pfac_ctx *ctx, const void *d_in, uint64_t n_starts, uint64_t n_valid,
                      uint64_t base_pos, void *d_out, uint64_t cap, void *d_count, void *stream);
 /* Same, synchronous; *count receives the device count.  PFAC_ERR_OUTPUT_FULL if *count > cap. */
@@ -238,7 +258,8 @@ void pfac_host_unregister(const void *ptr);
 
 /* Counters of the last scan on this context (for bench.py's gpu_launches / roofline):
  * info[0] = kernel launches, info[1] = tiles, info[2] = CTAs, info[3] = dynamic smem bytes,
- * info[4] = h2d bytes, info[5] = d2h bytes, info[6] = sub-chunks, info[7] = reserved (0) */
+ * info[4] = h2d bytes, info[5] = d2h bytes, info[6] = sub-chunks, info[7] = reserved (0).  The launches
+ * of a caseless set count the fold kernel of every scan. */
 int pfac_ctx_last_scan_info(const pfac_ctx *ctx, uint64_t info[8]);
 
 /* Optional CUDA-event timing of the detector kernel (pfac_scan_kernel) alone, for roofline

@@ -24,6 +24,9 @@ import numpy as np
 
 from ._lib import PFAC_ERR_OUTPUT_FULL, PfacError, check, lib
 
+PFAC_PATTERNS_ESCAPES = 1
+PFAC_PATTERNS_CASELESS = 2   # include/pfac_b200.h: ASCII letters match in either case
+
 MATCH_DTYPE = np.dtype([("pos", "<u4"), ("id", "<u4")])   # struct pfac_match
 FLOW_MATCH_DTYPE = np.dtype([("pos", "<u8"), ("id", "<u4")])   # a match of a flow: absolute stream position
 
@@ -93,17 +96,19 @@ class Tables:
         self.width = lib.pfac_tables_width(handle)
 
     @classmethod
-    def from_file(cls, path, n_parts=1, width=256, escapes=False):
+    def from_file(cls, path, n_parts=1, width=256, escapes=False, caseless=False):
         h = C.c_void_p()
-        check(lib.pfac_tables_build_file_ext(str(path).encode(), n_parts, width, 1 if escapes else 0, C.byref(h)))
+        check(lib.pfac_tables_build_file_ext(str(path).encode(), n_parts, width, _flags(escapes, caseless), C.byref(h)))
         return cls(h)
 
     @classmethod
-    def from_bytes(cls, data, n_parts=1, width=256, escapes=False):
-        """escapes=True: read_pattern_ext / fgetc_ext front-end (create_table_reorder.c:131, ctdef.h:37)."""
+    def from_bytes(cls, data, n_parts=1, width=256, escapes=False, caseless=False):
+        """escapes=True: read_pattern_ext / fgetc_ext front-end (create_table_reorder.c:131, ctdef.h:37).
+        caseless=True: ASCII letters match in either case (PFAC_PATTERNS_CASELESS): the patterns are folded to
+        lower case after the reader, and every scan with these tables folds its text on the device first."""
         data = bytes(data)
         h = C.c_void_p()
-        check(lib.pfac_tables_build_mem_ext(data, len(data), n_parts, width, 1 if escapes else 0, C.byref(h)))
+        check(lib.pfac_tables_build_mem_ext(data, len(data), n_parts, width, _flags(escapes, caseless), C.byref(h)))
         return cls(h)
 
     @classmethod
@@ -124,6 +129,11 @@ class Tables:
 
     def save(self, path):
         check(lib.pfac_tables_save(self._h, str(path).encode()))
+
+    @property
+    def caseless(self):
+        """True for a set built with caseless=True (also after save / load)."""
+        return bool(lib.pfac_tables_flags(self._h) & PFAC_PATTERNS_CASELESS)
 
     def source_hash(self):
         """Hash of the pattern file image + reader flags the set was built from (0: wrapped from arrays)."""
@@ -171,9 +181,13 @@ class Tables:
         self.close()
 
 
-def pattern_file_hash(path, escapes=False):
+def _flags(escapes, caseless):
+    return (PFAC_PATTERNS_ESCAPES if escapes else 0) | (PFAC_PATTERNS_CASELESS if caseless else 0)
+
+
+def pattern_file_hash(path, escapes=False, caseless=False):
     h = C.c_uint64(0)
-    check(lib.pfac_pattern_file_hash(str(path).encode(), 1 if escapes else 0, C.byref(h)))
+    check(lib.pfac_pattern_file_hash(str(path).encode(), _flags(escapes, caseless), C.byref(h)))
     return h.value
 
 

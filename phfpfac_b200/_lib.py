@@ -17,7 +17,7 @@ ABI_SYMBOLS = [
     "pfac_tables_build_file", "pfac_tables_build_mem", "pfac_tables_build_file_ext", "pfac_tables_build_mem_ext", "pfac_tables_from_arrays", "pfac_tables_save", "pfac_tables_load", "pfac_tables_destroy",
     "pfac_tables_source_hash", "pfac_pattern_file_hash",
     "pfac_tables_n_parts", "pfac_tables_n_patterns", "pfac_tables_max_pat_len", "pfac_tables_width",
-    "pfac_tables_part_info", "pfac_tables_s0", "pfac_tables_r", "pfac_tables_HT", "pfac_tables_val",
+    "pfac_tables_flags", "pfac_tables_part_info", "pfac_tables_s0", "pfac_tables_r", "pfac_tables_HT", "pfac_tables_val",
     "pfac_tables_idmap", "pfac_tables_lookup", "pfac_tables_pattern_lengths", "pfac_tables_derive_check",
     "pfac_tables_filter_profile",
     "pfac_device_count", "pfac_ctx_create", "pfac_ctx_destroy", "pfac_ctx_device",
@@ -70,6 +70,8 @@ def _load():
     lib.pfac_tables_destroy.restype = None
     for n in ("pfac_tables_n_parts", "pfac_tables_n_patterns", "pfac_tables_max_pat_len", "pfac_tables_width"):
         getattr(lib, n).argtypes = [_vp]
+    lib.pfac_tables_flags.argtypes = [_vp]
+    lib.pfac_tables_flags.restype = C.c_uint
     lib.pfac_tables_part_info.argtypes = [_vp, C.c_int, _i32p]
     for n in ("pfac_tables_s0", "pfac_tables_r", "pfac_tables_HT", "pfac_tables_val", "pfac_tables_idmap"):
         getattr(lib, n).argtypes = [_vp, C.c_int]

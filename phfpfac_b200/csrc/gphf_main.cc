@@ -68,9 +68,11 @@ int main(int argc, char **argv)
     double t0 = now();
     pfac_tables *tables = nullptr;
     // GPHF_ESCAPES=1: read the patterns through the reference's (unused) escape reader, read_pattern_ext
-    const unsigned pflags = getenv("GPHF_ESCAPES") && atoi(getenv("GPHF_ESCAPES")) ? PFAC_PATTERNS_ESCAPES : 0u;
+    // GPHF_CASELESS=1: ASCII letters match in either case (PFAC_PATTERNS_CASELESS)
+    const unsigned pflags = (getenv("GPHF_ESCAPES") && atoi(getenv("GPHF_ESCAPES")) ? PFAC_PATTERNS_ESCAPES : 0u) |
+                            (getenv("GPHF_CASELESS") && atoi(getenv("GPHF_CASELESS")) ? PFAC_PATTERNS_CASELESS : 0u);
     // GPHF_TABLE_CACHE=<file>: load the tables from it if it exists and was built from this pattern file
-    // (hash of the file image + escape flag in the cache header) at this width, else build them and write it
+    // (hash of the file image + front-end flags in the cache header) at this width, else build them and write it
     const char *cache = getenv("GPHF_TABLE_CACHE");
     bool from_cache = false;
     if (cache && *cache) {
@@ -81,8 +83,8 @@ int main(int argc, char **argv)
             uint64_t want = 0;
             if (pfac_pattern_file_hash(argv[1], pflags, &want)) return fail("read the pattern file");
             if (pfac_tables_width(tables) != width || pfac_tables_n_parts(tables) != 1 ||
-                pfac_tables_source_hash(tables) != want) {
-                // built from another pattern file, width or escape setting: rebuild (and rewrite the cache)
+                pfac_tables_source_hash(tables) != want || pfac_tables_flags(tables) != (pflags & PFAC_PATTERNS_CASELESS)) {
+                // built from another pattern file, width or front-end flags: rebuild (and rewrite the cache)
                 fprintf(stderr, "%s does not belong to this pattern file / width: rebuilding the tables\n", cache);
                 pfac_tables_destroy(tables);
                 tables = nullptr;

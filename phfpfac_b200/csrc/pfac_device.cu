@@ -11,6 +11,7 @@
 #include "pfac_batch.cuh"
 #include "pfac_derive.h"
 #include "pfac_flows.cuh"
+#include "pfac_fold.cuh"
 #include "pfac_internal.h"
 #include "pfac_kernel.cuh"
 
@@ -138,6 +139,9 @@ struct Slot {
     Buf<uint32_t> d_kpos;
     Staging doc;
     Buf<unsigned long long> d_blk;
+    // caseless sets: the folded copy of caller-owned input (pfac_scan_device, pfac_scan_batch_device) at the
+    // input's 16-byte phase; grows to the largest input scanned and is held until pfac_ctx_destroy
+    Buf<uint8_t> d_fold;
 };
 
 struct Stage {   // one pipeline stage of pfac_scan_host
@@ -176,6 +180,7 @@ struct pfac_ctx {
     Buf<uint8_t> d_wcache;  // walk cache of the dense-match kernel (pfac_derive.h)
     size_t dense_smem = 0;
     bool dense_first = false;      // no detector: the dense-match kernel walks every tile (sets with patterns <= 3 bytes)
+    bool caseless = false;         // PFAC_PATTERNS_CASELESS: every scan folds its input first (pfac_fold.cuh)
     // batch scans: pattern length of every id; batch_rc != PFAC_OK: the set does not support them (batch_why)
     Buf<int32_t> d_patlen;
     uint32_t n_ids = 0;
@@ -319,8 +324,11 @@ int slot_init(Slot &s)
 
 // Enqueue one scan (scan kernel + ordering pass) on `stream`.  On completion slot.d_result holds
 // {count, error}; d_count (optional, device) receives the count as well.  n: launches, tiles and CTAs.
+// own_input: d_in is the library's own buffer (a host scan's stage, a flow call's packed buffer), which a caseless
+// set folds in place; the caller's input is folded into slot.d_fold instead and never written.
 int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, uint64_t n_valid, uint64_t base_pos,
-                uint32_t pos_bias, void *d_out, uint64_t cap, void *d_count, cudaStream_t stream, Counters &n)
+                uint32_t pos_bias, void *d_out, uint64_t cap, void *d_count, cudaStream_t stream, Counters &n,
+                bool own_input)
 {
     if (n_valid < n_starts) return set_error(PFAC_ERR_ARG, "n_valid < n_starts");
     const uint64_t useful = n_starts + (uint64_t)(ctx->max_pat_len > 0 ? ctx->max_pat_len - 1 : 0);
@@ -347,6 +355,23 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
     } guard{slot};
     if (ctx->n_stages < (uint32_t)min_stages((int)ctx->dv.mode))
         return set_error(PFAC_ERR_INTERNAL, "input ring of %u stages is too shallow for the slot scheme", ctx->n_stages);
+    uint64_t folds = 0;
+    if (ctx->caseless) {   // the fold of the bytes the scan reads, at the input's phase: mis and every bound stay
+        uint8_t *out_al = const_cast<uint8_t *>((const uint8_t *)d_in - mis);
+        if (!own_input) {
+            if ((e = slot.d_fold.reserve((size_t)(mis + n_valid), 0, stream))) return e;
+            out_al = slot.d_fold.get();
+        }
+        const uint64_t words = (mis + n_valid + 15) / 16;
+        const uint32_t fg = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((words + kFoldThreads * kFoldUnroll - 1) /
+                                                                                   (kFoldThreads * kFoldUnroll),
+                                                                               4ull * (uint64_t)ctx->sm_count));
+        const cudaLaunchConfig_t fl = launch_config(ctx, stream, fg, kFoldThreads, 0);
+        CU_TRY(cudaLaunchKernelEx(&fl, pfac_fold_kernel, (const uint8_t *)d_in - mis, out_al, (unsigned long long)mis,
+                                  (unsigned long long)(mis + n_valid)));
+        d_in = out_al + mis;
+        folds = 1;
+    }
     ScanParams p = ctx->scan;
     p.in_al = (const uint8_t *)d_in - mis;
     p.mis = mis;
@@ -440,7 +465,7 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
         const cudaLaunchConfig_t fl = launch_config(ctx, stream, fgrid, kFinThreads, 0);
         CU_TRY(cudaLaunchKernelEx(&fl, pfac_finalize_kernel, f));
     }
-    n.launches = dense_first ? 1 : 3;
+    n.launches = (dense_first ? 1 : 3) + folds;
     n.tiles = p.n_tiles;
     n.ctas = grid;
     slot.flip++;
@@ -525,7 +550,7 @@ int launch_batch(pfac_ctx *ctx, Slot &slot, const void *d_in, const uint64_t *do
     });
     if (e) return e;
 
-    e = launch_scan(ctx, slot, d_in, total, total, 0, 0u, slot.d_raw.get(), slot.d_raw.cap(), nullptr, stream, n);
+    e = launch_scan(ctx, slot, d_in, total, total, 0, 0u, slot.d_raw.get(), slot.d_raw.cap(), nullptr, stream, n, false);
     if (e) return e;
     e = launch_split<false>(ctx, slot, grid, slot.doc.d.get(), nullptr, n_docs, d_out, cap, d_doc_first, d_count, stream, n);
     if (e) return e;
@@ -601,7 +626,7 @@ int launch_flows(pfac_flows *f, Slot &slot, const void *d_in, const uint64_t *ch
     CU_TRY(cudaLaunchKernelEx(&pl, pfac_flow_pack_kernel, fp));
     n.launches = 1;
     Counters k;
-    e = launch_scan(ctx, slot, fp.packed, packed, packed, 0, 0u, slot.d_raw.get(), slot.d_raw.cap(), nullptr, stream, k);
+    e = launch_scan(ctx, slot, fp.packed, packed, packed, 0, 0u, slot.d_raw.get(), slot.d_raw.cap(), nullptr, stream, k, true);
     if (e) return e;
     n.launches += k.launches;
     n.tiles = k.tiles;
@@ -875,6 +900,7 @@ int pfac_ctx_create(int device, const pfac_tables *t, int part, int n_streams, s
         (e = upload_walk_cache(*ctx, P, smem_max)) || (e = upload_pattern_lengths(*ctx, P)))
         return e;
     ctx->dense_first = ctx->dv.has_short != 0;
+    ctx->caseless = (t->flags & PFAC_PATTERNS_CASELESS) != 0;
     if (const char *v = getenv("PFAC_DENSE_FIRST")) ctx->dense_first = atoi(v) != 0;   // experiments: force either path
     ctx->dv.image.clear();
     ctx->dv.image.shrink_to_fit();
@@ -962,7 +988,7 @@ int pfac_scan_device(pfac_ctx *ctx, const void *d_in, uint64_t n_starts, uint64_
 {
     if (!ctx || (!d_in && n_starts) || (!d_out && cap) || !d_count) return set_error(PFAC_ERR_ARG, "bad arguments to pfac_scan_device");
     return run_own(ctx, stream, cap, nullptr, [&](cudaStream_t st, Counters &n) {
-        return launch_scan(ctx, ctx->own, d_in, n_starts, n_valid, base_pos, 0u, d_out, cap, d_count, st, n);
+        return launch_scan(ctx, ctx->own, d_in, n_starts, n_valid, base_pos, 0u, d_out, cap, d_count, st, n, false);
     });
 }
 
@@ -971,7 +997,7 @@ int pfac_scan_device_sync(pfac_ctx *ctx, const void *d_in, uint64_t n_starts, ui
 {
     if (!ctx || !count || (!d_in && n_starts) || (!d_out && cap)) return set_error(PFAC_ERR_ARG, "bad arguments to pfac_scan_device_sync");
     return run_own(ctx, stream, cap, count, [&](cudaStream_t st, Counters &n) {
-        return launch_scan(ctx, ctx->own, d_in, n_starts, n_valid, base_pos, 0u, d_out, cap, nullptr, st, n);
+        return launch_scan(ctx, ctx->own, d_in, n_starts, n_valid, base_pos, 0u, d_out, cap, nullptr, st, n, false);
     });
 }
 
@@ -1144,7 +1170,7 @@ int pfac_scan_host(pfac_ctx *ctx, const void *h_in, uint64_t n_starts, uint64_t 
         n.h2d += nv;
         Counters k;
         int e = launch_scan(ctx, st.slot, st.d_in.get(), ns, nv, base_pos + off, (uint32_t)off, st.d_out.get(),
-                            st.d_out.cap(), nullptr, st.stream, k);
+                            st.d_out.cap(), nullptr, st.stream, k, true);
         if (e) return e;
         n.launches += k.launches;
         n.tiles += k.tiles;

@@ -46,4 +46,5 @@ struct pfac_tables {
     int width = 256;
     std::vector<pfac::Partition> parts;
     uint64_t source_hash = 0;   // FNV-1a of the pattern file image + flags the set was built from (0: unknown)
+    unsigned flags = 0;         // PFAC_PATTERNS_CASELESS when the set matches ASCII letters in either case
 };

@@ -98,10 +98,6 @@ int read_patterns(const unsigned char *buf, size_t len, std::vector<Pattern> &ou
         out.push_back(Pattern{buf + i, (int)plen, (int)out.size() + 1});
         i += plen + 1;
     }
-    // qsort(&all_pattern[1], ...) (:116).  glibc's qsort is a stable merge sort, so equal
-    // patterns keep file order and the LAST duplicate wins its final state (:366).
-    std::stable_sort(out.begin(), out.end(),
-                     [](const Pattern &a, const Pattern &b) { return comp_pat(a, b) < 0; });
     return PFAC_OK;
 }
 
@@ -181,10 +177,11 @@ int read_patterns_ext(const unsigned char *buf, size_t len, std::vector<unsigned
         out.push_back(Pattern{arena.data() + start, (int)plen, (int)out.size() + 1});
         if (i >= len) break;
     }
-    std::stable_sort(out.begin(), out.end(),
-                     [](const Pattern &a, const Pattern &b) { return comp_pat(a, b) < 0; });
     return PFAC_OK;
 }
+
+// PFAC_PATTERNS_CASELESS: ASCII 'A'-'Z' -> 'a'-'z', every other byte (0x80-0xFF included) unchanged
+inline unsigned char ascii_fold(unsigned char c) { return (c >= 'A' && c <= 'Z') ? (unsigned char)(c | 0x20) : c; }
 
 // create_table_reorder.c:277-378 (patternsToPFAC) for an already sorted slice.
 // State numbering: finals 0..n-1 = index in the slice (:366), n unused, initial n+1 (:288),
@@ -483,11 +480,28 @@ int build(const unsigned char *buf, size_t len, int n_parts, int width, unsigned
         return set_error(PFAC_ERR_WIDTH, "width must be a power of two in [1,4096], got %d", width);
     std::vector<Pattern> pats;
     std::vector<unsigned char> arena;
-    int e = (flags & PFAC_PATTERNS_ESCAPES) ? read_patterns_ext(buf, len, arena, pats) : read_patterns(buf, len, pats);
+    const bool caseless = (flags & PFAC_PATTERNS_CASELESS) != 0;
+    int e;
+    if (flags & PFAC_PATTERNS_ESCAPES) {
+        e = read_patterns_ext(buf, len, arena, pats);
+    } else if (caseless) {   // the plain reader's patterns point into the image: fold a copy of it
+        arena.assign(buf, buf + len);
+        e = read_patterns(arena.data(), len, pats);
+    } else {
+        e = read_patterns(buf, len, pats);
+    }
     if (e) return e;
+    // the fold comes after the reader (an escaped \x41 is 'A', then 'a') and before the sort, so that lines equal
+    // after folding are duplicates like any other
+    if (caseless)
+        for (unsigned char &c : arena) c = ascii_fold(c);
+    // qsort(&all_pattern[1], ...) (create_table_reorder.c:116).  glibc's qsort is a stable merge sort, so equal
+    // patterns keep file order and the LAST duplicate wins its final state (:366).
+    std::stable_sort(pats.begin(), pats.end(), [](const Pattern &a, const Pattern &b) { return comp_pat(a, b) < 0; });
     std::unique_ptr<pfac_tables> t(new pfac_tables);
     t->n_patterns = (int)pats.size();
     t->width = width;
+    t->flags = flags & PFAC_PATTERNS_CASELESS;
     t->parts.resize((size_t)n_parts);
     const int n = (int)pats.size();
     const int k = n / n_parts;            // create_table_reorder.c:220
@@ -668,6 +682,8 @@ int pfac_tables_from_arrays(const int32_t *s0, const int32_t *r, int32_t n_r, co
 // ---- on-disk cache of the canonical arrays (the reference serialises nothing: it rebuilds the trie
 // and the PHF on every run, main.cc:100-126).  Little-endian int32 fields:
 //   "PFACTBL2", n_parts, n_patterns, max_pat_len, width, source hash (u64: pattern file image + flags),
+//   ["PFACTBL3" only: u32 flags (PFAC_PATTERNS_CASELESS): written for caseless sets alone, so that a case-sensitive
+//    set writes the same file as before and a library that does not know the flag refuses the cache by its magic],
 //   per partition: state_num, n_final, max_len, min_len, width, n_keys, max_key, max_row, max_offset,
 //                  ht_size, n_r, then s0[256], r[n_r], HT[ht_size], val[ht_size], idmap[n_final],
 //   FNV-1a 64 of everything before it.
@@ -699,9 +715,10 @@ int pfac_tables_save(const pfac_tables *t, const char *path)
     FILE *f = fopen(path, "wb");
     if (!f) return set_error(PFAC_ERR_IO, "cannot create %s", path);
     Fnv h;
-    bool ok = put(f, h, "PFACTBL2", 8);
+    const uint32_t flags = t->flags;
+    bool ok = put(f, h, flags ? "PFACTBL3" : "PFACTBL2", 8);
     const int32_t head[4] = {(int32_t)t->parts.size(), t->n_patterns, t->max_pat_len, t->width};
-    ok = ok && put(f, h, head, sizeof head) && put(f, h, &t->source_hash, 8);
+    ok = ok && put(f, h, head, sizeof head) && put(f, h, &t->source_hash, 8) && (!flags || put(f, h, &flags, 4));
     for (const Partition &P : t->parts) {
         const int32_t ph[11] = {P.state_num, P.n_final, P.max_len, P.min_len, P.width, P.n_keys, P.max_key, P.max_row,
                                 P.max_offset, P.ht_size, (int32_t)P.r.size()};
@@ -730,13 +747,17 @@ int pfac_tables_load(const char *path, pfac_tables **out)
         Fnv h;
         char magic[8];
         int32_t head[4];
-        if (!get(f, h, magic, 8) || memcmp(magic, "PFACTBL2", 8) != 0) return bad("magic");
+        if (!get(f, h, magic, 8) || (memcmp(magic, "PFACTBL2", 8) != 0 && memcmp(magic, "PFACTBL3", 8) != 0)) return bad("magic");
+        const bool v3 = magic[7] == '3';
         uint64_t src_hash = 0;
+        uint32_t flags = 0;
         if (!get(f, h, head, sizeof head) || !get(f, h, &src_hash, 8) || head[0] < 1 || head[0] > (1 << 20) || head[1] < 0 ||
             head[2] < 0 || width_bits(head[3]) < 0)
             return bad("header");
+        if (v3 && (!get(f, h, &flags, 4) || flags != PFAC_PATTERNS_CASELESS)) return bad("flags");
         std::unique_ptr<pfac_tables> t(new pfac_tables);
         t->source_hash = src_hash;
+        t->flags = flags;
         t->n_patterns = head[1];
         t->max_pat_len = head[2];
         t->width = head[3];
@@ -785,6 +806,7 @@ int pfac_tables_n_parts(const pfac_tables *t) { return t ? (int)t->parts.size() 
 int pfac_tables_n_patterns(const pfac_tables *t) { return t ? t->n_patterns : 0; }
 int pfac_tables_max_pat_len(const pfac_tables *t) { return t ? t->max_pat_len : 0; }
 int pfac_tables_width(const pfac_tables *t) { return t ? t->width : 0; }
+unsigned pfac_tables_flags(const pfac_tables *t) { return t ? t->flags : 0u; }
 
 static const Partition *part_of(const pfac_tables *t, int part)
 {
@@ -885,6 +907,12 @@ int pfac_tables_filter_profile(const pfac_tables *t, int part, uint32_t t2_bytes
     try {
         Derived d;
         derive_tables(*P, t2_bytes, t3_bytes, tm2_bytes, d);
+        std::vector<uint8_t> folded;   // a caseless set counts the text its scans see
+        if (t->flags & PFAC_PATTERNS_CASELESS) {
+            folded.assign((const uint8_t *)text, (const uint8_t *)text + n);
+            for (uint8_t &c : folded) c = ascii_fold(c);
+            text = folded.data();
+        }
         derive_profile(*P, d, (const uint8_t *)text, (size_t)n, counts);
         return PFAC_OK;
     } catch (const std::bad_alloc &) {
