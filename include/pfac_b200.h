@@ -84,13 +84,34 @@ int pfac_tables_build_mem(const void *pattern_bytes, size_t len, int n_parts, in
  * the folded pattern file, and every scan of such a set folds its text on the device first:
  *   scan(set of P with PFAC_PATTERNS_CASELESS, T) == scan(set of fold(P), fold(T)), record for record.
  * Lines equal after folding are duplicates: the last such line owns the match ("GET" then "get": only the
- * second line's id is reported; pfac_tables_pattern_lengths reports 0 for the first).  One case rule per set:
- * a set cannot mix caseless and exact patterns. */
+ * second line's id is reported; pfac_tables_pattern_lengths reports 0 for the first).  This flag gives the whole
+ * set one case rule; the _rules calls below give one rule per pattern. */
 #define PFAC_PATTERNS_CASELESS 2u
 int pfac_tables_build_file_ext(const char *pattern_file, int n_parts, int width, unsigned flags,
                                pfac_tables **out);
 int pfac_tables_build_mem_ext(const void *pattern_bytes, size_t len, int n_parts, int width,
                               unsigned flags, pfac_tables **out);
+/* Per-pattern case rules (DESIGN.md section 3.11).  caseless[i] is the rule of pattern id i + 1 (one per pattern
+ * the reader returns, so with PFAC_PATTERNS_ESCAPES one per decoded pattern): 1 matches ASCII letters in either
+ * case, fold(T[pos, pos+L)) == fold(p); 0 matches byte for byte, T[pos, pos+L) == p.  Two lines are duplicates
+ * (the last one owns the match) iff they have the same rule and are equal under it; an exact and a caseless line
+ * never are, so several ids can report at one (pos, length): records are ordered by (pos, length, id).  flags may
+ * be PFAC_PATTERNS_ESCAPES or 0.  PFAC_ERR_ARG for PFAC_PATTERNS_CASELESS in flags, a NULL rules pointer, a rule
+ * other than 0 or 1, and n_patterns != the number of patterns the reader returns.
+ * All 1 builds exactly the PFAC_PATTERNS_CASELESS set of the file, all 0 exactly the plain set (same tables,
+ * flags, source hash and cache file).  Mixed rules build the automaton of the folded patterns -- bit-identical to
+ * the caseless build -- plus verify tables: every scan folds its text out of place, the unchanged detector reports
+ * owner ids, and a verify pass expands each record to the members of its owner that pass (exact members are
+ * compared with the original bytes).  pfac_tables_flags reports PFAC_PATTERNS_CASE_RULES for such a set; the
+ * flag is never passed in. */
+#define PFAC_PATTERNS_CASE_RULES 4u
+int pfac_tables_build_file_rules(const char *pattern_file, int n_parts, int width, unsigned flags,
+                                 const uint8_t *caseless, uint32_t n_patterns, pfac_tables **out);
+int pfac_tables_build_mem_rules(const void *pattern_bytes, size_t len, int n_parts, int width, unsigned flags,
+                                const uint8_t *caseless, uint32_t n_patterns, pfac_tables **out);
+/* The rules of any set, one per pattern (n = pfac_tables_n_patterns, PFAC_ERR_ARG otherwise): all 1 for caseless
+ * sets, all 0 for plain sets and sets wrapped from arrays. */
+int pfac_tables_case_rules(const pfac_tables *t, uint8_t *caseless, uint32_t n);
 /* Wrap caller-built canonical arrays (the thread_data fields of main.cc:19-32) as a
  * one-partition table set; arrays are copied.  n_r = state_num*256/width + 1
  * (master_kernel.cu:221). */
@@ -100,13 +121,18 @@ int pfac_tables_from_arrays(const int32_t *s0, const int32_t *r, int32_t n_r, co
                             pfac_tables **out);
 /* On-disk cache of the canonical arrays of every partition (checksummed; the reference rebuilds its
  * tables on every run, main.cc:100-126).  A loaded set scans exactly like the set that was saved,
- * caseless sets included: they are written as PFACTBL3 files (PFACTBL2 plus the flags), which older
- * libraries refuse, and case-sensitive sets as PFACTBL2 files.  pfac_tables_load reads both. */
+ * caseless and mixed sets included: they are written as PFACTBL3 files (PFACTBL2 plus the flags; a mixed set
+ * adds its rules and verify tables under the checksum), which older libraries refuse, and case-sensitive sets as
+ * PFACTBL2 files.  pfac_tables_load reads both. */
 /* What a table set was built from: a 64-bit hash of the pattern file image and the front-end flags
  * (0 for sets wrapped from arrays).  It travels with pfac_tables_save/_load, so that a cache can be
  * checked against the pattern file it is about to stand in for (pfac_pattern_file_hash). */
 uint64_t pfac_tables_source_hash(const pfac_tables *t);
 int pfac_pattern_file_hash(const char *pattern_file, unsigned flags, uint64_t *hash);
+/* The source hash of the set pfac_tables_build_file_rules builds: FNV over the image, the flags and the rule
+ * bytes for mixed rules, the uniform set's hash for uniform ones.  The refusals of the builder apply. */
+int pfac_pattern_file_hash_rules(const char *pattern_file, unsigned flags, const uint8_t *caseless,
+                                 uint32_t n_patterns, uint64_t *hash);
 int pfac_tables_save(const pfac_tables *t, const char *path);
 int pfac_tables_load(const char *path, pfac_tables **out);
 void pfac_tables_destroy(pfac_tables *t);
@@ -115,8 +141,8 @@ int pfac_tables_n_parts(const pfac_tables *t);
 int pfac_tables_n_patterns(const pfac_tables *t);
 int pfac_tables_max_pat_len(const pfac_tables *t); /* over all partitions, main.cc:59 */
 int pfac_tables_width(const pfac_tables *t);
-/* The front-end flags that change what a set matches: PFAC_PATTERNS_CASELESS or 0 (sets wrapped from arrays
- * are case-sensitive). */
+/* The front-end flags that change what a set matches: PFAC_PATTERNS_CASELESS, PFAC_PATTERNS_CASE_RULES (mixed
+ * per-pattern rules) or 0 (sets wrapped from arrays are case-sensitive). */
 unsigned pfac_tables_flags(const pfac_tables *t);
 /* info[0..8] = state_num, n_final, max_len, ht_size, n_r, n_keys, max_key, max_offset, min_len */
 int pfac_tables_part_info(const pfac_tables *t, int part, int32_t info[9]);
@@ -135,14 +161,17 @@ int pfac_tables_derive_check(const pfac_tables *t, int part, uint32_t t2_bytes, 
 /* Diagnostics: how many start positions of `text` survive each stage of the detector's filter
  * cascade (a host model that COUNTS; it reports no matches).  counts[0..8] = positions, T1 pass,
  * prefix found (T2 / level 1), level-1 window pass, level-2 window pass, bypass, starts left as
- * candidates, 512-byte slices flagged, slices.  A caseless set counts its folded text, as the scan sees it. */
+ * candidates, 512-byte slices flagged, slices.  A caseless or mixed set counts its folded text, as the detector
+ * sees it. */
 int pfac_tables_filter_profile(const pfac_tables *t, int part, uint32_t t2_bytes, uint32_t t3_bytes,
                                uint32_t tm2_bytes, const void *text, uint64_t n, uint64_t counts[12]);
 /* One transition through the PHF exactly as master_kernel.cu:52-64 does it; -1 = none. */
 int32_t pfac_tables_lookup(const pfac_tables *t, int part, int32_t state, int32_t byte);
 /* Pattern length of every id: lengths[id] = depth of the final state that reports id, 0 for ids no final
  * state reports (earlier duplicates, which caseless sets make common: with "GET" and "get" in one file
- * only the later line's id is ever reported).  lengths may be NULL: *n_ids receives max id + 1 (size of the array).
+ * only the later line's id is ever reported).  A mixed set (PFAC_PATTERNS_CASE_RULES) reports the length of every
+ * member of its verify tables, so 0 only for lines shadowed within their rule class.
+ * lengths may be NULL: *n_ids receives max id + 1 (size of the array).
  * PFAC_ERR_ARG if the automaton is not a tree, PFAC_ERR_OUTPUT_FULL if n < max id + 1. */
 int pfac_tables_pattern_lengths(const pfac_tables *t, int part, int32_t *lengths, int32_t n, int32_t *n_ids);
 
@@ -173,7 +202,14 @@ int pfac_ctx_device(const pfac_ctx *ctx);
  * Caseless sets (PFAC_PATTERNS_CASELESS): the caller's bytes are never written; they are folded into a
  * buffer of the context at the same 16-byte phase, which grows to the largest input scanned so far (up
  * to 4 GiB) and is held until pfac_ctx_destroy.  pfac_scan_batch_device does the same; pfac_scan_host and
- * the flow calls fold the library's own copy of the input in place. */
+ * the flow calls fold the library's own copy of the input in place.
+ * Mixed sets (PFAC_PATTERNS_CASE_RULES) fold every input out of place, the library's own buffers included (the
+ * exact patterns are checked against the original bytes, and a flow's carried tails stay unfolded): one folded
+ * buffer per pipeline stage of pfac_scan_host, one of the packed-buffer size for flow calls, and one for the
+ * caller's input, each held until pfac_ctx_destroy.  The detector's records (owner ids) go to a buffer of
+ * max(cap, 4096) records; the verify pass expands them into d_out.  If the detector's records overflow that
+ * buffer, the count returned is their count times the largest group (a capacity with which a rescan fits);
+ * if only the expanded records overflow, the count is exact.  Either way nothing is written past d_out[cap). */
 int pfac_scan_device(pfac_ctx *ctx, const void *d_in, uint64_t n_starts, uint64_t n_valid,
                      uint64_t base_pos, void *d_out, uint64_t cap, void *d_count, void *stream);
 /* Same, synchronous; *count receives the device count.  PFAC_ERR_OUTPUT_FULL if *count > cap. */
@@ -259,7 +295,8 @@ void pfac_host_unregister(const void *ptr);
 /* Counters of the last scan on this context (for bench.py's gpu_launches / roofline):
  * info[0] = kernel launches, info[1] = tiles, info[2] = CTAs, info[3] = dynamic smem bytes,
  * info[4] = h2d bytes, info[5] = d2h bytes, info[6] = sub-chunks, info[7] = reserved (0).  The launches
- * of a caseless set count the fold kernel of every scan. */
+ * of a caseless set count the fold kernel of every scan; those of a mixed set (PFAC_PATTERNS_CASE_RULES) count
+ * the fold and the two kernels of the verify pass of every scan (caseless launches + 2). */
 int pfac_ctx_last_scan_info(const pfac_ctx *ctx, uint64_t info[8]);
 
 /* Optional CUDA-event timing of the detector kernel (pfac_scan_kernel) alone, for roofline

@@ -26,6 +26,7 @@ from ._lib import PFAC_ERR_OUTPUT_FULL, PfacError, check, lib
 
 PFAC_PATTERNS_ESCAPES = 1
 PFAC_PATTERNS_CASELESS = 2   # include/pfac_b200.h: ASCII letters match in either case
+PFAC_PATTERNS_CASE_RULES = 4   # include/pfac_b200.h: a set with per-pattern case rules (reported, never passed in)
 
 MATCH_DTYPE = np.dtype([("pos", "<u4"), ("id", "<u4")])   # struct pfac_match
 FLOW_MATCH_DTYPE = np.dtype([("pos", "<u8"), ("id", "<u4")])   # a match of a flow: absolute stream position
@@ -98,17 +99,29 @@ class Tables:
     @classmethod
     def from_file(cls, path, n_parts=1, width=256, escapes=False, caseless=False):
         h = C.c_void_p()
-        check(lib.pfac_tables_build_file_ext(str(path).encode(), n_parts, width, _flags(escapes, caseless), C.byref(h)))
+        rules = _rules(caseless)
+        if rules is None:
+            check(lib.pfac_tables_build_file_ext(str(path).encode(), n_parts, width, _flags(escapes, caseless), C.byref(h)))
+        else:
+            check(lib.pfac_tables_build_file_rules(str(path).encode(), n_parts, width, _flags(escapes, False),
+                                                   rules.ctypes.data, len(rules), C.byref(h)))
         return cls(h)
 
     @classmethod
     def from_bytes(cls, data, n_parts=1, width=256, escapes=False, caseless=False):
         """escapes=True: read_pattern_ext / fgetc_ext front-end (create_table_reorder.c:131, ctdef.h:37).
         caseless=True: ASCII letters match in either case (PFAC_PATTERNS_CASELESS): the patterns are folded to
-        lower case after the reader, and every scan with these tables folds its text on the device first."""
+        lower case after the reader, and every scan with these tables folds its text on the device first.
+        caseless=[bool per pattern]: per-pattern case rules (one per pattern the reader returns): True matches in
+        either case, False byte for byte.  Uniform rules give exactly the caseless=True / False set."""
         data = bytes(data)
         h = C.c_void_p()
-        check(lib.pfac_tables_build_mem_ext(data, len(data), n_parts, width, _flags(escapes, caseless), C.byref(h)))
+        rules = _rules(caseless)
+        if rules is None:
+            check(lib.pfac_tables_build_mem_ext(data, len(data), n_parts, width, _flags(escapes, caseless), C.byref(h)))
+        else:
+            check(lib.pfac_tables_build_mem_rules(data, len(data), n_parts, width, _flags(escapes, False),
+                                                  rules.ctypes.data, len(rules), C.byref(h)))
         return cls(h)
 
     @classmethod
@@ -132,8 +145,16 @@ class Tables:
 
     @property
     def caseless(self):
-        """True for a set built with caseless=True (also after save / load)."""
+        """True for a set built with caseless=True or all rules True (also after save / load); False for mixed rules."""
         return bool(lib.pfac_tables_flags(self._h) & PFAC_PATTERNS_CASELESS)
+
+    @property
+    def case_rules(self):
+        """np.uint8[n_patterns]: 1 where pattern id i + 1 matches in either case, 0 where it matches byte for byte."""
+        out = np.zeros(self.n_patterns, dtype=np.uint8)
+        if self.n_patterns:
+            check(lib.pfac_tables_case_rules(self._h, out.ctypes.data, len(out)))
+        return out
 
     def source_hash(self):
         """Hash of the pattern file image + reader flags the set was built from (0: wrapped from arrays)."""
@@ -181,13 +202,26 @@ class Tables:
         self.close()
 
 
+def _rules(caseless):
+    """None for one rule for the whole set (a bool), else the per-pattern rules as a uint8 array."""
+    if np.ndim(caseless) == 0:
+        return None
+    return np.ascontiguousarray([1 if c else 0 for c in caseless], dtype=np.uint8)
+
+
 def _flags(escapes, caseless):
     return (PFAC_PATTERNS_ESCAPES if escapes else 0) | (PFAC_PATTERNS_CASELESS if caseless else 0)
 
 
 def pattern_file_hash(path, escapes=False, caseless=False):
+    """The source hash of the set from_file(path, escapes=..., caseless=...) builds (caseless: a bool or one per pattern)."""
     h = C.c_uint64(0)
-    check(lib.pfac_pattern_file_hash(str(path).encode(), _flags(escapes, caseless), C.byref(h)))
+    rules = _rules(caseless)
+    if rules is None:
+        check(lib.pfac_pattern_file_hash(str(path).encode(), _flags(escapes, caseless), C.byref(h)))
+    else:
+        check(lib.pfac_pattern_file_hash_rules(str(path).encode(), _flags(escapes, False), rules.ctypes.data, len(rules),
+                                               C.byref(h)))
     return h.value
 
 

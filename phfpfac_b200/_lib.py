@@ -14,7 +14,9 @@ LIB_PATH = os.environ.get("PFAC_B200_LIB") or os.path.join(PKG_DIR, "_build", "l
 # every symbol include/pfac_b200.h declares
 ABI_SYMBOLS = [
     "pfac_last_error", "pfac_abi_version",
-    "pfac_tables_build_file", "pfac_tables_build_mem", "pfac_tables_build_file_ext", "pfac_tables_build_mem_ext", "pfac_tables_from_arrays", "pfac_tables_save", "pfac_tables_load", "pfac_tables_destroy",
+    "pfac_tables_build_file", "pfac_tables_build_mem", "pfac_tables_build_file_ext", "pfac_tables_build_mem_ext",
+    "pfac_tables_build_file_rules", "pfac_tables_build_mem_rules", "pfac_tables_case_rules", "pfac_pattern_file_hash_rules",
+    "pfac_tables_from_arrays", "pfac_tables_save", "pfac_tables_load", "pfac_tables_destroy",
     "pfac_tables_source_hash", "pfac_pattern_file_hash",
     "pfac_tables_n_parts", "pfac_tables_n_patterns", "pfac_tables_max_pat_len", "pfac_tables_width",
     "pfac_tables_flags", "pfac_tables_part_info", "pfac_tables_s0", "pfac_tables_r", "pfac_tables_HT", "pfac_tables_val",
@@ -59,6 +61,10 @@ def _load():
     lib.pfac_tables_build_mem.argtypes = [_vp, C.c_size_t, C.c_int, C.c_int, C.POINTER(_vp)]
     lib.pfac_tables_build_file_ext.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_uint, C.POINTER(_vp)]
     lib.pfac_tables_build_mem_ext.argtypes = [_vp, C.c_size_t, C.c_int, C.c_int, C.c_uint, C.POINTER(_vp)]
+    lib.pfac_tables_build_file_rules.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_uint, _vp, C.c_uint32, C.POINTER(_vp)]
+    lib.pfac_tables_build_mem_rules.argtypes = [_vp, C.c_size_t, C.c_int, C.c_int, C.c_uint, _vp, C.c_uint32, C.POINTER(_vp)]
+    lib.pfac_tables_case_rules.argtypes = [_vp, _vp, C.c_uint32]
+    lib.pfac_pattern_file_hash_rules.argtypes = [C.c_char_p, C.c_uint, _vp, C.c_uint32, C.POINTER(C.c_uint64)]
     lib.pfac_tables_save.argtypes = [_vp, C.c_char_p]
     lib.pfac_tables_source_hash.argtypes = [_vp]
     lib.pfac_tables_source_hash.restype = C.c_uint64

@@ -51,6 +51,72 @@ static int write_results(const pfac_job *job, const char *out_name)
     return 0;
 }
 
+static bool read_all(const char *path, std::vector<unsigned char> &out)
+{
+    FILE *f = fopen(path, "rb");
+    if (!f) return false;
+    unsigned char tmp[1 << 16];
+    size_t got;
+    while ((got = fread(tmp, 1, sizeof tmp, f)) > 0) out.insert(out.end(), tmp, tmp + got);
+    fclose(f);
+    return true;
+}
+
+// The patterns a well-formed pattern file holds: one per raw newline, except, with the escape reader, a newline
+// that "\x" skips as white space before its hex digits (a malformed file is refused by the builder)
+static uint32_t count_patterns(const std::vector<unsigned char> &b, bool escapes)
+{
+    uint32_t n = 0;
+    for (size_t i = 0; i < b.size(); i++) {
+        if (escapes && b[i] == '\\' && i + 1 < b.size()) {
+            const unsigned char c = b[i + 1];
+            if (c == 'x') {
+                size_t j = i + 2;
+                while (j < b.size() && (b[j] == ' ' || (b[j] >= 9 && b[j] <= 13))) j++;
+                i = j - 1;
+            } else if (c && strchr("abtnvfr'\"\\", c)) {
+                i++;   // a two-byte escape
+            }          // else octal digits or no escape: the bytes after the backslash are read on their own
+            continue;
+        }
+        n += b[i] == '\n';
+    }
+    return n;
+}
+
+// GPHF_NOCASE_LINES=<file>: the 1-based numbers of the patterns that match in either case, one decimal per line;
+// every other pattern of the n matches byte for byte.  false (with a message) for an unparsable line or a number
+// out of range.
+static bool read_nocase_lines(const char *path, uint32_t n, std::vector<uint8_t> &rules)
+{
+    std::vector<unsigned char> b;
+    if (!read_all(path, b)) {
+        fprintf(stderr, "GPHF_NOCASE_LINES: cannot read %s\n", path);
+        return false;
+    }
+    rules.assign(n, 0);
+    size_t line = 0;
+    for (size_t i = 0; i < b.size();) {
+        line++;
+        size_t j = i;
+        uint64_t v = 0;
+        for (; j < b.size() && b[j] >= '0' && b[j] <= '9'; j++)
+            if (v <= n) v = v * 10 + (uint64_t)(b[j] - '0');   // (saturates above n: out of range)
+        if (j == i || (j < b.size() && b[j] != '\n')) {
+            fprintf(stderr, "GPHF_NOCASE_LINES: line %zu of %s is not a pattern number\n", line, path);
+            return false;
+        }
+        if (v < 1 || v > n) {
+            fprintf(stderr, "GPHF_NOCASE_LINES: pattern %llu (line %zu of %s) is out of range: the file has %u patterns\n",
+                    (unsigned long long)v, line, path, n);
+            return false;
+        }
+        rules[(size_t)v - 1] = 1;
+        i = j + 1;
+    }
+    return true;
+}
+
 int main(int argc, char **argv)
 {
     if (argc != 5) {   // main.cc:93-96
@@ -71,8 +137,29 @@ int main(int argc, char **argv)
     // GPHF_CASELESS=1: ASCII letters match in either case (PFAC_PATTERNS_CASELESS)
     const unsigned pflags = (getenv("GPHF_ESCAPES") && atoi(getenv("GPHF_ESCAPES")) ? PFAC_PATTERNS_ESCAPES : 0u) |
                             (getenv("GPHF_CASELESS") && atoi(getenv("GPHF_CASELESS")) ? PFAC_PATTERNS_CASELESS : 0u);
+    // GPHF_NOCASE_LINES=<file>: per-pattern case rules (pfac_tables_build_file_rules): the patterns it numbers
+    // match in either case, every other one byte for byte
+    const char *nocase = getenv("GPHF_NOCASE_LINES");
+    std::vector<uint8_t> rules;
+    unsigned want_flags = pflags & PFAC_PATTERNS_CASELESS;
+    if (nocase && *nocase) {
+        if (pflags & PFAC_PATTERNS_CASELESS) {
+            fprintf(stderr, "GPHF_NOCASE_LINES and GPHF_CASELESS=1 exclude each other\n");
+            return 1;
+        }
+        std::vector<unsigned char> image;
+        if (!read_all(argv[1], image)) {
+            fprintf(stderr, "Open input file failed: %s\n", argv[1]);
+            return 1;
+        }
+        if (!read_nocase_lines(nocase, count_patterns(image, (pflags & PFAC_PATTERNS_ESCAPES) != 0), rules)) return 1;
+        const size_t ones = (size_t)std::count(rules.begin(), rules.end(), (uint8_t)1);
+        want_flags = ones == rules.size() ? PFAC_PATTERNS_CASELESS : ones == 0 ? 0u : PFAC_PATTERNS_CASE_RULES;
+    }
+    const bool with_rules = !rules.empty();
     // GPHF_TABLE_CACHE=<file>: load the tables from it if it exists and was built from this pattern file
-    // (hash of the file image + front-end flags in the cache header) at this width, else build them and write it
+    // (hash of the file image + front-end flags [+ case rules] in the cache header) at this width, else build them
+    // and write it
     const char *cache = getenv("GPHF_TABLE_CACHE");
     bool from_cache = false;
     if (cache && *cache) {
@@ -81,9 +168,11 @@ int main(int argc, char **argv)
             fclose(probe);
             if (pfac_tables_load(cache, &tables)) return fail("load the table cache");
             uint64_t want = 0;
-            if (pfac_pattern_file_hash(argv[1], pflags, &want)) return fail("read the pattern file");
+            if (with_rules ? pfac_pattern_file_hash_rules(argv[1], pflags, rules.data(), (uint32_t)rules.size(), &want)
+                           : pfac_pattern_file_hash(argv[1], pflags, &want))
+                return fail("read the pattern file");
             if (pfac_tables_width(tables) != width || pfac_tables_n_parts(tables) != 1 ||
-                pfac_tables_source_hash(tables) != want || pfac_tables_flags(tables) != (pflags & PFAC_PATTERNS_CASELESS)) {
+                pfac_tables_source_hash(tables) != want || pfac_tables_flags(tables) != want_flags) {
                 // built from another pattern file, width or front-end flags: rebuild (and rewrite the cache)
                 fprintf(stderr, "%s does not belong to this pattern file / width: rebuilding the tables\n", cache);
                 pfac_tables_destroy(tables);
@@ -94,7 +183,9 @@ int main(int argc, char **argv)
         }
     }
     if (!from_cache) {
-        if (pfac_tables_build_file_ext(argv[1], 1, width, pflags, &tables)) return fail("create PFAC/PHF tables");
+        if (with_rules ? pfac_tables_build_file_rules(argv[1], 1, width, pflags, rules.data(), (uint32_t)rules.size(), &tables)
+                       : pfac_tables_build_file_ext(argv[1], 1, width, pflags, &tables))
+            return fail("create PFAC/PHF tables");
         if (cache && *cache && pfac_tables_save(tables, cache)) return fail("write the table cache");
     }
     double t1 = now();

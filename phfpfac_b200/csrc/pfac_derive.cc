@@ -653,6 +653,11 @@ int pattern_lengths(const Partition &P, std::vector<int32_t> &len)
         }
         for (uint32_t e = g.begin(it.state); e < g.end(it.state); e++) stack.push_back({g.edges[e].next, it.depth + 1});
     }
+    // per-pattern case rules: every member of a group reports its owner's length (members never exceed their
+    // owner's id, the last line of the group)
+    const Partition::CaseGroups &cg = P.groups;
+    for (size_t m = 0; m < cg.id.size(); m++)
+        if (cg.id[m] >= 0 && (size_t)cg.id[m] < len.size()) len[(size_t)cg.id[m]] = cg.len[m];
     return PFAC_OK;
 }
 

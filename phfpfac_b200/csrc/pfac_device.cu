@@ -14,6 +14,7 @@
 #include "pfac_fold.cuh"
 #include "pfac_internal.h"
 #include "pfac_kernel.cuh"
+#include "pfac_rules.cuh"
 
 using namespace pfac;
 
@@ -140,8 +141,13 @@ struct Slot {
     Staging doc;
     Buf<unsigned long long> d_blk;
     // caseless sets: the folded copy of caller-owned input (pfac_scan_device, pfac_scan_batch_device) at the
-    // input's 16-byte phase; grows to the largest input scanned and is held until pfac_ctx_destroy
+    // input's 16-byte phase; grows to the largest input scanned and is held until pfac_ctx_destroy.  Mixed sets
+    // fold every input here, the library's own buffers included
     Buf<uint8_t> d_fold;
+    // mixed sets (pfac_rules.cuh): the detector's records (owner ids), max(cap, 4096) of them, and the verify
+    // pass's per-CTA counts
+    Buf<uint2> d_pre;
+    Buf<unsigned long long> d_vblk;
 };
 
 struct Stage {   // one pipeline stage of pfac_scan_host
@@ -181,6 +187,14 @@ struct pfac_ctx {
     size_t dense_smem = 0;
     bool dense_first = false;      // no detector: the dense-match kernel walks every tile (sets with patterns <= 3 bytes)
     bool caseless = false;         // PFAC_PATTERNS_CASELESS: every scan folds its input first (pfac_fold.cuh)
+    // PFAC_PATTERNS_CASE_RULES: the verify tables (pfac_rules.cuh); mixed: every scan folds out of place and ends
+    // with the verify pass
+    bool mixed = false;
+    Buf<int2> d_vgrp;
+    Buf<int4> d_vmem;
+    Buf<uint8_t> d_vpool;
+    uint32_t v_ids = 0;
+    uint32_t max_group = 0;
     // batch scans: pattern length of every id; batch_rc != PFAC_OK: the set does not support them (batch_why)
     Buf<int32_t> d_patlen;
     uint32_t n_ids = 0;
@@ -215,7 +229,8 @@ struct pfac_ctx {
     size_t table_bytes() const
     {
         return d_r.bytes() + d_idmap.bytes() + d_s0.bytes() + d_htval.bytes() + d_step.bytes() + d_s0r.bytes() +
-               d_patdir.bytes() + d_image.bytes() + d_gimage.bytes() + d_wcache.bytes() + d_patlen.bytes();
+               d_patdir.bytes() + d_image.bytes() + d_gimage.bytes() + d_wcache.bytes() + d_patlen.bytes() +
+               d_vgrp.bytes() + d_vmem.bytes() + d_vpool.bytes();
     }
 };
 
@@ -325,7 +340,9 @@ int slot_init(Slot &s)
 // Enqueue one scan (scan kernel + ordering pass) on `stream`.  On completion slot.d_result holds
 // {count, error}; d_count (optional, device) receives the count as well.  n: launches, tiles and CTAs.
 // own_input: d_in is the library's own buffer (a host scan's stage, a flow call's packed buffer), which a caseless
-// set folds in place; the caller's input is folded into slot.d_fold instead and never written.
+// set folds in place; the caller's input is folded into slot.d_fold instead and never written.  A mixed set folds
+// every input into slot.d_fold (the verify pass reads the original bytes) and scans into slot.d_pre; the verify
+// pass then writes d_out, d_count and slot.d_result.
 int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, uint64_t n_valid, uint64_t base_pos,
                 uint32_t pos_bias, void *d_out, uint64_t cap, void *d_count, cudaStream_t stream, Counters &n,
                 bool own_input)
@@ -356,9 +373,11 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
     if (ctx->n_stages < (uint32_t)min_stages((int)ctx->dv.mode))
         return set_error(PFAC_ERR_INTERNAL, "input ring of %u stages is too shallow for the slot scheme", ctx->n_stages);
     uint64_t folds = 0;
-    if (ctx->caseless) {   // the fold of the bytes the scan reads, at the input's phase: mis and every bound stay
+    const bool mixed = ctx->mixed;
+    const uint8_t *orig_al = (const uint8_t *)d_in - mis;
+    if (ctx->caseless || mixed) {   // the fold of the bytes the scan reads, at the input's phase: mis and every bound stay
         uint8_t *out_al = const_cast<uint8_t *>((const uint8_t *)d_in - mis);
-        if (!own_input) {
+        if (!own_input || mixed) {
             if ((e = slot.d_fold.reserve((size_t)(mis + n_valid), 0, stream))) return e;
             out_al = slot.d_fold.get();
         }
@@ -390,6 +409,18 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
     p.partial = partial_now;
     p.partial_next = slot.d_partial.get() + ((slot.flip + 1u) & 1u) * kMaxParts;
     p.ctrl = slot.d_ctrl.get();
+    // a mixed set's scan writes the owners' records to slot.d_pre; the verify pass writes the caller's
+    void *scan_out = d_out, *scan_count = d_count;
+    uint64_t scan_cap = cap;
+    if (mixed) {
+        const size_t want = (size_t)std::max<uint64_t>(cap, 4096);
+        if ((e = slot.d_pre.reserve(want, want, stream)) ||
+            (!slot.d_vblk.get() && (e = slot.d_vblk.alloc(2u * (uint32_t)ctx->sm_count + 1))))
+            return e;
+        scan_out = slot.d_pre.get();
+        scan_cap = slot.d_pre.cap();
+        scan_count = nullptr;
+    }
     const uint32_t grid = (uint32_t)std::min<uint64_t>(p.n_tiles, (uint64_t)ctx->sm_count);
     // tile ranges of the ordering pass: many small ones, so that dense outputs (every tile a long run
     // of records) are moved by the whole GPU
@@ -437,12 +468,12 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
     dp.n_dense = &slot.d_ctrl.get()->n_dense;
     const cudaLaunchConfig_t dl = launch_config(ctx, stream, grid, kDenseThreads, ctx->dense_smem);
     if (dense_first) {   // the dense-match kernel is the whole scan: records go straight to the caller's buffer
-        dp.out = (uint2 *)d_out;
-        dp.cap = cap;
+        dp.out = (uint2 *)scan_out;
+        dp.cap = scan_cap;
         dp.prefix = slot.d_tile_src.get();
         dp.epoch = slot.flip % 0xFFFFFEu + 1u;
         dp.result = slot.d_result.get();
-        dp.count_out = (unsigned long long *)d_count;
+        dp.count_out = (unsigned long long *)scan_count;
         CU_TRY(cudaLaunchKernelEx(&dl, pfac_dense_kernel<true>, dp));
         if (ev_after) CU_TRY(cudaEventRecord(ev_after, stream));
     } else {   // dense-match pass and ordering pass
@@ -452,20 +483,43 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
         f.tile_src = slot.d_tile_src.get();
         f.scratch = slot.d_scratch.get();
         f.scratch_cap = slot.d_scratch.cap();
-        f.out = (uint2 *)d_out;
-        f.cap = cap;
+        f.out = (uint2 *)scan_out;
+        f.cap = scan_cap;
         f.n_tiles = p.n_tiles;
         f.tiles_per_part = tiles_per_part;
         f.partial = partial_now;
         f.ctrl = slot.d_ctrl.get();
         f.result = slot.d_result.get();
-        f.count_out = (unsigned long long *)d_count;
+        f.count_out = (unsigned long long *)scan_count;
         f.debug = ctx->debug;
         f.trace_ctas = grid;
         const cudaLaunchConfig_t fl = launch_config(ctx, stream, fgrid, kFinThreads, 0);
         CU_TRY(cudaLaunchKernelEx(&fl, pfac_finalize_kernel, f));
     }
-    n.launches = (dense_first ? 1 : 3) + folds;
+    uint64_t verify = 0;
+    if (mixed) {   // the verify pass: owners' records -> the members' records that match the original bytes
+        RulesParams rp;
+        rp.pre = slot.d_pre.get();
+        rp.pre_cap = slot.d_pre.cap();
+        rp.in_al = orig_al;
+        rp.mis = mis;
+        rp.pos_bias = pos_bias;
+        rp.grp = ctx->d_vgrp.get();
+        rp.n_ids = ctx->v_ids;
+        rp.mem = ctx->d_vmem.get();
+        rp.pool = ctx->d_vpool.get();
+        rp.max_group = ctx->max_group;
+        rp.blk = slot.d_vblk.get();
+        rp.out = (uint2 *)d_out;
+        rp.cap = cap;
+        rp.result = slot.d_result.get();
+        rp.count_out = (unsigned long long *)d_count;
+        const cudaLaunchConfig_t vl = launch_config(ctx, stream, 2u * (uint32_t)ctx->sm_count, kRulesThreads, 0);
+        CU_TRY(cudaLaunchKernelEx(&vl, pfac_rules_count_kernel, rp));
+        CU_TRY(cudaLaunchKernelEx(&vl, pfac_rules_write_kernel, rp));
+        verify = 2;
+    }
+    n.launches = (dense_first ? 1 : 3) + folds + verify;
     n.tiles = p.n_tiles;
     n.ctas = grid;
     slot.flip++;
@@ -828,6 +882,29 @@ int upload_walk_cache(pfac_ctx &ctx, const Partition &P, size_t smem_max)
     return PFAC_OK;
 }
 
+// per-pattern case rules: the verify tables of pfac_rules.cuh, indexed by owner id
+int upload_case_groups(pfac_ctx &ctx, const Partition &P)
+{
+    const Partition::CaseGroups &G = P.groups;
+    int32_t max_owner = 0;
+    for (int32_t o : G.owner) max_owner = std::max(max_owner, o);
+    std::vector<int2> grp((size_t)max_owner + 1, make_int2(0, 0));
+    for (size_t g = 0; g < G.owner.size(); g++) {
+        grp[(size_t)G.owner[g]] = make_int2(G.first[g], G.first[g + 1] - G.first[g]);
+        ctx.max_group = std::max<uint32_t>(ctx.max_group, (uint32_t)(G.first[g + 1] - G.first[g]));
+    }
+    std::vector<int4> mem(std::max<size_t>(G.id.size(), 1), make_int4(0, 0, -1, 0));
+    for (size_t m = 0; m < G.id.size(); m++) mem[m] = make_int4(G.id[m], G.len[m], G.off[m], 0);
+    std::vector<uint8_t> pool(G.pool);
+    pool.resize(std::max<size_t>(pool.size(), 16), 0);
+    ctx.v_ids = (uint32_t)grp.size();
+    ctx.max_group = std::max<uint32_t>(ctx.max_group, 1u);
+    int e;
+    if ((e = ctx.d_vgrp.upload(grp)) || (e = ctx.d_vmem.upload(mem)) || (e = ctx.d_vpool.upload(pool))) return e;
+    ctx.mixed = true;
+    return PFAC_OK;
+}
+
 // batch scans need each id's pattern length (a tree-shaped automaton) and results that do not depend on
 // where a document lies in the packed buffer (no reference tile bound: patterns of <= 513 bytes)
 int upload_pattern_lengths(pfac_ctx &ctx, const Partition &P)
@@ -901,6 +978,7 @@ int pfac_ctx_create(int device, const pfac_tables *t, int part, int n_streams, s
         return e;
     ctx->dense_first = ctx->dv.has_short != 0;
     ctx->caseless = (t->flags & PFAC_PATTERNS_CASELESS) != 0;
+    if ((t->flags & PFAC_PATTERNS_CASE_RULES) && (e = upload_case_groups(*ctx, P))) return e;
     if (const char *v = getenv("PFAC_DENSE_FIRST")) ctx->dense_first = atoi(v) != 0;   // experiments: force either path
     ctx->dv.image.clear();
     ctx->dv.image.shrink_to_fit();

@@ -30,6 +30,17 @@ struct Partition {
     // transitions sorted by key = state*256 + byte (the non-negative cells of PFAC[][])
     std::vector<int32_t> keys;
     std::vector<int32_t> next;
+    // Sets with per-pattern case rules (PFAC_PATTERNS_CASE_RULES) only: the verify tables.  The automaton is that
+    // of the folded patterns, so its final state of a folded string reports one owner id (the last fold-equal line
+    // of the partition); group g lists the live lines that fold to that string, ascending by id.  A member with
+    // off >= 0 is an exact line with at least one letter: it matches only where the original text equals
+    // pool[off, off + len).  Every other member matches wherever its owner does.
+    struct CaseGroups {
+        std::vector<int32_t> owner;    // [n_groups]
+        std::vector<int32_t> first;    // [n_groups + 1]: members first[g] .. first[g + 1] - 1
+        std::vector<int32_t> id, len, off;   // [n_members]
+        std::vector<uint8_t> pool;
+    } groups;
 
     // master_kernel.cu:52-64
     int32_t lookup(int32_t state, int32_t byte) const;
@@ -46,5 +57,6 @@ struct pfac_tables {
     int width = 256;
     std::vector<pfac::Partition> parts;
     uint64_t source_hash = 0;   // FNV-1a of the pattern file image + flags the set was built from (0: unknown)
-    unsigned flags = 0;         // PFAC_PATTERNS_CASELESS when the set matches ASCII letters in either case
+    unsigned flags = 0;         // PFAC_PATTERNS_CASELESS or PFAC_PATTERNS_CASE_RULES (include/pfac_b200.h)
+    std::vector<uint8_t> rules; // PFAC_PATTERNS_CASE_RULES: caseless[i] of pattern id i + 1 (n_patterns entries)
 };

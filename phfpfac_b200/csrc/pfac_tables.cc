@@ -473,14 +473,57 @@ int ffdm(Partition &P, int width)
     return PFAC_OK;
 }
 
-int build(const unsigned char *buf, size_t len, int n_parts, int width, unsigned flags, pfac_tables **out)
+// Per-pattern case rules: the groups of one partition's sorted slice.  Lines equal after folding are adjacent (the
+// sort is stable, so in file order); the automaton reports the last of each run.  A caseless line is live if no
+// later caseless line of the run exists (they are all fold-equal), an exact line if no later exact line of the run
+// is byte-equal to it.  orig[id - 1]: the line's bytes before the fold.
+void case_groups(const Pattern *pats, int n, const std::vector<const unsigned char *> &orig, const uint8_t *rules,
+                 Partition::CaseGroups &G)
+{
+    G = Partition::CaseGroups();
+    G.first.push_back(0);
+    for (int a = 0; a < n;) {
+        int b = a + 1;
+        while (b < n && comp_pat(pats[a], pats[b]) == 0) b++;
+        G.owner.push_back(pats[b - 1].id);
+        const int L = pats[a].len;
+        for (int i = a; i < b; i++) {
+            const int id = pats[i].id;
+            const bool caseless = rules[id - 1] != 0;
+            bool live = true;
+            for (int j = i + 1; j < b && live; j++) {
+                const int jd = pats[j].id;
+                if (caseless) live = rules[jd - 1] == 0;
+                else live = rules[jd - 1] != 0 || memcmp(orig[(size_t)id - 1], orig[(size_t)jd - 1], (size_t)L) != 0;
+            }
+            if (!live) continue;
+            int32_t off = -1;
+            if (!caseless) {
+                const unsigned char *o = orig[(size_t)id - 1];
+                if (std::any_of(o, o + L, [](unsigned char c) { return (c | 0x20) >= 'a' && (c | 0x20) <= 'z'; })) {
+                    off = (int32_t)G.pool.size();
+                    G.pool.insert(G.pool.end(), o, o + L);
+                }
+            }
+            G.id.push_back(id);
+            G.len.push_back(L);
+            G.off.push_back(off);
+        }
+        G.first.push_back((int32_t)G.id.size());
+        a = b;
+    }
+}
+
+// rules: null, or (PFAC_PATTERNS_CASE_RULES) caseless[i] of every pattern the reader returns, not all equal
+int build(const unsigned char *buf, size_t len, int n_parts, int width, unsigned flags, const uint8_t *rules,
+          pfac_tables **out)
 {
     if (!out || n_parts < 1) return set_error(PFAC_ERR_ARG, "bad arguments");
     if (width_bits(width) < 0)
         return set_error(PFAC_ERR_WIDTH, "width must be a power of two in [1,4096], got %d", width);
     std::vector<Pattern> pats;
     std::vector<unsigned char> arena;
-    const bool caseless = (flags & PFAC_PATTERNS_CASELESS) != 0;
+    const bool caseless = (flags & PFAC_PATTERNS_CASELESS) != 0 || rules;
     int e;
     if (flags & PFAC_PATTERNS_ESCAPES) {
         e = read_patterns_ext(buf, len, arena, pats);
@@ -491,6 +534,14 @@ int build(const unsigned char *buf, size_t len, int n_parts, int width, unsigned
         e = read_patterns(buf, len, pats);
     }
     if (e) return e;
+    // mixed rules: the exact lines are checked against their bytes before the fold
+    std::vector<unsigned char> orig_arena;
+    std::vector<const unsigned char *> orig;
+    if (rules) {
+        orig_arena = arena;
+        orig.resize(pats.size());
+        for (const Pattern &p : pats) orig[(size_t)p.id - 1] = orig_arena.data() + (p.p - arena.data());
+    }
     // the fold comes after the reader (an escaped \x41 is 'A', then 'a') and before the sort, so that lines equal
     // after folding are duplicates like any other
     if (caseless)
@@ -501,7 +552,8 @@ int build(const unsigned char *buf, size_t len, int n_parts, int width, unsigned
     std::unique_ptr<pfac_tables> t(new pfac_tables);
     t->n_patterns = (int)pats.size();
     t->width = width;
-    t->flags = flags & PFAC_PATTERNS_CASELESS;
+    t->flags = rules ? PFAC_PATTERNS_CASE_RULES : (flags & PFAC_PATTERNS_CASELESS);
+    if (rules) t->rules.assign(rules, rules + pats.size());
     t->parts.resize((size_t)n_parts);
     const int n = (int)pats.size();
     const int k = n / n_parts;            // create_table_reorder.c:220
@@ -520,6 +572,7 @@ int build(const unsigned char *buf, size_t len, int n_parts, int width, unsigned
             return;
         }
         build_trie(pats.data() + (size_t)g * (size_t)k, cnt, P);
+        if (rules) case_groups(pats.data() + (size_t)g * (size_t)k, cnt, orig, rules, P.groups);
         const int rc = ffdm(P, width);
         if (rc) {
             rcs[(size_t)g] = rc;
@@ -561,13 +614,78 @@ int pfac_abi_version(void) { return PFAC_B200_ABI_VERSION; }
 
 namespace {
 // FNV-1a 64 of the pattern file image and the front-end flags: identifies what a table set was built from
-uint64_t source_hash_of(const void *bytes, size_t len, unsigned flags)
+// (mixed case rules: and the rule bytes after the flags)
+uint64_t source_hash_of(const void *bytes, size_t len, unsigned flags, const uint8_t *rules = nullptr, size_t n_rules = 0)
 {
     uint64_t h = 1469598103934665603ull;
     const unsigned char *b = (const unsigned char *)bytes;
     for (size_t i = 0; i < len; i++) h = (h ^ b[i]) * 1099511628211ull;
     for (int i = 0; i < 4; i++) h = (h ^ ((flags >> (8 * i)) & 255u)) * 1099511628211ull;
+    for (size_t i = 0; i < n_rules; i++) h = (h ^ rules[i]) * 1099511628211ull;
     return h ? h : 1;   // 0 = unknown (tables wrapped from arrays)
+}
+
+// Per-pattern case rules: the refusals of the _rules calls, then the rule class.  Returns 1 (all caseless: the
+// PFAC_PATTERNS_CASELESS set), 0 (all exact: the plain set) or 2 (mixed) in *kind.
+int check_rules(const unsigned char *buf, size_t len, unsigned flags, const uint8_t *rules, uint32_t n, int *kind)
+{
+    if (flags & PFAC_PATTERNS_CASELESS)
+        return set_error(PFAC_ERR_ARG, "flags %#x: PFAC_PATTERNS_CASELESS (%#x) is not taken with per-pattern rules "
+                         "(caseless[i] = 1 for all %u patterns gives that set)", flags, PFAC_PATTERNS_CASELESS, n);
+    if (flags & ~PFAC_PATTERNS_ESCAPES)
+        return set_error(PFAC_ERR_ARG, "flags %#x: per-pattern rules take PFAC_PATTERNS_ESCAPES (%#x) only", flags,
+                         PFAC_PATTERNS_ESCAPES);
+    if (!rules) return set_error(PFAC_ERR_ARG, "the rules of %u patterns are NULL", n);
+    uint32_t ones = 0;
+    for (uint32_t i = 0; i < n; i++) {
+        if (rules[i] > 1) return set_error(PFAC_ERR_ARG, "caseless[%u] = %u: a rule is 0 (exact) or 1 (caseless)", i, rules[i]);
+        ones += rules[i];
+    }
+    std::vector<pfac::Pattern> pats;
+    std::vector<unsigned char> arena;
+    const int e = (flags & PFAC_PATTERNS_ESCAPES) ? pfac::read_patterns_ext(buf, len, arena, pats) : pfac::read_patterns(buf, len, pats);
+    if (e) return e;
+    if (pats.size() != n)
+        return set_error(PFAC_ERR_ARG, "%u rules for %zu patterns: one rule per pattern the reader returns", n, pats.size());
+    *kind = ones == n ? 1 : ones == 0 ? 0 : 2;
+    return PFAC_OK;
+}
+
+// The source hash of a set built with these rules: that of the uniform set for uniform rules
+uint64_t rules_hash(const unsigned char *buf, size_t len, unsigned flags, const uint8_t *rules, uint32_t n, int kind)
+{
+    if (kind != 2) return source_hash_of(buf, len, flags | (kind ? PFAC_PATTERNS_CASELESS : 0u));
+    return source_hash_of(buf, len, flags | PFAC_PATTERNS_CASE_RULES, rules, n);
+}
+
+// the image of a pattern file; *e = PFAC_ERR_IO if it cannot be opened
+std::vector<unsigned char> read_file(const char *path, int *e)
+{
+    std::vector<unsigned char> buf;
+    FILE *f = path ? fopen(path, "rb") : nullptr;
+    if (!f) {
+        *e = set_error(PFAC_ERR_IO, "Open input file failed: %s", path ? path : "(null)");
+        return buf;
+    }
+    unsigned char tmp[1 << 16];
+    size_t got;
+    while ((got = fread(tmp, 1, sizeof tmp, f)) > 0) buf.insert(buf.end(), tmp, tmp + got);
+    fclose(f);
+    *e = PFAC_OK;
+    return buf;
+}
+// The verify pass indexes its tables with the owner ids and offsets these arrays hold
+const char *validate_groups(const pfac::Partition::CaseGroups &G, int32_t n_patterns)
+{
+    if (G.first.size() != G.owner.size() + 1 || G.first[0] != 0 || G.first.back() != (int32_t)G.id.size())
+        return "case group ranges";
+    for (size_t g = 0; g < G.owner.size(); g++)
+        if (G.first[g + 1] < G.first[g] || G.owner[g] < 1 || G.owner[g] > n_patterns) return "case group";
+    for (size_t m = 0; m < G.id.size(); m++)
+        if (G.id[m] < 1 || G.id[m] > n_patterns || G.len[m] < 1 || G.len[m] > pfac::kMaxPatternBytes || G.off[m] < -1 ||
+            (G.off[m] >= 0 && (size_t)G.off[m] + (size_t)G.len[m] > G.pool.size()))
+            return "case group member";
+    return nullptr;
 }
 // The kernels index r[] / {HT,val} / s0 / idmap with what these arrays hold, unchecked (as the
 // reference does): a table set that did not come out of the builder is checked once, here.
@@ -602,7 +720,7 @@ int pfac_tables_build_mem_ext(const void *pattern_bytes, size_t len, int n_parts
 {
     if (!pattern_bytes && len) return set_error(PFAC_ERR_ARG, "null pattern buffer");
     try {
-        const int rc = build((const unsigned char *)pattern_bytes, len, n_parts, width, flags, out);
+        const int rc = build((const unsigned char *)pattern_bytes, len, n_parts, width, flags, nullptr, out);
         if (rc == PFAC_OK && out && *out) (*out)->source_hash = source_hash_of(pattern_bytes, len, flags);
         return rc;
     } catch (const std::bad_alloc &) {
@@ -615,13 +733,9 @@ uint64_t pfac_tables_source_hash(const pfac_tables *t) { return t ? t->source_ha
 int pfac_pattern_file_hash(const char *pattern_file, unsigned flags, uint64_t *hash)
 {
     if (!hash) return set_error(PFAC_ERR_ARG, "null hash");
-    FILE *f = pattern_file ? fopen(pattern_file, "rb") : nullptr;
-    if (!f) return set_error(PFAC_ERR_IO, "Open input file failed: %s", pattern_file ? pattern_file : "(null)");
-    std::vector<unsigned char> buf;
-    unsigned char tmp[1 << 16];
-    size_t got;
-    while ((got = fread(tmp, 1, sizeof tmp, f)) > 0) buf.insert(buf.end(), tmp, tmp + got);
-    fclose(f);
+    int e;
+    std::vector<unsigned char> buf = read_file(pattern_file, &e);
+    if (e) return e;
     *hash = source_hash_of(buf.data(), buf.size(), flags);
     return PFAC_OK;
 }
@@ -633,14 +747,61 @@ int pfac_tables_build_file(const char *pattern_file, int n_parts, int width, pfa
 
 int pfac_tables_build_file_ext(const char *pattern_file, int n_parts, int width, unsigned flags, pfac_tables **out)
 {
-    FILE *f = pattern_file ? fopen(pattern_file, "rb") : nullptr;
-    if (!f) return set_error(PFAC_ERR_IO, "Open input file failed: %s", pattern_file ? pattern_file : "(null)");
-    std::vector<unsigned char> buf;
-    unsigned char tmp[1 << 16];
-    size_t got;
-    while ((got = fread(tmp, 1, sizeof tmp, f)) > 0) buf.insert(buf.end(), tmp, tmp + got);
-    fclose(f);
+    int e;
+    std::vector<unsigned char> buf = read_file(pattern_file, &e);
+    if (e) return e;
     return pfac_tables_build_mem_ext(buf.data(), buf.size(), n_parts, width, flags, out);
+}
+
+int pfac_tables_build_mem_rules(const void *pattern_bytes, size_t len, int n_parts, int width, unsigned flags,
+                                const uint8_t *caseless, uint32_t n_patterns, pfac_tables **out)
+{
+    if (!pattern_bytes && len) return set_error(PFAC_ERR_ARG, "null pattern buffer");
+    const unsigned char *buf = (const unsigned char *)pattern_bytes;
+    try {
+        int kind = 0;
+        int rc = check_rules(buf, len, flags, caseless, n_patterns, &kind);
+        if (rc) return rc;
+        rc = build(buf, len, n_parts, width, flags | (kind == 1 ? PFAC_PATTERNS_CASELESS : 0u), kind == 2 ? caseless : nullptr, out);
+        if (rc == PFAC_OK && out && *out) (*out)->source_hash = rules_hash(buf, len, flags, caseless, n_patterns, kind);
+        return rc;
+    } catch (const std::bad_alloc &) {
+        return set_error(PFAC_ERR_NOMEM, "out of memory building tables");
+    }
+}
+
+int pfac_tables_build_file_rules(const char *pattern_file, int n_parts, int width, unsigned flags, const uint8_t *caseless,
+                                 uint32_t n_patterns, pfac_tables **out)
+{
+    int e;
+    std::vector<unsigned char> buf = read_file(pattern_file, &e);
+    if (e) return e;
+    return pfac_tables_build_mem_rules(buf.data(), buf.size(), n_parts, width, flags, caseless, n_patterns, out);
+}
+
+int pfac_pattern_file_hash_rules(const char *pattern_file, unsigned flags, const uint8_t *caseless, uint32_t n_patterns,
+                                 uint64_t *hash)
+{
+    if (!hash) return set_error(PFAC_ERR_ARG, "null hash");
+    try {
+        int e, kind = 0;
+        std::vector<unsigned char> buf = read_file(pattern_file, &e);
+        if (e || (e = check_rules(buf.data(), buf.size(), flags, caseless, n_patterns, &kind))) return e;
+        *hash = rules_hash(buf.data(), buf.size(), flags, caseless, n_patterns, kind);
+        return PFAC_OK;
+    } catch (const std::bad_alloc &) {
+        return set_error(PFAC_ERR_NOMEM, "out of memory");
+    }
+}
+
+int pfac_tables_case_rules(const pfac_tables *t, uint8_t *caseless, uint32_t n)
+{
+    if (!t || !caseless || n != (uint32_t)t->n_patterns)
+        return set_error(PFAC_ERR_ARG, "pfac_tables_case_rules takes one rule per pattern: %u for %d patterns", n,
+                         t ? t->n_patterns : 0);
+    if (t->flags & PFAC_PATTERNS_CASE_RULES) memcpy(caseless, t->rules.data(), n);
+    else memset(caseless, (t->flags & PFAC_PATTERNS_CASELESS) ? 1 : 0, n);
+    return PFAC_OK;
 }
 
 int pfac_tables_from_arrays(const int32_t *s0, const int32_t *r, int32_t n_r, const int32_t *HT,
@@ -682,10 +843,14 @@ int pfac_tables_from_arrays(const int32_t *s0, const int32_t *r, int32_t n_r, co
 // ---- on-disk cache of the canonical arrays (the reference serialises nothing: it rebuilds the trie
 // and the PHF on every run, main.cc:100-126).  Little-endian int32 fields:
 //   "PFACTBL2", n_parts, n_patterns, max_pat_len, width, source hash (u64: pattern file image + flags),
-//   ["PFACTBL3" only: u32 flags (PFAC_PATTERNS_CASELESS): written for caseless sets alone, so that a case-sensitive
-//    set writes the same file as before and a library that does not know the flag refuses the cache by its magic],
+//   ["PFACTBL3" only: u32 flags (PFAC_PATTERNS_CASELESS or PFAC_PATTERNS_CASE_RULES): written for those sets alone,
+//    so that a case-sensitive set writes the same file as before and a library that does not know the flag refuses
+//    the cache by its magic (and a library that knows PFAC_PATTERNS_CASELESS only, by the flags value)],
+//   [PFAC_PATTERNS_CASE_RULES only: u8 rules[n_patterns]],
 //   per partition: state_num, n_final, max_len, min_len, width, n_keys, max_key, max_row, max_offset,
 //                  ht_size, n_r, then s0[256], r[n_r], HT[ht_size], val[ht_size], idmap[n_final],
+//                  [PFAC_PATTERNS_CASE_RULES only: n_groups, n_members, pool bytes, owner[n_groups],
+//                   first[n_groups + 1], id[n_members], len[n_members], off[n_members], u8 pool[]],
 //   FNV-1a 64 of everything before it.
 namespace {
 struct Fnv {
@@ -718,7 +883,9 @@ int pfac_tables_save(const pfac_tables *t, const char *path)
     const uint32_t flags = t->flags;
     bool ok = put(f, h, flags ? "PFACTBL3" : "PFACTBL2", 8);
     const int32_t head[4] = {(int32_t)t->parts.size(), t->n_patterns, t->max_pat_len, t->width};
-    ok = ok && put(f, h, head, sizeof head) && put(f, h, &t->source_hash, 8) && (!flags || put(f, h, &flags, 4));
+    const bool mixed = (flags & PFAC_PATTERNS_CASE_RULES) != 0;
+    ok = ok && put(f, h, head, sizeof head) && put(f, h, &t->source_hash, 8) && (!flags || put(f, h, &flags, 4)) &&
+         (!mixed || put(f, h, t->rules.data(), t->rules.size()));
     for (const Partition &P : t->parts) {
         const int32_t ph[11] = {P.state_num, P.n_final, P.max_len, P.min_len, P.width, P.n_keys, P.max_key, P.max_row,
                                 P.max_offset, P.ht_size, (int32_t)P.r.size()};
@@ -727,6 +894,14 @@ int pfac_tables_save(const pfac_tables *t, const char *path)
         ok = ok && put(f, h, ph, sizeof ph) && put(f, h, s0.data(), kCharSet * 4) && put(f, h, P.r.data(), P.r.size() * 4) &&
              put(f, h, P.HT.data(), (size_t)P.ht_size * 4) && put(f, h, P.val.data(), (size_t)P.ht_size * 4) &&
              put(f, h, P.idmap.data(), (size_t)P.n_final * 4);
+        if (mixed) {
+            const Partition::CaseGroups &G = P.groups;
+            const int32_t gh[3] = {(int32_t)G.owner.size(), (int32_t)G.id.size(), (int32_t)G.pool.size()};
+            ok = ok && put(f, h, gh, sizeof gh) && put(f, h, G.owner.data(), G.owner.size() * 4) &&
+                 put(f, h, G.first.data(), G.first.size() * 4) && put(f, h, G.id.data(), G.id.size() * 4) &&
+                 put(f, h, G.len.data(), G.len.size() * 4) && put(f, h, G.off.data(), G.off.size() * 4) &&
+                 put(f, h, G.pool.data(), G.pool.size());
+        }
     }
     const uint64_t sum = h.h;
     ok = ok && fwrite(&sum, 1, 8, f) == 8;
@@ -754,10 +929,15 @@ int pfac_tables_load(const char *path, pfac_tables **out)
         if (!get(f, h, head, sizeof head) || !get(f, h, &src_hash, 8) || head[0] < 1 || head[0] > (1 << 20) || head[1] < 0 ||
             head[2] < 0 || width_bits(head[3]) < 0)
             return bad("header");
-        if (v3 && (!get(f, h, &flags, 4) || flags != PFAC_PATTERNS_CASELESS)) return bad("flags");
+        if (v3 && (!get(f, h, &flags, 4) || (flags != PFAC_PATTERNS_CASELESS && flags != PFAC_PATTERNS_CASE_RULES)))
+            return bad("flags");
+        const bool mixed = flags == PFAC_PATTERNS_CASE_RULES;
+        std::vector<uint8_t> rules(mixed ? (size_t)head[1] : 0);
+        if (mixed && !get(f, h, rules.data(), rules.size())) return bad("truncated");
         std::unique_ptr<pfac_tables> t(new pfac_tables);
         t->source_hash = src_hash;
         t->flags = flags;
+        t->rules.swap(rules);
         t->n_patterns = head[1];
         t->max_pat_len = head[2];
         t->width = head[3];
@@ -787,11 +967,34 @@ int pfac_tables_load(const char *path, pfac_tables **out)
                 !get(f, h, P.HT.data(), P.HT.size() * 4) || !get(f, h, P.val.data(), P.val.size() * 4) ||
                 !get(f, h, P.idmap.data(), P.idmap.size() * 4))
                 return bad("truncated");
+            if (mixed) {   // (the sizes are bounded before anything is allocated for them)
+                Partition::CaseGroups &G = P.groups;
+                int32_t gh[3];
+                if (!get(f, h, gh, sizeof gh)) return bad("truncated");
+                if (gh[0] < 0 || gh[1] < 0 || gh[2] < 0 || gh[0] > head[1] || gh[1] > head[1] ||
+                    (int64_t)gh[2] > (int64_t)gh[1] * kMaxPatternBytes)
+                    return bad("case groups header");
+                G.owner.resize((size_t)gh[0]);
+                G.first.resize((size_t)gh[0] + 1);
+                G.id.resize((size_t)gh[1]);
+                G.len.resize((size_t)gh[1]);
+                G.off.resize((size_t)gh[1]);
+                G.pool.resize((size_t)gh[2]);
+                if (!get(f, h, G.owner.data(), G.owner.size() * 4) || !get(f, h, G.first.data(), G.first.size() * 4) ||
+                    !get(f, h, G.id.data(), G.id.size() * 4) || !get(f, h, G.len.data(), G.len.size() * 4) ||
+                    !get(f, h, G.off.data(), G.off.size() * 4) || !get(f, h, G.pool.data(), G.pool.size()))
+                    return bad("truncated");
+            }
         }
         uint64_t sum = 0;
         if (fread(&sum, 1, 8, f) != 8 || sum != h.h) return bad("checksum");
         for (const Partition &P : t->parts)
             if (const char *why = validate_partition(P)) return bad(why);
+        for (uint8_t r : t->rules)
+            if (r > 1) return bad("case rule");
+        if (mixed)
+            for (const Partition &P : t->parts)
+                if (const char *why = validate_groups(P.groups, t->n_patterns)) return bad(why);
         fclose(f);
         *out = t.release();
         return PFAC_OK;
@@ -907,8 +1110,8 @@ int pfac_tables_filter_profile(const pfac_tables *t, int part, uint32_t t2_bytes
     try {
         Derived d;
         derive_tables(*P, t2_bytes, t3_bytes, tm2_bytes, d);
-        std::vector<uint8_t> folded;   // a caseless set counts the text its scans see
-        if (t->flags & PFAC_PATTERNS_CASELESS) {
+        std::vector<uint8_t> folded;   // a caseless or mixed set counts the text its detector sees
+        if (t->flags & (PFAC_PATTERNS_CASELESS | PFAC_PATTERNS_CASE_RULES)) {
             folded.assign((const uint8_t *)text, (const uint8_t *)text + n);
             for (uint8_t &c : folded) c = ascii_fold(c);
             text = folded.data();

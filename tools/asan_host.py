@@ -113,3 +113,41 @@ for t in range(200):
         lib.pfac_tables_destroy(h2)   # (a flipped bit in unused padding may load)
 lib.pfac_tables_destroy(h)
 print("asan table cache ok")
+# per-pattern case rules: mixed builds (escapes included), lengths, save / load and damaged files
+lib.pfac_tables_build_mem_rules.argtypes = [C.c_char_p, C.c_size_t, C.c_int, C.c_int, C.c_uint, C.c_void_p, C.c_uint32, C.POINTER(vp)]
+lib.pfac_tables_pattern_lengths.argtypes = [vp, C.c_int, C.c_void_p, C.c_int32, C.POINTER(C.c_int32)]
+lib.pfac_tables_case_rules.argtypes = [vp, C.c_void_p, C.c_uint32]
+lib.pfac_tables_n_patterns.argtypes = [vp]
+mixed = [(b"GET\nget\nGeT\nGET\n123\nget\n", 0), (b"a\\x41\\n\\\nb\\0c\nA\\x61\n", 1), (synth(1, 3000, 3, 4, 64), 0),
+         (b"x" * 1022 + b"\n" + b"X" * 1022 + b"\n", 0), (b"ab\nAB\n", 1), (b"", 0), (b"abc", 0)]
+for blob, flags in mixed:
+    n_pat = blob.count(b"\n") if not flags else 2
+    for parts in (1, 3):
+        rules = (np.arange(max(n_pat, 1)) % 3 == 0).astype(np.uint8)
+        h = vp()
+        rc = lib.pfac_tables_build_mem_rules(blob, len(blob), parts, 256, flags, rules.ctypes.data, n_pat, C.byref(h))
+        if rc != 0:
+            continue
+        got = np.zeros(lib.pfac_tables_n_patterns(h), dtype=np.uint8)
+        assert lib.pfac_tables_case_rules(h, got.ctypes.data, len(got)) == 0
+        for g in range(parts):
+            nid = C.c_int32(0)
+            assert lib.pfac_tables_pattern_lengths(h, g, None, 0, C.byref(nid)) == 0
+            lens = np.zeros(max(nid.value, 1), dtype=np.int32)
+            assert lib.pfac_tables_pattern_lengths(h, g, lens.ctypes.data, len(lens), C.byref(nid)) == 0
+        assert lib.pfac_tables_save(h, b"/tmp/asan_rules.bin") == 0
+        h2 = vp(); assert lib.pfac_tables_load(b"/tmp/asan_rules.bin", C.byref(h2)) == 0
+        lib.pfac_tables_destroy(h2)
+        raw = open("/tmp/asan_rules.bin", "rb").read()
+        for t in range(60):
+            bad = bytearray(raw)
+            if t % 2:
+                bad = bad[:int(rng.integers(0, len(bad)))]
+            else:
+                bad[int(rng.integers(0, len(bad)))] ^= 1 << int(rng.integers(0, 8))
+            open("/tmp/asan_rules_bad.bin", "wb").write(bytes(bad))
+            h2 = vp()
+            if lib.pfac_tables_load(b"/tmp/asan_rules_bad.bin", C.byref(h2)) == 0:
+                lib.pfac_tables_destroy(h2)
+        lib.pfac_tables_destroy(h)
+print("asan case rules ok")
