@@ -10,7 +10,7 @@ NVFLAGS := $(EXTRA) $(ARCH) -lineinfo -O3 -std=c++17 -ccbin $(HOSTCXX) -Iinclude
            -Xcompiler -fPIC,-Wall,-Wextra,-pthread -Xptxas -v
 HOST_SRCS := $(SRC)/pfac_tables.cc $(SRC)/pfac_writer.cc $(SRC)/pfac_job.cc $(SRC)/pfac_derive.cc
 CUDA_SRCS := $(SRC)/pfac_device.cu
-HDRS := include/pfac_b200.h $(SRC)/pfac_internal.h $(SRC)/pfac_kernel.cuh $(SRC)/pfac_batch.cuh $(SRC)/pfac_flows.cuh $(SRC)/pfac_fold.cuh $(SRC)/pfac_rules.cuh $(SRC)/pfac_derive.h
+HDRS := include/pfac_b200.h $(SRC)/pfac_internal.h $(SRC)/pfac_kernel.cuh $(SRC)/pfac_compact.cuh $(SRC)/pfac_batch.cuh $(SRC)/pfac_flows.cuh $(SRC)/pfac_fold.cuh $(SRC)/pfac_rules.cuh $(SRC)/pfac_derive.h
 
 .PHONY: all lib cli oracle synth clean
 all: lib cli oracle synth

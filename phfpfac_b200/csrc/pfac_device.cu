@@ -134,20 +134,19 @@ struct Slot {
     Buf<unsigned long long> d_tile_src;
     Buf<uint2> d_scratch;
     bool dirty = false;       // a launch sequence failed half way: the control block is reset before the next scan
+    // per-CTA counts of the stable expansions (pfac_compact.cuh: the split and verify passes), compact_grid + 1
+    Buf<unsigned long long> d_blk;
     // batch scans (pfac_batch.cuh): raw records of the packed buffer and the global positions of the kept ones,
-    // the document offsets and the split pass's per-CTA counts
+    // the document offsets
     Buf<uint2> d_raw;
     Buf<uint32_t> d_kpos;
     Staging doc;
-    Buf<unsigned long long> d_blk;
     // caseless sets: the folded copy of caller-owned input (pfac_scan_device, pfac_scan_batch_device) at the
     // input's 16-byte phase; grows to the largest input scanned and is held until pfac_ctx_destroy.  Mixed sets
     // fold every input here, the library's own buffers included
     Buf<uint8_t> d_fold;
-    // mixed sets (pfac_rules.cuh): the detector's records (owner ids), max(cap, 4096) of them, and the verify
-    // pass's per-CTA counts
+    // mixed sets (pfac_rules.cuh): the detector's records (owner ids), max(cap, 4096) of them
     Buf<uint2> d_pre;
-    Buf<unsigned long long> d_vblk;
 };
 
 struct Stage {   // one pipeline stage of pfac_scan_host
@@ -327,18 +326,36 @@ void set_info(pfac_ctx *ctx, const Counters &c)
     memcpy(ctx->info, v, sizeof v);
 }
 
-int slot_init(Slot &s)
+// CTAs of the count and write kernels of a stable expansion (pfac_compact.cuh)
+uint32_t compact_grid(const pfac_ctx *ctx) { return 2u * (uint32_t)ctx->sm_count; }
+
+int slot_init(const pfac_ctx *ctx, Slot &s)
 {
     if (s.h_result.get()) return PFAC_OK;
     int e;
     if ((e = s.d_ctrl.alloc(1, true)) || (e = s.d_result.alloc(1)) || (e = s.d_partial.alloc(2 * kMaxParts, true)) ||
-        (e = s.h_result.alloc(1)))
+        (e = s.d_blk.alloc(compact_grid(ctx) + 1)) || (e = s.h_result.alloc(1)))
         return e;
     return PFAC_OK;
 }
 
+// Enqueue a stable expansion (pfac_compact.cuh): its count kernel, then its write kernel, over the slot's per-CTA
+// counts.  The passes of one call (a mixed batch's verify and split passes) share that buffer: a count kernel writes
+// it only after griddepcontrol.wait, when the write kernel before it has finished reading it.
+template <typename P>
+int launch_compact(pfac_ctx *ctx, Slot &slot, void (*count)(P), void (*write)(P), P p, cudaStream_t stream, Counters &n)
+{
+    p.blk = slot.d_blk.get();
+    const cudaLaunchConfig_t lc = launch_config(ctx, stream, compact_grid(ctx), kCompactThreads, 0);
+    CU_TRY(cudaLaunchKernelEx(&lc, count, p));
+    CU_TRY(cudaLaunchKernelEx(&lc, write, p));
+    n.launches += 2;
+    return PFAC_OK;
+}
+
 // Enqueue one scan (scan kernel + ordering pass) on `stream`.  On completion slot.d_result holds
-// {count, error}; d_count (optional, device) receives the count as well.  n: launches, tiles and CTAs.
+// {count, error}; d_count (optional, device) receives the count as well.  n: tiles and CTAs, and the launches,
+// added up as they are enqueued.
 // own_input: d_in is the library's own buffer (a host scan's stage, a flow call's packed buffer), which a caseless
 // set folds in place; the caller's input is folded into slot.d_fold instead and never written.  A mixed set folds
 // every input into slot.d_fold (the verify pass reads the original bytes) and scans into slot.d_pre; the verify
@@ -353,7 +370,7 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
     const uint32_t mis = (uint32_t)((uintptr_t)d_in & 15u);
     if (n_valid + mis + (uint64_t)kTile + 4096 >= (1ull << 32))
         return set_error(PFAC_ERR_LIMIT, "one scan call covers less than 4 GiB; split the input");
-    int e = slot_init(slot);
+    int e = slot_init(ctx, slot);
     if (e) return e;
     if (n_starts == 0 || ctx->max_pat_len == 0) {
         CU_TRY(cudaMemsetAsync(slot.d_result.get(), 0, sizeof(Result), stream));
@@ -372,7 +389,6 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
     } guard{slot};
     if (ctx->n_stages < (uint32_t)min_stages((int)ctx->dv.mode))
         return set_error(PFAC_ERR_INTERNAL, "input ring of %u stages is too shallow for the slot scheme", ctx->n_stages);
-    uint64_t folds = 0;
     const bool mixed = ctx->mixed;
     const uint8_t *orig_al = (const uint8_t *)d_in - mis;
     if (ctx->caseless || mixed) {   // the fold of the bytes the scan reads, at the input's phase: mis and every bound stay
@@ -389,7 +405,7 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
         CU_TRY(cudaLaunchKernelEx(&fl, pfac_fold_kernel, (const uint8_t *)d_in - mis, out_al, (unsigned long long)mis,
                                   (unsigned long long)(mis + n_valid)));
         d_in = out_al + mis;
-        folds = 1;
+        n.launches += 1;
     }
     ScanParams p = ctx->scan;
     p.in_al = (const uint8_t *)d_in - mis;
@@ -414,9 +430,7 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
     uint64_t scan_cap = cap;
     if (mixed) {
         const size_t want = (size_t)std::max<uint64_t>(cap, 4096);
-        if ((e = slot.d_pre.reserve(want, want, stream)) ||
-            (!slot.d_vblk.get() && (e = slot.d_vblk.alloc(2u * (uint32_t)ctx->sm_count + 1))))
-            return e;
+        if ((e = slot.d_pre.reserve(want, want, stream))) return e;
         scan_out = slot.d_pre.get();
         scan_cap = slot.d_pre.cap();
         scan_count = nullptr;
@@ -460,6 +474,7 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
         const cudaLaunchConfig_t lc = launch_config(ctx, stream, grid, kThreads, ctx->smem_bytes);
         CU_TRY(cudaLaunchKernelEx(&lc, detector_kernel(ctx->dv), p));
         if (ev_after) CU_TRY(cudaEventRecord(ev_after, stream));
+        n.launches += 1;
     }
 
     // the tiles the detector handed over whole (dense matches); returns at once when there are none
@@ -476,6 +491,7 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
         dp.count_out = (unsigned long long *)scan_count;
         CU_TRY(cudaLaunchKernelEx(&dl, pfac_dense_kernel<true>, dp));
         if (ev_after) CU_TRY(cudaEventRecord(ev_after, stream));
+        n.launches += 1;
     } else {   // dense-match pass and ordering pass
         CU_TRY(cudaLaunchKernelEx(&dl, pfac_dense_kernel<false>, dp));
         FinalizeParams f;
@@ -495,8 +511,8 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
         f.trace_ctas = grid;
         const cudaLaunchConfig_t fl = launch_config(ctx, stream, fgrid, kFinThreads, 0);
         CU_TRY(cudaLaunchKernelEx(&fl, pfac_finalize_kernel, f));
+        n.launches += 2;
     }
-    uint64_t verify = 0;
     if (mixed) {   // the verify pass: owners' records -> the members' records that match the original bytes
         RulesParams rp;
         rp.pre = slot.d_pre.get();
@@ -509,17 +525,12 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
         rp.mem = ctx->d_vmem.get();
         rp.pool = ctx->d_vpool.get();
         rp.max_group = ctx->max_group;
-        rp.blk = slot.d_vblk.get();
         rp.out = (uint2 *)d_out;
         rp.cap = cap;
         rp.result = slot.d_result.get();
         rp.count_out = (unsigned long long *)d_count;
-        const cudaLaunchConfig_t vl = launch_config(ctx, stream, 2u * (uint32_t)ctx->sm_count, kRulesThreads, 0);
-        CU_TRY(cudaLaunchKernelEx(&vl, pfac_rules_count_kernel, rp));
-        CU_TRY(cudaLaunchKernelEx(&vl, pfac_rules_write_kernel, rp));
-        verify = 2;
+        if ((e = launch_compact(ctx, slot, pfac_rules_count_kernel, pfac_rules_write_kernel, rp, stream, n))) return e;
     }
-    n.launches = (dense_first ? 1 : 3) + folds + verify;
     n.tiles = p.n_tiles;
     n.ctas = grid;
     slot.flip++;
@@ -527,14 +538,11 @@ int launch_scan(pfac_ctx *ctx, Slot &slot, const void *d_in, uint64_t n_starts, 
     return PFAC_OK;
 }
 
-// The slot's buffers of a batch or flow call: raw records and kept positions for max(cap, 4096) records, the split
-// pass's per-CTA counts.  *grid = the CTAs of the count and split kernels.
-int split_prepare(pfac_ctx *ctx, Slot &slot, uint64_t cap, cudaStream_t stream, uint32_t *grid)
+// The slot's buffers of a batch or flow call: raw records and kept positions for max(cap, 4096) records
+int split_prepare(pfac_ctx *ctx, Slot &slot, uint64_t cap, cudaStream_t stream)
 {
-    int e = slot_init(slot);
+    int e = slot_init(ctx, slot);
     if (e) return e;
-    *grid = 2u * (uint32_t)ctx->sm_count;
-    if (!slot.d_blk.get() && (e = slot.d_blk.alloc(*grid + 1))) return e;
     const size_t want = (size_t)std::max<uint64_t>(cap, 4096);
     if ((e = slot.d_raw.reserve(want, want, stream)) || (e = slot.d_kpos.reserve(want, want, stream))) return e;
     return PFAC_OK;
@@ -543,7 +551,7 @@ int split_prepare(pfac_ctx *ctx, Slot &slot, uint64_t cap, cudaStream_t stream, 
 // Enqueue the split pass (pfac_batch.cuh) over the raw records of the packed scan: n_docs documents at the device
 // offsets doc[n_docs + 1]; CARRY: the first tail[d] bytes of document d are carried (device, n_docs).
 template <bool CARRY>
-int launch_split(pfac_ctx *ctx, Slot &slot, uint32_t grid, const uint32_t *doc, const uint32_t *tail, uint32_t n_docs,
+int launch_split(pfac_ctx *ctx, Slot &slot, const uint32_t *doc, const uint32_t *tail, uint32_t n_docs,
                  void *d_out, uint64_t cap, void *d_doc_first, void *d_count, cudaStream_t stream, Counters &n)
 {
     BatchParams bp;
@@ -554,7 +562,6 @@ int launch_split(pfac_ctx *ctx, Slot &slot, uint32_t grid, const uint32_t *doc, 
     bp.n_docs = n_docs;
     bp.len = ctx->d_patlen.get();
     bp.n_ids = ctx->n_ids;
-    bp.blk = slot.d_blk.get();
     bp.out = (uint2 *)d_out;
     bp.cap = cap;
     bp.kpos = slot.d_kpos.get();
@@ -562,14 +569,14 @@ int launch_split(pfac_ctx *ctx, Slot &slot, uint32_t grid, const uint32_t *doc, 
     bp.result = slot.d_result.get();
     bp.count_out = (unsigned long long *)d_count;
     bp.tail = tail;
+    int e = launch_compact(ctx, slot, pfac_batch_count_kernel<CARRY>, pfac_batch_split_kernel<CARRY>, bp, stream, n);
+    if (e) return e;
     const size_t n_off = (size_t)n_docs + 1;
-    const cudaLaunchConfig_t lc = launch_config(ctx, stream, grid, kBatchThreads, 0);
-    CU_TRY(cudaLaunchKernelEx(&lc, pfac_batch_count_kernel<CARRY>, bp));
-    CU_TRY(cudaLaunchKernelEx(&lc, pfac_batch_split_kernel<CARRY>, bp));
-    const cudaLaunchConfig_t dl =
-        launch_config(ctx, stream, (uint32_t)std::min<uint64_t>((n_off + kBatchThreads - 1) / kBatchThreads, grid), kBatchThreads, 0);
+    const cudaLaunchConfig_t dl = launch_config(
+        ctx, stream, (uint32_t)std::min<uint64_t>((n_off + kCompactThreads - 1) / kCompactThreads, compact_grid(ctx)),
+        kCompactThreads, 0);
     CU_TRY(cudaLaunchKernelEx(&dl, pfac_batch_docs_kernel, bp));
-    n.launches += 3;
+    n.launches += 1;
     return PFAC_OK;
 }
 
@@ -586,8 +593,7 @@ int launch_batch(pfac_ctx *ctx, Slot &slot, const void *d_in, const uint64_t *do
     const uint64_t total = doc_offsets[n_docs];
     if (total >= (1ull << 32)) return set_error(PFAC_ERR_LIMIT, "one batch covers less than 4 GiB; split the input");
     if (!d_in && total) return set_error(PFAC_ERR_ARG, "null input of %llu bytes", (unsigned long long)total);
-    uint32_t grid = 0;
-    int e = split_prepare(ctx, slot, cap, stream, &grid);
+    int e = split_prepare(ctx, slot, cap, stream);
     if (e) return e;
     // the offsets, checked on the way (32 bits suffice: total < 4 GiB)
     const size_t n_off = (size_t)n_docs + 1;
@@ -606,7 +612,7 @@ int launch_batch(pfac_ctx *ctx, Slot &slot, const void *d_in, const uint64_t *do
 
     e = launch_scan(ctx, slot, d_in, total, total, 0, 0u, slot.d_raw.get(), slot.d_raw.cap(), nullptr, stream, n, false);
     if (e) return e;
-    e = launch_split<false>(ctx, slot, grid, slot.doc.d.get(), nullptr, n_docs, d_out, cap, d_doc_first, d_count, stream, n);
+    e = launch_split<false>(ctx, slot, slot.doc.d.get(), nullptr, n_docs, d_out, cap, d_doc_first, d_count, stream, n);
     if (e) return e;
     n.h2d = n_off * sizeof(uint32_t);
     return PFAC_OK;
@@ -640,8 +646,7 @@ int launch_flows(pfac_flows *f, Slot &slot, const void *d_in, const uint64_t *ch
     if (total_in >= (1ull << 32) || packed + (uint64_t)kTile + 4096 >= (1ull << 32))
         return set_error(PFAC_ERR_LIMIT, "one call covers less than 4 GiB of chunks and carried tails; split the input");
     if (!d_in && total_in) return set_error(PFAC_ERR_ARG, "null input of %llu bytes", (unsigned long long)total_in);
-    uint32_t grid = 0;
-    int e = split_prepare(ctx, slot, cap, stream, &grid);
+    int e = split_prepare(ctx, slot, cap, stream);
     if (e || (e = f->d_packed.reserve((size_t)packed + 48, std::max<size_t>((size_t)packed + 48, 1 << 20), stream))) return e;
     const size_t nc = n_chunks;
     e = f->stage.upload(4 * nc + 1, stream, [&](uint32_t *h) {
@@ -685,7 +690,7 @@ int launch_flows(pfac_flows *f, Slot &slot, const void *d_in, const uint64_t *ch
     n.launches += k.launches;
     n.tiles = k.tiles;
     n.ctas = k.ctas;
-    e = launch_split<true>(ctx, slot, grid, fp.doc, fp.tail, n_chunks, d_out, cap, d_chunk_first, nullptr, stream, n);
+    e = launch_split<true>(ctx, slot, fp.doc, fp.tail, n_chunks, d_out, cap, d_chunk_first, nullptr, stream, n);
     if (e) return e;
     const uint32_t tgrid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((nc + 7) / 8, 2ull * (uint64_t)ctx->sm_count));
     const cudaLaunchConfig_t tl = launch_config(ctx, stream, tgrid, kFlowThreads, 0);
@@ -995,7 +1000,7 @@ int pfac_ctx_create(int device, const pfac_tables *t, int part, int n_streams, s
 
     CU_TRY(cudaStreamCreateWithFlags(&ctx->own_stream, cudaStreamNonBlocking));
     CU_TRY(cudaEventCreateWithFlags(&ctx->own_done, cudaEventDisableTiming));
-    e = slot_init(ctx->own);
+    e = slot_init(ctx.get(), ctx->own);
     if (e) return e;
     *out = ctx.release();
     return PFAC_OK;
@@ -1220,7 +1225,7 @@ int pfac_scan_host(pfac_ctx *ctx, const void *h_in, uint64_t n_starts, uint64_t 
         if (!st.stream) {
             CU_TRY(cudaStreamCreateWithFlags(&st.stream, cudaStreamNonBlocking));
             CU_TRY(cudaEventCreateWithFlags(&st.done, cudaEventDisableTiming));
-            if ((e = slot_init(st.slot))) return e;
+            if ((e = slot_init(ctx, st.slot))) return e;
         }
         const size_t need_out = std::max<size_t>((size_t)(first / 8), 4096);
         if ((e = st.d_in.reserve((size_t)(first + halo + 64), 0, st.stream)) || (e = st.d_out.reserve(need_out, 0, st.stream)))

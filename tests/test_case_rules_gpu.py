@@ -304,6 +304,71 @@ def test_capacity_and_one_rescan():
     m.close()
 
 
+def test_batch_whose_verify_pass_overflows():
+    """A mixed batch runs the verify pass and then the batch split pass over one per-CTA count buffer.  With the
+    detector's records beyond their buffer (max(cap, 4096) records) the verify pass overflows first and the split
+    pass passes its count on: PFAC_ERR_OUTPUT_FULL with a count of at least the exact one, nothing past d_out[cap),
+    and one rescan with that count gives every document's records and doc_first.  A smaller batch and a flow call
+    on the same context then match the reference: nothing carries over from one pass or call to the next."""
+    torch = torch_cuda()
+    blob = b"abc\nXyZ\nxyz\nQQQq\n"
+    rules = [1, 0, 1, 0]
+    ref = CaseRulesRef(blob, rules)
+    unit = b"abc xyz XyZ XYZ qqqq qqqq qqqq "    # 7 detector records, 5 expanded
+    m = pf.Matcher(pf.Tables.from_bytes(blob, 1, 256, caseless=rules), device=0)
+
+    def per_doc(text, cuts, first, rec, what):
+        want_first = [0]
+        for i in range(len(cuts) - 1):
+            a, b = int(cuts[i]), int(cuts[i + 1])
+            wp, wi = ref.scan(text[a:b])
+            got = rec[int(first[i]):int(first[i + 1])]
+            assert np.array_equal(got[:, 0], wp) and np.array_equal(got[:, 1], wi), (what, i)
+            want_first.append(want_first[-1] + len(wp))
+        assert np.array_equal(first, want_first), what
+        return want_first[-1]
+
+    text = np.frombuffer(unit * 2000, dtype=np.uint8)
+    n = len(text)
+    cuts = np.unique(np.concatenate([[0, n], np.random.default_rng(8).integers(0, n, 40)])).astype(np.uint64)
+    exact = sum(len(ref.scan(text[int(cuts[i]):int(cuts[i + 1])])[0]) for i in range(len(cuts) - 1))
+    d = torch.from_numpy(text.copy()).cuda()
+
+    def batch(cap):
+        out = torch.zeros((cap + 16, 2), dtype=torch.int32, device="cuda")
+        first = torch.zeros(len(cuts), dtype=torch.int64, device="cuda")
+        cnt = C.c_uint64(0)
+        torch.cuda.synchronize()
+        rc = lib.pfac_scan_batch_device_sync(m._h, d.data_ptr(), cuts.ctypes.data, len(cuts) - 1, out.data_ptr(), cap,
+                                             first.data_ptr(), C.byref(cnt), None)
+        return rc, cnt.value, out, first
+
+    cap = 100
+    rc, cnt, out, _ = batch(cap)
+    assert 7 * 2000 > max(cap, 4096)
+    assert rc == PFAC_ERR_OUTPUT_FULL and cnt >= exact, (rc, cnt, exact)
+    assert out[cap:].abs().sum().item() == 0   # nothing past d_out[cap)
+    rc, cnt2, out, first = batch(cnt)
+    assert rc == 0 and cnt2 == exact
+    rec = out[:cnt2].cpu().numpy().astype(np.int64)
+    assert per_doc(text, cuts, first.cpu().numpy(), rec, "rescan") == exact
+    # a smaller batch on the same context
+    small = np.frombuffer(unit * 300, dtype=np.uint8)
+    cuts2 = np.unique(np.concatenate([[0, len(small)], np.random.default_rng(9).integers(0, len(small), 25)]))
+    first2, rec2 = m.scan_batch(small, cuts2)
+    rec2 = np.stack([rec2["pos"].astype(np.int64), rec2["id"].astype(np.int64)], axis=1)
+    per_doc(small, cuts2, first2.astype(np.int64), rec2, "second batch")
+    # and a flow call
+    fl = m.flows(2)
+    offs = np.array([0, 1000, len(small)], dtype=np.uint64)
+    chunk_first, base, rec3 = fl.scan([0, 1], small, offs)
+    assert base.tolist() == [0, 0]
+    rec3 = np.stack([rec3["pos"].astype(np.int64), rec3["id"].astype(np.int64)], axis=1)
+    per_doc(small, offs, chunk_first.astype(np.int64), rec3, "flows")
+    fl.close()
+    m.close()
+
+
 def test_uniform_rules_launch_and_report_as_the_uniform_sets():
     torch = torch_cuda()
     pats = mixed_set(5)
